@@ -2,6 +2,7 @@
 """Benchmark of the differentiable stepping hot path: world-steps/s, forward + backward.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--worlds 4096] [--sim-steps 30]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (BASELINE.json configs[1], "system_identification shape"): W independent worlds per GPU, each a 1x1x1
@@ -45,6 +46,9 @@ def parse():
     ap.add_argument('--no-secondary', action='store_true', help='skip the config-3 / 4 / 5 secondary workloads')
     ap.add_argument('--strong-total', type=int, default=65536,
                     help='total worlds of the strong-scaling pass (config 5; 0 = skip)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned (loss, gradients, final poses and velocities) as '
+                         'DIR/<name>.npy, to compare two builds output for output')
     return ap.parse_args()
 
 
@@ -110,6 +114,29 @@ def gpu_iteration(spec, params_dev, sim_steps, device):
     return loss.detach(), {k: v.grad for k, v in leaves.items()}, world
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, loss, grads, world):
+    """What one optimisation iteration hands its caller -- the loss, the per-world gradients and the final poses and
+    velocities of every body -- as float64 `out_dir/<name>.npy`.  Above DUMP_LIMIT bytes in all, a fixed seeded
+    sample of the worlds is written instead; `world_index.npy` names the worlds written."""
+    import numpy as np
+    per_world = {'grad_' + k: g.detach() for k, g in grads.items()}
+    per_world['final_p'] = world.get_p().detach().reshape(world.W, -1)
+    per_world['final_v'] = world.get_v().detach().reshape(world.W, -1)
+    row_bytes = 8 * (1 + sum(t.numel() // world.W for t in per_world.values()))
+    keep = min(world.W, (DUMP_LIMIT - 8) // row_bytes)
+    idx = torch.arange(world.W)
+    if keep < world.W:
+        idx = torch.randperm(world.W, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'loss': loss.detach().reshape(1), 'world_index': idx}
+    arrays.update({k: t[idx.to(t.device)] for k, t in per_world.items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy().astype(np.float64))
+
+
 def run_ours(args):
     import torch.distributed as dist
     from diffsdfsim_b200 import _lib, scenes, distributed as D
@@ -160,6 +187,7 @@ def run_ours(args):
             torch.cuda.synchronize(); dbg.append(time.time())
     e1.record()
     barrier()
+    last = (loss, grads, world)
     ms = e0.elapsed_time(e1)
     if dbg:
         print('rank', rank, 'value-loop step end times (s):', [round(t - dbg[0], 3) for t in dbg], 'total ms', ms, file=sys.stderr)
@@ -183,6 +211,8 @@ def run_ours(args):
     barrier()
     ms_e2e = e2.elapsed_time(e3)
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     # ---- separate profiling pass (NOT part of any reported throughput): per-kernel device time of one iteration
     prof = kernel_profile(spec, dev, args.sim_steps, device) if rank == 0 else {}
     final_pos = world.bodies[-1].pos.detach().cpu()

@@ -255,7 +255,8 @@ def golden_sdf():
         pts[:64] = torch.round(pts[:64] / s * 4) / 4 * s
         sd, gr = b.query_sdfs(pts.clone())
         d[nm + '_pts'], d[nm + '_sdf'], d[nm + '_dir'] = pts.numpy(), sd.numpy(), gr.numpy()
-    np.savez_compressed(os.path.join(HERE, 'sdf_query.npz'), **d)
+    # the first 3072 points of each kind (the 64 tie / surface points included) keep the file under 1 MB
+    np.savez_compressed(os.path.join(HERE, 'sdf_query.npz'), **{k: v[:3072] for k, v in d.items()})
     print('sdf_query', {k: v.shape for k, v in d.items()})
 
 
