@@ -158,6 +158,47 @@ __device__ inline void block_lu_solve(const double* LU, int ld, int n, const int
     __syncthreads();
 }
 
+// In-place LU with partial (row) pivoting by one warp, same contract as block_lu; returns 1 on a zero / NaN pivot column.
+__device__ inline int warp_lu(double* A, int ld, int n, int* perm) {
+    const int lane = threadIdx.x & 31;
+    int fail = 0;
+    for (int i = lane; i < n; i += 32) perm[i] = i;
+    __syncwarp();
+    for (int k = 0; k < n; ++k) {
+        double best = -1.0; int bi = k;
+        for (int i = k + lane; i < n; i += 32) { double v = fabs(A[i * ld + k]); if (v > best) { best = v; bi = i; } }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            double ob = __shfl_xor_sync(DSDF_FULL, best, o); int oi = __shfl_xor_sync(DSDF_FULL, bi, o);
+            if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+        }
+        if (!(best > 0.0)) fail = 1;
+        if (bi != k) {
+            for (int j = lane; j < n; j += 32) { double t = A[k * ld + j]; A[k * ld + j] = A[bi * ld + j]; A[bi * ld + j] = t; }
+            if (lane == 0) { int t = perm[k]; perm[k] = perm[bi]; perm[bi] = t; }
+        }
+        __syncwarp();
+        const double piv = A[k * ld + k];
+        for (int i = k + 1 + lane; i < n; i += 32) {
+            const double l = A[i * ld + k] / piv;
+            A[i * ld + k] = l;
+            for (int j = k + 1; j < n; ++j) A[i * ld + j] -= l * A[k * ld + j];
+        }
+        __syncwarp();
+    }
+    return fail;
+}
+
+// x <- (P L U)^-1 b by one warp.  b and x in shared memory, may NOT alias.
+__device__ inline void warp_lu_solve(const double* LU, int ld, int n, const int* perm, const double* b, double* x) {
+    const int lane = threadIdx.x & 31;
+    for (int i = lane; i < n; i += 32) x[i] = b[perm[i]];
+    __syncwarp();
+    warp_trsv_lower_unit(LU, ld, n, x);
+    warp_trsv_upper(LU, ld, n, x);
+    __syncwarp();
+}
+
 // Per-thread solve of one right-hand side with a SMALL factorisation (used for many-RHS solves):
 // src read with stride ss, result written with stride ds; `n` small (nz / neq).
 __device__ inline void thread_lu_solve(const double* LU, int ld, int n, const int* perm,

@@ -1,5 +1,5 @@
 // Fused contact dynamics: LCP assembly + primal-dual interior point + (backward) implicit differentiation,
-// ONE WARP PER WORLD, exploiting the contact structure of the reference's LCP instead of a dense factorisation.
+// exploiting the contact structure of the reference's LCP instead of a dense factorisation.
 //
 // Replaces PdipmEngine.solve_dynamics (lcp_physics/physics/engines.py:31-83) end to end, i.e. the same mathematics
 // as dsdf_dynamics_assemble + dsdf_lcp_forward/backward (which remain the dense, general LCPFunction path):
@@ -16,120 +16,193 @@
 // more: pivoted LU of the FREE block M~_FF only ((6 nb - neq)^2: 6 x 6 for the box-on-plane scene instead of
 // 100 x 100), multipliers dy = r_P - M~_PF dx_F from the pinned rows.  Same Newton systems, same iterates up to
 // round-off; verified against the dense kernels and the oracle in tests/test_dynsolve_gpu.py.
+//
+// One solver, run by a team of threads per world (SURVEY.md hard part 4: KKT beyond shared memory / body-pair block
+// sparsity):
+//   * WarpTeam, one warp per world: the whole world in shared memory, up to 64 contacts.  The default.
+//   * CtaTeam, one CTA of 256 threads per world: many bodies (6 nb - neq free velocity components up to ~120) and / or
+//     many contacts (hundreds).  Shared memory holds only what scales with the number of BODIES; what scales with the
+//     number of CONTACTS lives in a caller-provided global workspace (L2 resident, ~1.5 KB per contact), so there is
+//     no cap on the contact count.
+// Per-body contact lists (ascending contact index, so every sum keeps a fixed order) give G'w, the assembly of M~_FF
+// and the per-body gradients: cost O(nF^2 * contacts per body) instead of O(nF^2 * contacts).
 #include "dsdf_math.cuh"
 #include "dsdf_dense.cuh"
 #include "dsdf_steploop.cuh"
-#include "dsdf_dyn_common.cuh"
 #include "../../include/dsdf_b200.h"
 
 namespace dsdf {
 
-struct DynSmem {
-    int C, per, R, nz, neq, nq, nF, ldF, nb, half, gs;   // gs = doubles of G per contact = (1 + fd/2) * 12
-    size_t oG, oYG, oA, oDen, oAP, oV, oK, oQ, oS, oI, bytes;
-};
-enum { DV_S = 0, DV_Z, DV_RZ, DV_T, DV_DSA, DV_DZA, DV_DS, DV_DZ, DV_D, DV_COUNT };   // 9 row vectors per world
-enum { DS_XY = 0, DS_RXY, DS_DXYA, DS_DXY, DS_BXY, DS_P, DS_RHS, DS_TF, DS_XF, DS_COUNT };
+// ---- contact-row geometry: tangent basis (physics3d/utils.py:247-256, physics3d/world.py:84-94), Jacobian rows
+// (physics3d/world.py:56-101), world-frame inertia (bodies.py:509-511), reference row order
+template <class S> __device__ __forceinline__ V3<S> tseed(V3<S> n) {
+    const double ax = fabs(val(n.x)), ay = fabs(val(n.y)), az = fabs(val(n.z));
+    int k = 0;
+    double m = ax;
+    if (ay < m) { m = ay; k = 1; }
+    if (az < m) { k = 2; }
+    S one = cst(n.x, 1.0), zero = cst(n.x, 0.0);
+    return cross(v3<S>(k == 0 ? one : zero, k == 1 ? one : zero, k == 2 ? one : zero), n);
+}
+template <class S> __device__ __forceinline__ void fdirs(V3<S> n, int fd, V3<S>* dirs) {
+    V3<S> d1 = normalize3(tseed(n));
+    V3<S> d2 = normalize3(cross(d1, n));
+    const int half = fd / 2;
+    dirs[0] = d1; dirs[1] = d2;
+    if (fd == 8) {
+        V3<S> d3 = normalize3(d1 + d2);
+        dirs[2] = d3; dirs[3] = normalize3(cross(d3, n));
+    }
+    for (int r = 0; r < half; ++r) dirs[half + r] = neg(dirs[r]);
+}
+// 12-entry row [p1 x d, d, -(p2 x d), -d]
+template <class S> __device__ __forceinline__ void row12(V3<S> p1, V3<S> p2, V3<S> d, S* o) {
+    V3<S> c1 = cross(p1, d), c2 = cross(p2, d);
+    o[0] = c1.x; o[1] = c1.y; o[2] = c1.z; o[3] = d.x; o[4] = d.y; o[5] = d.z;
+    o[6] = -c2.x; o[7] = -c2.y; o[8] = -c2.z; o[9] = -d.x; o[10] = -d.y; o[11] = -d.z;
+}
+template <class S> __device__ __forceinline__ M3<S> winertia(Q4<S> q, const S* I9) {
+    M3<S> R = q2mat(q), I, Rt;
+#pragma unroll
+    for (int e = 0; e < 9; ++e) I.m[e] = I9[e];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) Rt.m[3 * i + j] = R.m[3 * j + i];
+    return mat_mul(mat_mul(R, I), Rt);
+}
+// reference row index of contact-major row (cc, j): [normal nc | friction fd nc | cone nc]
+__device__ __forceinline__ int ref_row(int cc, int j, int nc, int fd) {
+    return j == 0 ? cc : (j <= fd ? nc + fd * cc + (j - 1) : nc + fd * nc + cc);
+}
 
-__host__ __device__ inline DynSmem dyn_layout(int nb, int neq, int C, int fd) {
-    DynSmem L;
+// ---- teams: who iterates, synchronises, reduces and factors.  Every member is called by all threads of the team.
+struct WarpTeam {
+    static constexpr int kThreads = 32, kFwdMinBlocks = 12, kBwdMinBlocks = 10;
+    static constexpr bool kContactsInSmem = true;      // both layout regions in dynamic shared memory
+    __device__ __forceinline__ static int rank() { return threadIdx.x & 31; }
+    __device__ __forceinline__ static constexpr int size() { return 32; }
+    __device__ __forceinline__ static void sync() { __syncwarp(); }
+    __device__ __forceinline__ static double sum(double v) { return warp_sum(v); }
+    __device__ __forceinline__ static double min(double v) { return warp_min(v); }
+    __device__ __forceinline__ static double max(double v) { return warp_max(v); }
+    __device__ __forceinline__ static int lu(double* A, int ld, int n, int* perm) { return warp_lu(A, ld, n, perm); }
+    __device__ __forceinline__ static void lu_solve(const double* LU, int ld, int n, const int* perm, const double* b,
+                                                    double* x) {
+        warp_lu_solve(LU, ld, n, perm, b, x);
+    }
+};
+struct CtaTeam {
+    // forward: two CTAs per SM, i.e. at most 128 registers (no spills); backward: no minimum (0), one CTA per SM
+    static constexpr int kThreads = 256, kFwdMinBlocks = 2, kBwdMinBlocks = 0;
+    static constexpr bool kContactsInSmem = false;     // contact region in the global workspace
+    __device__ __forceinline__ static int rank() { return threadIdx.x; }
+    __device__ __forceinline__ static int size() { return blockDim.x; }
+    __device__ __forceinline__ static void sync() { __syncthreads(); }
+    __device__ __forceinline__ static double* red() { __shared__ double r[33]; return r; }
+    __device__ __forceinline__ static double sum(double v) { return block_reduce<RED_SUM>(v, red()); }
+    __device__ __forceinline__ static double min(double v) { return block_reduce<RED_MIN>(v, red()); }
+    __device__ __forceinline__ static double max(double v) { return block_reduce<RED_MAX>(v, red()); }
+    __device__ __forceinline__ static int lu(double* A, int ld, int n, int* perm) {
+        __shared__ int piv[2];                         // pivot row, failure flag
+        if (threadIdx.x == 0) piv[1] = 0;
+        __syncthreads();
+        block_lu(A, ld, n, perm, &piv[0], &piv[1]);
+        __syncthreads();
+        return piv[1];
+    }
+    __device__ __forceinline__ static void lu_solve(const double* LU, int ld, int n, const int* perm, const double* b,
+                                                    double* x) {
+        block_lu_solve(LU, ld, n, perm, b, x);
+    }
+};
+// i = rank, rank + size, ... < n over the team of the enclosing template (`Team`)
+#define TFOR(i, n) for (int i = Team::rank(); i < (n); i += Team::size())
+
+// ---- per-world layout: a body region (shared memory) and a contact region (shared memory after the body region for
+// the warp; the global workspace for the CTA).  Offsets in doubles.
+enum { DV_S = 0, DV_Z, DV_RZ, DV_T, DV_DSA, DV_DZA, DV_DS, DV_DZ, DV_D, DV_COUNT };   // 9 row vectors per world
+enum { DS_XY = 0, DS_RXY, DS_DXYA, DS_DXY, DS_BXY, DS_P, DS_RHS, DS_TF, DS_XF, DS_COUNT };   // nq-sized vectors
+
+struct DynLayout {
+    int C, per, R, nz, neq, nq, nF, ldF, nb, half, gs;   // gs = doubles of G per contact = (1 + fd/2) * 12
+    size_t oK, oQ, oS, oI, body;
+    size_t oG, oYG, oA, oDen, oAP, oV, oMu, oE, oH, oCb, contact;
+};
+
+__host__ __device__ inline DynLayout dyn_layout(int nb, int neq, int C, int fd) {
+    DynLayout L;
     L.C = C; L.per = 2 + fd; L.R = C * L.per; L.nz = 6 * nb; L.neq = neq; L.nq = L.nz + neq; L.nb = nb;
     L.nF = L.nz - neq; L.ldF = L.nF | 1; L.half = fd / 2; L.gs = (1 + L.half) * 12;
     size_t o = 0;
-    L.oG = o;   o += (size_t)C * L.gs;        // normal row + the first fd/2 friction rows (the rest are their negatives)
-    L.oYG = o;  o += (size_t)C * 12;
-    L.oA = o;   o += L.R;                 // a = 1/d
-    L.oDen = o; o += C;
-    L.oAP = o;  o += (size_t)2 * C * L.half;  // per friction pair: 1/a_q + 1/a_{q+half}, 1/a_q - 1/a_{q+half}
-    L.oV = o;   o += (size_t)DV_COUNT * L.R;
-    L.oK = o;   o += (size_t)L.nz * L.ldF;      // rows [0,nF): M~_FF (LU in place); rows [nF,nz): M~_PF
+    // ints first: bstart then sits at the start of dynamic shared memory, a constant address (one register fewer in the
+    // one-warp backward, which spills otherwise)
+    L.oI = o;   o += ((size_t)nb + 1 + 2 * C + 2 * neq + L.nF + 2 * L.nz + 1) / 2;   // ints: bstart blist eq perm fidx fpos
+    L.oK = o;   o += (size_t)L.nF * L.ldF;        // M~_FF, LU in place
     L.oQ = o;   o += (size_t)nb * 36;
     L.oS = o;   o += (size_t)DS_COUNT * L.nq;
-    L.oI = o;   o += (size_t)(2 * C + 2 * neq + L.nq + 2 * L.nz + 8 + 1) / 2 + 1;
-    L.bytes = o * sizeof(double);
+    L.body = o;
+    o = 0;
+    L.oG = o;   o += (size_t)C * L.gs;            // normal row + the first fd/2 friction rows (the rest are their negatives)
+    L.oYG = o;  o += (size_t)C * 12;
+    L.oA = o;   o += L.R;                         // a = 1/d
+    L.oDen = o; o += C;
+    L.oAP = o;  o += (size_t)2 * C * L.half;      // per friction pair: 1/a_q + 1/a_{q+half}, 1/a_q - 1/a_{q+half}
+    L.oV = o;   o += (size_t)DV_COUNT * L.R;
+    L.oMu = o;  o += C;                           // per contact: friction coefficient, restitution, h
+    L.oE = o;   o += C;
+    L.oH = o;   o += C;
+    L.oCb = o;  o += C;                           // 2 ints per contact: its bodies
+    L.contact = o;
     return L;
 }
 
 struct DynCtx {
-    DynSmem L;
-    int nc, ni;                     // active contacts / rows of this world
-    double *G, *YG, *a, *den, *AP, *V, *K, *Qb, *Sv;
-    int *cb, *eq, *perm, *fidx, *fpos;   // fidx[jf] = free dof; fpos[I] = jf (free) or -(m+1) (pinned by row m)
+    DynLayout L;
+    int nc, ni;                                         // active contacts / rows of this world
+    double *K, *Qb, *Sv;                                // body region
+    int *eq, *perm, *fidx, *fpos, *bstart, *blist;     // fidx[jf] = free dof; fpos[I] = jf (free) or -(m+1) (pinned by
+                                                        // row m); blist[bstart[b] .. bstart[b+1]) = 2 contact + side
+    double *G, *YG, *a, *den, *AP, *V, *mu, *e, *h;     // contact region
+    int* cb;
     __device__ double* vec(int k) const { return V + (size_t)k * L.R; }
     __device__ double* sv(int k) const { return Sv + (size_t)k * L.nq; }
     __device__ int gidx(int c, int k) const { return 6 * cb[2 * c + (k >= 6)] + (k % 6); }
 };
 
-// DSDF_DYN_OUTLINE: keep ONE out-of-line copy of the building blocks (the kernel is 17 k SASS instructions = 280 KB when
-// everything is inlined, far beyond the instruction cache; ncu: 13-34 % of stall samples "no_instructions")
-#ifdef DSDF_DYN_OUTLINE
-#define DYN_FN __device__ __noinline__
-#else
-#define DYN_FN __device__ __forceinline__
-#endif
-__device__ __forceinline__ double wsum(double v) { return warp_sum(v); }
-
-// ---- warp-level pivoted LU / solve on a small matrix in shared memory ---------------------------------------
-DYN_FN int warp_lu(double* A, int ld, int n, int* perm) {
-    const int lane = threadIdx.x & 31;
-    int fail = 0;
-    for (int i = lane; i < n; i += 32) perm[i] = i;
-    __syncwarp();
-    for (int k = 0; k < n; ++k) {
-        double best = -1.0; int bi = k;
-        for (int i = k + lane; i < n; i += 32) { double v = fabs(A[i * ld + k]); if (v > best) { best = v; bi = i; } }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            double ob = __shfl_xor_sync(DSDF_FULL, best, o); int oi = __shfl_xor_sync(DSDF_FULL, bi, o);
-            if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-        }
-        if (!(best > 0.0)) fail = 1;
-        if (bi != k) {
-            for (int j = lane; j < n; j += 32) { double t = A[k * ld + j]; A[k * ld + j] = A[bi * ld + j]; A[bi * ld + j] = t; }
-            if (lane == 0) { int t = perm[k]; perm[k] = perm[bi]; perm[bi] = t; }
-        }
-        __syncwarp();
-        const double piv = A[k * ld + k];
-        for (int i = k + 1 + lane; i < n; i += 32) {
-            const double l = A[i * ld + k] / piv;
-            A[i * ld + k] = l;
-            for (int j = k + 1; j < n; ++j) A[i * ld + j] -= l * A[k * ld + j];
-        }
-        __syncwarp();
-    }
-    return fail;
-}
-// x <- (PLU)^-1 b ; b, x distinct shared vectors
-DYN_FN void warp_lu_solve(const double* LU, int ld, int n, const int* perm, const double* b, double* x) {
-    const int lane = threadIdx.x & 31;
-    for (int i = lane; i < n; i += 32) x[i] = b[perm[i]];
-    __syncwarp();
-    warp_trsv_lower_unit(LU, ld, n, x);
-    warp_trsv_upper(LU, ld, n, x);
-    __syncwarp();
+__device__ inline DynCtx dyn_ctx(double* body, double* contact, const DynLayout& L) {
+    DynCtx c;
+    c.L = L;
+    c.K = body + L.oK; c.Qb = body + L.oQ; c.Sv = body + L.oS;
+    c.bstart = reinterpret_cast<int*>(body + L.oI); c.blist = c.bstart + L.nb + 1; c.eq = c.blist + 2 * L.C;
+    c.perm = c.eq + 2 * L.neq; c.fidx = c.perm + L.nF; c.fpos = c.fidx + L.nz;
+    c.G = contact + L.oG; c.YG = contact + L.oYG; c.a = contact + L.oA; c.den = contact + L.oDen; c.AP = contact + L.oAP;
+    c.V = contact + L.oV; c.mu = contact + L.oMu; c.e = contact + L.oE; c.h = contact + L.oH;
+    c.cb = reinterpret_cast<int*>(contact + L.oCb);
+    c.nc = c.ni = 0;
+    return c;
 }
 
-// ---- load one world's problem into shared memory ---------------------------------------------------------------
-DYN_FN void dyn_load(DynCtx& c, int w, const double* p, const double* v, const double* mass, const double* Ibody,
-                         const double* fric, const double* rest, const double* f, double dtw, const int* count,
-                         const int* cbody, const double* cgeo, const int* eq_rows, int maxc, int fd, double* mu_out,
-                         double* e_out, double* h_out) {
-    const int lane = threadIdx.x & 31;
-    const DynSmem& L = c.L;
+// ---- load one world's problem ------------------------------------------------------------------------------------
+template <class Team>
+__device__ __forceinline__ void dyn_load(DynCtx& c, int w, const double* p, const double* v, const double* mass,
+                                         const double* Ibody, const double* fric, const double* rest, const double* f,
+                                         double dtw, const int* count, const int* cbody, const double* cgeo,
+                                         const int* eq_rows, int maxc, int fd) {
+    const DynLayout& L = c.L;
     const int nb = L.nb, nz = L.nz;
     c.nc = min(min(count[w], maxc), L.C);
     c.ni = c.nc * L.per;
-    for (int i = lane; i < 2 * L.neq; i += 32) c.eq[i] = eq_rows[i];
-    for (int i = lane; i < nz; i += 32) c.fpos[i] = 0;
-    __syncwarp();
-    for (int m = lane; m < L.neq; m += 32) c.fpos[6 * c.eq[2 * m] + c.eq[2 * m + 1]] = -(m + 1);
-    __syncwarp();
-    if (lane == 0) {
+    TFOR(i, 2 * L.neq) c.eq[i] = eq_rows[i];
+    TFOR(i, nz) c.fpos[i] = 0;
+    Team::sync();
+    TFOR(m, L.neq) c.fpos[6 * c.eq[2 * m] + c.eq[2 * m + 1]] = -(m + 1);
+    Team::sync();
+    if (Team::rank() == 0) {
         int jf = 0;
         for (int i = 0; i < nz; ++i) if (c.fpos[i] == 0) { c.fidx[jf] = i; c.fpos[i] = jf++; }
     }
-    __syncwarp();
-    for (int b = lane; b < nb; b += 32) {
+    TFOR(b, nb) {
         const double* pb = p + ((size_t)w * nb + b) * 7;
         M3<double> Iw = winertia<double>(q4<double>(pb[0], pb[1], pb[2], pb[3]), Ibody + ((size_t)w * nb + b) * 9);
         const double m = mass[(size_t)w * nb + b];
@@ -140,7 +213,7 @@ DYN_FN void dyn_load(DynCtx& c, int w, const double* p, const double* v, const d
             Q[6 * (3 + i) + 3 + i] = m;
         }
     }
-    for (int cc = lane; cc < c.nc; cc += 32) {
+    TFOR(cc, c.nc) {
         const size_t oo = (size_t)w * maxc + cc;
         const int i1 = cbody[2 * oo], i2 = cbody[2 * oo + 1];
         c.cb[2 * cc] = i1; c.cb[2 * cc + 1] = i2;
@@ -151,13 +224,33 @@ DYN_FN void dyn_load(DynCtx& c, int w, const double* p, const double* v, const d
         V3<double> dirs[8];
         fdirs<double>(n, fd, dirs);
         for (int r = 0; r < L.half; ++r) row12<double>(p1, p2, dirs[r], Gc + 12 * (1 + r));   // rows r + half = -rows r
-        mu_out[cc] = 0.5 * (fric[(size_t)w * nb + i1] + fric[(size_t)w * nb + i2]);
-        e_out[cc] = (rest[(size_t)w * nb + i1] + rest[(size_t)w * nb + i2]) / 2;
+        c.mu[cc] = 0.5 * (fric[(size_t)w * nb + i1] + fric[(size_t)w * nb + i2]);
+        c.e[cc] = (rest[(size_t)w * nb + i1] + rest[(size_t)w * nb + i2]) / 2;
     }
-    __syncwarp();
+    Team::sync();
+    // per-body contact lists: entry = 2 * contact + side, ascending contact index (one thread per body).  A contact
+    // joins two different bodies, so it appears at most once in a list.
+    TFOR(b, nb) {
+        int n = 0;
+        for (int cc = 0; cc < c.nc; ++cc) n += (c.cb[2 * cc] == b) + (c.cb[2 * cc + 1] == b);
+        c.bstart[b + 1] = n;
+    }
+    Team::sync();
+    if (Team::rank() == 0) {
+        c.bstart[0] = 0;
+        for (int b = 0; b < nb; ++b) c.bstart[b + 1] += c.bstart[b];
+    }
+    Team::sync();
+    TFOR(b, nb) {
+        int o = c.bstart[b];
+        for (int cc = 0; cc < c.nc; ++cc) {
+            if (c.cb[2 * cc] == b) c.blist[o++] = 2 * cc;
+            if (c.cb[2 * cc + 1] == b) c.blist[o++] = 2 * cc + 1;
+        }
+    }
     // u = M v + dt f
     double* pv = c.sv(DS_P);
-    for (int i = lane; i < nz; i += 32) {
+    TFOR(i, nz) {
         const int b = i / 6, k = i % 6;
         const double* Q = c.Qb + 36 * b;
         double acc = 0.0;
@@ -165,28 +258,28 @@ DYN_FN void dyn_load(DynCtx& c, int w, const double* p, const double* v, const d
         pv[i] = acc + dtw * f[(size_t)w * nz + i];
     }
     // h = [e (Jc v); 0; 0]: one value per contact (normal row), zero on the friction and cone rows
-    for (int cc = lane; cc < c.nc; cc += 32) {
+    TFOR(cc, c.nc) {
         const double* Gc = c.G + (size_t)cc * L.gs;
         double jv = 0.0;
         for (int k = 0; k < 12; ++k) jv += Gc[k] * v[(size_t)w * nz + c.gidx(cc, k)];
-        h_out[cc] = jv * e_out[cc];
+        c.h[cc] = jv * c.e[cc];
     }
-    __syncwarp();
+    Team::sync();
 }
 
 // (F z)[r] for the engine's F in contact-major rows
-__device__ __forceinline__ double Fz_row(const DynCtx& c, const double* z, const double* mu, int r, int fd) {
+__device__ __forceinline__ double Fz_row(const DynCtx& c, const double* z, int r, int fd) {
     const int per = c.L.per, cc = r / per, j = r % per;
     if (j == 0) return 0.0;
     if (j <= fd) return z[cc * per + per - 1];
-    double acc = mu[cc] * z[cc * per];
+    double acc = c.mu[cc] * z[cc * per];
     for (int q = 1; q <= fd; ++q) acc -= z[cc * per + q];
     return acc;
 }
 // out = G x for all rows (contact-major): friction row q + half is the negative of row q, the cone row is zero
-DYN_FN void Gx_all(const DynCtx& c, const double* x, double* out) {
-    const int lane = threadIdx.x & 31, per = c.L.per, half = c.L.half, rows = 1 + half;
-    for (int e = lane; e < c.nc * rows; e += 32) {
+template <class Team> __device__ __forceinline__ void Gx_all(const DynCtx& c, const double* x, double* out) {
+    const int per = c.L.per, half = c.L.half, rows = 1 + half;
+    TFOR(e, c.nc * rows) {
         const int cc = e / rows, j = e % rows;
         const double* Gc = c.G + (size_t)cc * c.L.gs + 12 * j;
         double acc = 0.0;
@@ -196,15 +289,14 @@ DYN_FN void Gx_all(const DynCtx& c, const double* x, double* out) {
         if (j >= 1) out[cc * per + j + half] = -acc;
         else out[cc * per + per - 1] = 0.0;
     }
-    __syncwarp();
+    Team::sync();
 }
-// (G' w)[I]
-DYN_FN double Gtw_row(const DynCtx& c, const double* w, int I, int fd) {
+// (G' w)[I] through the contact list of I's body
+__device__ __forceinline__ double Gtw_row(const DynCtx& c, const double* w, int I) {
     const int per = c.L.per, half = c.L.half, b = I / 6, k6 = I % 6;
     double acc = 0.0;
-    for (int cc = 0; cc < c.nc; ++cc) {
-        int k;
-        if (c.cb[2 * cc] == b) k = k6; else if (c.cb[2 * cc + 1] == b) k = 6 + k6; else continue;
+    for (int t = c.bstart[b]; t < c.bstart[b + 1]; ++t) {
+        const int cc = c.blist[t] >> 1, k = (c.blist[t] & 1) * 6 + k6;
         const double* Gc = c.G + (size_t)cc * c.L.gs + k;
         const double* wc = w + cc * per;
         double a2 = Gc[0] * wc[0];
@@ -214,63 +306,63 @@ DYN_FN double Gtw_row(const DynCtx& c, const double* w, int I, int fd) {
     return acc;
 }
 // solve B_c u = t for every contact in place on t (contact-major), thread per contact
-DYN_FN void block_solve(const DynCtx& c, const double* mu, double* t, int fd) {
-    const int lane = threadIdx.x & 31, per = c.L.per;
-    for (int cc = lane; cc < c.nc; cc += 32) {
+template <class Team> __device__ __forceinline__ void block_solve(const DynCtx& c, double* t, int fd) {
+    const int per = c.L.per;
+    TFOR(cc, c.nc) {
         double* tc = t + cc * per;
         const double* ac = c.a + cc * per;
         const double un = tc[0] * ac[0];                 // ac = 1/a: reciprocals of B's diagonal (no fp64 divides here)
         double sum = 0.0;
         for (int q = 1; q <= fd; ++q) sum += tc[q] * ac[q];
-        const double ug = (tc[per - 1] - mu[cc] * un + sum) * c.den[cc];
+        const double ug = (tc[per - 1] - c.mu[cc] * un + sum) * c.den[cc];
         tc[0] = un;
         for (int q = 1; q <= fd; ++q) tc[q] = (tc[q] - ug) * ac[q];
         tc[per - 1] = ug;
     }
-    __syncwarp();
+    Team::sync();
 }
 
 // factor: a = 1/d, den, YG, K = [[Q + sum G' B^-1 G, A'],[A,0]] -> LU.  Returns 1 on a singular K.
-DYN_FN int dyn_factor(DynCtx& c, const double* d, const double* mu, int fd) {
-    const int lane = threadIdx.x & 31;
-    const DynSmem& L = c.L;
-    const int per = L.per, nz = L.nz, nF = L.nF, ld = L.ldF;
+template <class Team> __device__ __forceinline__ int dyn_factor(DynCtx& c, const double* d, int fd) {
+    const DynLayout& L = c.L;
+    const int per = L.per, nF = L.nF, ld = L.ldF, half = L.half;
     // a = 1/d is B's diagonal (batch.py:496); the kernel keeps 1/a and 1/den so the hot loops multiply
-    for (int r = lane; r < c.ni; r += 32) c.a[r] = 1.0 / (1.0 / d[r]);
-    __syncwarp();
-    for (int cc = lane; cc < c.nc; cc += 32) {
+    TFOR(r, c.ni) c.a[r] = 1.0 / (1.0 / d[r]);
+    Team::sync();
+    TFOR(cc, c.nc) {
         const double* ac = c.a + cc * per;
         double dn = 1.0 / d[cc * per + per - 1];
         for (int q = 1; q <= fd; ++q) dn += ac[q];
         c.den[cc] = 1.0 / dn;
     }
-    __syncwarp();
-    const int half = L.half;
-    for (int e = lane; e < c.nc * half; e += 32) {
+    TFOR(e, c.nc * half) {
         const int cc = e / half, q = 1 + e % half;
         const double* ac = c.a + cc * per;
         c.AP[(size_t)2 * e] = ac[q] + ac[q + half];
         c.AP[(size_t)2 * e + 1] = ac[q] - ac[q + half];
     }
-    __syncwarp();
-    for (int e = lane; e < c.nc * 12; e += 32) {
+    Team::sync();
+    TFOR(e, c.nc * 12) {
         const int cc = e / 12, k = e % 12;
         const double* Gc = c.G + (size_t)cc * L.gs + k;
         const double* ap = c.AP + (size_t)2 * cc * half;
-        double acc = -mu[cc] * Gc[0] * c.a[cc * per];
+        double acc = -c.mu[cc] * Gc[0] * c.a[cc * per];
         for (int q = 1; q <= half; ++q) acc += Gc[12 * q] * ap[2 * (q - 1) + 1];
         c.YG[e] = acc * c.den[cc];
     }
-    __syncwarp();
-    // M~_FF = Q_FF + sum_c G_c' B_c^-1 G_c restricted to the free components; thread per entry
-    for (int e = lane; e < nF * nF; e += 32) {
+    Team::sync();
+    // M~_FF = Q_FF + sum_c G_c' B_c^-1 G_c restricted to the free components; thread per entry.  Entry (If, jf) gathers
+    // the contacts that touch BOTH bodies, walking the list of I's body.
+    TFOR(e, nF * nF) {
         const int If = e / nF, jf = e % nF, I = c.fidx[If], J = c.fidx[jf], bI = I / 6, bJ = J / 6;
         double acc = bI == bJ ? c.Qb[36 * bI + 6 * (I % 6) + (J % 6)] : 0.0;
-        for (int cc = 0; cc < c.nc; ++cc) {
-            const int i1 = c.cb[2 * cc], i2 = c.cb[2 * cc + 1];
-            int ki, kj;
-            if (i1 == bI) ki = I % 6; else if (i2 == bI) ki = 6 + I % 6; else continue;
-            if (i1 == bJ) kj = J % 6; else if (i2 == bJ) kj = 6 + J % 6; else continue;
+        for (int t = c.bstart[bI]; t < c.bstart[bI + 1]; ++t) {
+            const int cc = c.blist[t] >> 1, sI = c.blist[t] & 1;
+            int kj;
+            if (bJ == bI) kj = sI * 6 + J % 6;
+            else if (c.cb[2 * cc + (1 - sI)] == bJ) kj = (1 - sI) * 6 + J % 6;
+            else continue;
+            const int ki = sI * 6 + I % 6;
             const double* Gc = c.G + (size_t)cc * L.gs;
             const double* ap = c.AP + (size_t)2 * cc * half;
             double a2 = Gc[ki] * (Gc[kj] * c.a[cc * per]);
@@ -281,85 +373,71 @@ DYN_FN int dyn_factor(DynCtx& c, const double* d, const double* mu, int fd) {
         }
         c.K[If * ld + jf] = acc;
     }
-    __syncwarp();
-    return warp_lu(c.K, ld, nF, c.perm);
+    Team::sync();
+    return Team::lu(c.K, ld, nF, c.perm);
 }
 
 // dx of [[M~, A'], [A, 0]] [dx; dy] = rhs with A a 0/1 selection of the pinned components and rhs_y = 0 (b = 0, x_P = 0):
 // dx_P = rhs_y (= 0), dx_F = (M~_FF)^-1 rhs_F.  The multipliers dy follow from the pinned rows of the un-reduced
 // system once dz is known: dy = -rx_P - (G' dz)_P - (Q dx)_P   (see dyn_solve).
-__device__ inline void kkt_solve(DynCtx& c, const double* rhs, double* dxy) {
-    const int lane = threadIdx.x & 31;
-    const DynSmem& L = c.L;
+template <class Team> __device__ inline void kkt_solve(DynCtx& c, const double* rhs, double* dxy) {
+    const DynLayout& L = c.L;
     const int nz = L.nz, nF = L.nF, ld = L.ldF;
     double *tF = c.sv(DS_TF), *xF = c.sv(DS_XF);
-    for (int jf = lane; jf < nF; jf += 32) tF[jf] = rhs[c.fidx[jf]];
-    __syncwarp();
-    warp_lu_solve(c.K, ld, nF, c.perm, tF, xF);
-    for (int I = lane; I < nz; I += 32) { const int fp = c.fpos[I]; dxy[I] = fp >= 0 ? xF[fp] : rhs[nz + (-fp - 1)]; }
-    __syncwarp();
+    TFOR(jf, nF) tF[jf] = rhs[c.fidx[jf]];
+    Team::sync();
+    Team::lu_solve(c.K, ld, nF, c.perm, tF, xF);
+    TFOR(I, nz) { const int fp = c.fpos[I]; dxy[I] = fp >= 0 ? xF[fp] : rhs[nz + (-fp - 1)]; }
+    Team::sync();
 }
 
 // KKT solve (batch.py:380-410 semantics).  rxy = [rx; ry] (NULL = 0), rs (NULL = 0), rz (NULL = 0).
 // Outputs dxy = [dx; dy], ds, dz.  Scratch: vec(DV_T), sv(DS_RHS).
-DYN_FN void dyn_solve(DynCtx& c, const double* d, const double* mu, int fd, const double* rxy, const double* rs,
-                          const double* rz, double* dxy, double* ds, double* dz) {
-    const int lane = threadIdx.x & 31;
-    const DynSmem& L = c.L;
+template <class Team>
+__device__ __forceinline__ void dyn_solve(DynCtx& c, const double* d, int fd, const double* rxy, const double* rs,
+                                          const double* rz, double* dxy, double* ds, double* dz) {
+    const DynLayout& L = c.L;
     const int nz = L.nz, nq = L.nq;
     double* t = c.vec(DV_T);
     double* rhs = c.sv(DS_RHS);
-    for (int r = lane; r < c.ni; r += 32) t[r] = (rz ? rz[r] : 0.0) - (rs ? rs[r] / d[r] : 0.0);
-    __syncwarp();
-    for (int r = lane; r < c.ni; r += 32) dz[r] = t[r];          // keep t (dz doubles as a second copy)
-    __syncwarp();
-    block_solve(c, mu, t, fd);                                     // t <- u = B^-1 t
-    for (int I = lane; I < nq; I += 32) {
+    TFOR(r, c.ni) { const double tv = (rz ? rz[r] : 0.0) - (rs ? rs[r] / d[r] : 0.0); t[r] = tv; dz[r] = tv; }
+    Team::sync();
+    block_solve<Team>(c, t, fd);                                    // t <- u = B^-1 t (dz keeps a copy of t)
+    TFOR(I, nq) {
         double acc = rxy ? -rxy[I] : 0.0;
-        if (I < nz) acc -= Gtw_row(c, t, I, fd);
+        if (I < nz) acc -= Gtw_row(c, t, I);
         rhs[I] = acc;
     }
-    __syncwarp();
-    kkt_solve(c, rhs, dxy);
-    double* gx = t;                                                                 // t is dead from here on
-    Gx_all(c, dxy, gx);
-    for (int r = lane; r < c.ni; r += 32) dz[r] = gx[r] + dz[r];                    // G dx + t
-    __syncwarp();
-    block_solve(c, mu, dz, fd);
-    for (int m = lane; m < L.neq; m += 32) {                                       // multipliers of the pinned rows
+    Team::sync();
+    kkt_solve<Team>(c, rhs, dxy);
+    double* gx = t;                                                 // t is dead from here on
+    Gx_all<Team>(c, dxy, gx);
+    TFOR(r, c.ni) dz[r] = gx[r] + dz[r];                            // G dx + t
+    Team::sync();
+    block_solve<Team>(c, dz, fd);
+    TFOR(m, L.neq) {                                                // multipliers of the pinned rows
         const int b = c.eq[2 * m], k = c.eq[2 * m + 1], I = 6 * b + k;
-        double acc = (rxy ? -rxy[I] : 0.0) - Gtw_row(c, dz, I, fd);
+        double acc = (rxy ? -rxy[I] : 0.0) - Gtw_row(c, dz, I);
         for (int j = 0; j < 6; ++j) acc -= c.Qb[36 * b + 6 * k + j] * dxy[6 * b + j];
         dxy[nz + m] = acc;
     }
-    __syncwarp();
-    for (int r = lane; r < c.ni; r += 32) ds[r] = ((rs ? -rs[r] : 0.0) - dz[r]) / d[r];
-    __syncwarp();
+    TFOR(r, c.ni) ds[r] = ((rs ? -rs[r] : 0.0) - dz[r]) / d[r];
+    Team::sync();
 }
 
-DYN_FN double dyn_ratio_step(const DynCtx& c, const double* v, const double* dv) {
-    const int lane = threadIdx.x & 31;
+template <class Team> __device__ __forceinline__ double dyn_ratio_step(const DynCtx& c, const double* v, const double* dv) {
     double mx = -INFINITY;
-    for (int r = lane; r < c.ni; r += 32) mx = fmax(mx, -v[r] / dv[r]);
-    mx = warp_max(mx);
+    TFOR(r, c.ni) mx = fmax(mx, -v[r] / dv[r]);
+    mx = Team::max(mx);
     const double repl = fmax(1.0, mx);
     double mn = INFINITY;
-    for (int r = lane; r < c.ni; r += 32) mn = fmin(mn, dv[r] > 0.0 ? repl : -v[r] / dv[r]);
-    return warp_min(mn);
+    TFOR(r, c.ni) mn = fmin(mn, dv[r] > 0.0 ? repl : -v[r] / dv[r]);
+    return Team::min(mn);
 }
 
-__device__ inline DynCtx dyn_ctx(double* sm, const DynSmem& L) {
-    DynCtx c;
-    c.L = L;
-    c.G = sm + L.oG; c.YG = sm + L.oYG; c.a = sm + L.oA; c.den = sm + L.oDen; c.AP = sm + L.oAP; c.V = sm + L.oV; c.K = sm + L.oK;
-    c.Qb = sm + L.oQ; c.Sv = sm + L.oS;
-    int* ib = reinterpret_cast<int*>(sm + L.oI);
-    c.cb = ib; c.eq = ib + 2 * L.C; c.perm = c.eq + 2 * L.neq; c.fidx = c.perm + L.nq; c.fpos = c.fidx + L.nz;
-    c.nc = c.ni = 0;
-    return c;
-}
-
-__global__ void __launch_bounds__(32, 12)
+// work: the global workspace of the CTA kernel (contact regions, one per world); unused by the warp kernel
+template <class Team>
+__global__ void __launch_bounds__(Team::kThreads, Team::kFwdMinBlocks)
 dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, const double* __restrict__ mass,
                    const double* __restrict__ Ibody, const double* __restrict__ fric, const double* __restrict__ rest,
                    const double* __restrict__ f, const double* __restrict__ dt, const unsigned char* __restrict__ active,
@@ -368,37 +446,36 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
                    double eps, int not_improved_lim, int max_iter,
                    double* __restrict__ xo, double* __restrict__ nvo, double* __restrict__ nuo, double* __restrict__ lamo,
                    double* __restrict__ so, int* __restrict__ status_o, int* __restrict__ iters_o,
-                   const int* __restrict__ vmap, int* __restrict__ ctrl, int cmin, int last_class) {
+                   const int* __restrict__ vmap, int* __restrict__ ctrl, int cmin, int last_class,
+                   double* __restrict__ work) {
     extern __shared__ double smd[];
     // loop mode (ctrl != NULL, dsdf_steploop.cu): CTA w solves virtual world w = one attempt (its own dt[w]) of the real
     // world ws = vmap[w], whose state / parameters / contacts are read in place; outputs are indexed by w
-    const int w = blockIdx.x, lane = threadIdx.x & 31;
+    const int w = blockIdx.x;
     if (ctrl && (loop_idle(ctrl) || w >= ctrl[CT_NVIRT])) return;
     const int ws = vmap ? vmap[w] : w;
-    const DynSmem L = dyn_layout(nb, neq, C, fd);
+    const DynLayout L = dyn_layout(nb, neq, C, fd);
     const int nz = L.nz, nq = L.nq, per = L.per;
     if (active && !active[w]) {               // inactive world: velocity passes through
-        if (nvo) for (int i = lane; i < nz; i += 32) nvo[(size_t)w * nz + i] = v[(size_t)ws * nz + i];
+        if (nvo) TFOR(i, nz) nvo[(size_t)w * nz + i] = v[(size_t)ws * nz + i];
         return;
     }
-    DynCtx c = dyn_ctx(smd, L);
     // contact-count classes: one launch sized for the typical count, one for the few worlds with many contacts (a world
     // that gave up halving keeps a penetrating state with dozens of contacts; sizing every CTA for it costs occupancy)
     if (count[ws] <= cmin || (count[ws] > C && !last_class)) return;
-    if (count[ws] > C) {                      // more contacts than this launch's shared memory holds
-        for (int i = lane; i < nz; i += 32) { xo[(size_t)w * nz + i] = NAN; if (nvo) nvo[(size_t)w * nz + i] = NAN; }
-        if (lane == 0) {
+    if (count[ws] > C) {                      // more contacts than this launch's layout holds
+        TFOR(i, nz) { xo[(size_t)w * nz + i] = NAN; if (nvo) nvo[(size_t)w * nz + i] = NAN; }
+        if (Team::rank() == 0) {
             status_o[w] = DSDF_LCP_TOO_LARGE; if (iters_o) iters_o[w] = 0;
             if (ctrl) atomicOr(&ctrl[CT_ABORT], DSDF_STEP_DYN_SMEM);      // the host re-launches with a larger C
         }
         return;
     }
-    __shared__ double s_mu[64], s_e[64], s_h[64];   // per contact: friction coefficient, restitution, h (C <= 64)
-    const double* mu = s_mu;
-    dyn_load(c, ws, p, v, mass, Ibody, fric, rest, f, dt[w], count, cbody, cgeo, eq_rows, maxc, fd, s_mu, s_e, s_h);
-    auto hrow = [&](int r) { return (r % per == 0) ? s_h[r / per] : 0.0; };
+    DynCtx c = dyn_ctx(smd, Team::kContactsInSmem ? smd + L.body : work + (size_t)w * L.contact, L);
+    dyn_load<Team>(c, ws, p, v, mass, Ibody, fric, rest, f, dt[w], count, cbody, cgeo, eq_rows, maxc, fd);
+    auto hrow = [&](int r) { return (r % per == 0) ? c.h[r / per] : 0.0; };
     const int niCap = maxc * per;
-    for (int r = lane; r < niCap; r += 32) { lamo[(size_t)w * niCap + r] = 0.0; so[(size_t)w * niCap + r] = 0.0; }
+    TFOR(r, niCap) { lamo[(size_t)w * niCap + r] = 0.0; so[(size_t)w * niCap + r] = 0.0; }
     const int ni = c.ni;
     double *s = c.vec(DV_S), *z = c.vec(DV_Z), *rz = c.vec(DV_RZ), *dsa = c.vec(DV_DSA),
            *dza = c.vec(DV_DZA), *ds = c.vec(DV_DS), *dz = c.vec(DV_DZ),
@@ -415,13 +492,13 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
     for (int it = -1; it < max_iter; ++it) {
         double res = 0.0;
         if (it < 0) {
-            for (int r = lane; r < ni; r += 32) { d[r] = 1.0; rz[r] = -hrow(r); }
-            for (int i = lane; i < nq; i += 32) rxy[i] = i < nz ? pv[i] : 0.0;      // ry = -b = 0
+            TFOR(r, ni) { d[r] = 1.0; rz[r] = -hrow(r); }
+            TFOR(i, nq) rxy[i] = i < nz ? pv[i] : 0.0;      // ry = -b = 0
         } else {
             // residuals (batch.py:117-131)
             double nrx = 0.0, nry = 0.0, nrz = 0.0;
             sz = 0.0;
-            for (int I = lane; I < nq; I += 32) {
+            TFOR(I, nq) {
                 double acc;
                 if (I < nz) {
                     const int b = I / 6, k = I % 6;
@@ -429,7 +506,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
                     const double ay = fp < 0 ? xy[nz + (-fp - 1)] : 0.0;
                     double qx = 0.0;
                     for (int j = 0; j < 6; ++j) qx += xy[6 * b + j] * c.Qb[36 * b + 6 * k + j];
-                    acc = ay + Gtw_row(c, z, I, fd) + qx + pv[I];
+                    acc = ay + Gtw_row(c, z, I) + qx + pv[I];
                     nrx += acc * acc;
                 } else {
                     const int m = I - nz;
@@ -438,26 +515,26 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
                 }
                 rxy[I] = acc;
             }
-            Gx_all(c, xy, c.vec(DV_T));
-            for (int r = lane; r < ni; r += 32) {
-                const double val_ = c.vec(DV_T)[r] + s[r] - hrow(r) - Fz_row(c, z, mu, r, fd);
+            Gx_all<Team>(c, xy, c.vec(DV_T));
+            TFOR(r, ni) {
+                const double val_ = c.vec(DV_T)[r] + s[r] - hrow(r) - Fz_row(c, z, r, fd);
                 rz[r] = val_;
                 nrz += val_ * val_;
                 sz += s[r] * z[r];
             }
-            nrx = wsum(nrx); nry = wsum(nry); nrz = wsum(nrz); sz = wsum(sz);
+            nrx = Team::sum(nrx); nry = Team::sum(nry); nrz = Team::sum(nrz); sz = Team::sum(sz);
             mu_gap = fabs(sz / ni);
             res = (L.neq > 0 ? sqrt(nry) : 0.0) + sqrt(nrz) + sqrt(nrx) + ni * mu_gap;
-            for (int r = lane; r < ni; r += 32) d[r] = z[r] / s[r];
+            TFOR(r, ni) d[r] = z[r] / s[r];
         }
-        __syncwarp();
-        if (dyn_factor(c, d, mu, fd)) { status |= DSDF_LCP_FACTOR_FAIL; if (it >= 0) break; }
+        Team::sync();
+        if (dyn_factor<Team>(c, d, fd)) { status |= DSDF_LCP_FACTOR_FAIL; if (it >= 0) break; }
         if (it >= 0) {
             iters = it + 1;
             if (!have_best || res < best_res) {
                 have_best = true; best_res = res; stalled = 0;
-                for (int i = lane; i < nq; i += 32) bxy[i] = xy[i];
-                for (int r = lane; r < ni; r += 32) {        // best (lam, s) go straight to the outputs (reference row order)
+                TFOR(i, nq) bxy[i] = xy[i];
+                TFOR(r, ni) {        // best (lam, s) go straight to the outputs (reference row order)
                     const int rr = ref_row(r / per, r % per, c.nc, fd);
                     lamo[(size_t)w * niCap + rr] = z[r];
                     so[(size_t)w * niCap + rr] = s[r];
@@ -476,60 +553,61 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
             double* o_xy = pass == 0 ? (it < 0 ? xy : dxya) : dxy;
             double* o_s = pass == 0 ? (it < 0 ? s : dsa) : ds;
             double* o_z = pass == 0 ? (it < 0 ? z : dza) : dz;
-            dyn_solve(c, d, mu, fd, a_rxy, a_rs, a_rz, o_xy, o_s, o_z);
+            dyn_solve<Team>(c, d, fd, a_rxy, a_rs, a_rz, o_xy, o_s, o_z);
             if (it < 0) {
                 if (ni > 0) {                                   // batch.py:100-110
                     double ms = INFINITY, mz = INFINITY;
-                    for (int r = lane; r < ni; r += 32) { ms = fmin(ms, s[r]); mz = fmin(mz, z[r]); }
-                    ms = warp_min(ms); mz = warp_min(mz);
-                    for (int r = lane; r < ni; r += 32) {
+                    TFOR(r, ni) { ms = fmin(ms, s[r]); mz = fmin(mz, z[r]); }
+                    ms = Team::min(ms); mz = Team::min(mz);
+                    TFOR(r, ni) {
                         if (ms < 0.0) s[r] -= ms - 1.0;
                         if (mz < 0.0) z[r] -= mz - 1.0;
                     }
-                    __syncwarp();
+                    Team::sync();
                 }
                 init_done = true;
                 break;
             }
             if (pass == 0) {
-                double alpha = fmin(fmin(dyn_ratio_step(c, z, dza), dyn_ratio_step(c, s, dsa)), 1.0);
+                double alpha = fmin(fmin(dyn_ratio_step<Team>(c, z, dza), dyn_ratio_step<Team>(c, s, dsa)), 1.0);
                 double t3 = 0.0;
-                for (int r = lane; r < ni; r += 32) t3 += (s[r] + alpha * dsa[r]) * (z[r] + alpha * dza[r]);
-                t3 = wsum(t3);
+                TFOR(r, ni) t3 += (s[r] + alpha * dsa[r]) * (z[r] + alpha * dza[r]);
+                t3 = Team::sum(t3);
                 const double r3 = t3 / sz, sig = r3 * r3 * r3;
                 // corrector: rs = (-mu sig + dsa dza) / s  (stored in rz, which is free now)
-                for (int r = lane; r < ni; r += 32) rz[r] = (-mu_gap * sig + dsa[r] * dza[r]) / s[r];
-                __syncwarp();
+                TFOR(r, ni) rz[r] = (-mu_gap * sig + dsa[r] * dza[r]) / s[r];
+                Team::sync();
             }
         }
         if (init_done) {
             if (ni == 0) {                                      // no contacts: the equality-constrained solve is the answer
-                for (int i = lane; i < nq; i += 32) bxy[i] = xy[i];
+                TFOR(i, nq) bxy[i] = xy[i];
                 have_best = true;
                 break;
             }
             continue;
         }
-        for (int i = lane; i < nq; i += 32) dxy[i] += dxya[i];
-        for (int r = lane; r < ni; r += 32) { ds[r] += dsa[r]; dz[r] += dza[r]; }
-        __syncwarp();
-        const double alpha = fmin(0.999 * fmin(dyn_ratio_step(c, z, dz), dyn_ratio_step(c, s, ds)), 1.0);
-        for (int i = lane; i < nq; i += 32) xy[i] += alpha * dxy[i];
-        for (int r = lane; r < ni; r += 32) { s[r] += alpha * ds[r]; z[r] += alpha * dz[r]; }
-        __syncwarp();
+        TFOR(i, nq) dxy[i] += dxya[i];
+        TFOR(r, ni) { ds[r] += dsa[r]; dz[r] += dza[r]; }
+        Team::sync();
+        const double alpha = fmin(0.999 * fmin(dyn_ratio_step<Team>(c, z, dz), dyn_ratio_step<Team>(c, s, ds)), 1.0);
+        TFOR(i, nq) xy[i] += alpha * dxy[i];
+        TFOR(r, ni) { s[r] += alpha * ds[r]; z[r] += alpha * dz[r]; }
+        Team::sync();
     }
     if (ni > 0 && have_best && best_res > 1.0) status |= DSDF_LCP_INACCURATE;
-    __syncwarp();
-    for (int i = lane; i < nz; i += 32) {
+    Team::sync();
+    TFOR(i, nz) {
         xo[(size_t)w * nz + i] = have_best ? bxy[i] : NAN;
         if (nvo) nvo[(size_t)w * nz + i] = have_best ? -bxy[i] : NAN;       // engines.py:81-82
     }
-    for (int m = lane; m < L.neq; m += 32) nuo[(size_t)w * L.neq + m] = have_best ? bxy[nz + m] : NAN;
-    if (lane == 0) { status_o[w] = status; if (iters_o) iters_o[w] = iters; }
+    TFOR(m, L.neq) nuo[(size_t)w * L.neq + m] = have_best ? bxy[nz + m] : NAN;
+    if (Team::rank() == 0) { status_o[w] = status; if (iters_o) iters_o[w] = iters; }
 }
 
 // ---- backward: implicit differentiation at the solution, contracted straight onto the physical inputs ---------
-__global__ void __launch_bounds__(32, 10)
+template <class Team>
+__global__ void __launch_bounds__(Team::kThreads, Team::kBwdMinBlocks)
 dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, const double* __restrict__ mass,
                     const double* __restrict__ Ibody, const double* __restrict__ fric, const double* __restrict__ rest,
                     const double* __restrict__ f, const double* __restrict__ dt, const unsigned char* __restrict__ active,
@@ -540,68 +618,65 @@ dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, 
                     const double* __restrict__ gnv,
                     double* __restrict__ gp, double* __restrict__ gv, double* __restrict__ gmass, double* __restrict__ gI,
                     double* __restrict__ gfric, double* __restrict__ grest, double* __restrict__ gf,
-                    double* __restrict__ gdt, double* __restrict__ ggeo, int cmin, int last_class) {
+                    double* __restrict__ gdt, double* __restrict__ ggeo, int cmin, int last_class,
+                    double* __restrict__ work) {
     extern __shared__ double smd[];
-    const int w = blockIdx.x, lane = threadIdx.x & 31;
-    const DynSmem L = dyn_layout(nb, neq, C, fd);
-    DynCtx c = dyn_ctx(smd, L);
+    const int w = blockIdx.x;
+    const DynLayout L = dyn_layout(nb, neq, C, fd);
     const int nz = L.nz, nq = L.nq, per = L.per, niCap = maxc * per;
     const bool masked = active && !active[w];
     // contact-count classes (see dyn_forward_kernel): masked worlds are written by the first-class launch only
     if (masked ? cmin >= 0 : (count[w] <= cmin || (count[w] > C && !last_class))) return;
     const bool on = !masked && count[w] <= C;
     if (!on) {
-        for (int i = lane; i < nb * 7; i += 32) gp[(size_t)w * nb * 7 + i] = 0.0;
-        for (int i = lane; i < nz; i += 32) {               // inactive world: new_v = v
+        TFOR(i, nb * 7) gp[(size_t)w * nb * 7 + i] = 0.0;
+        TFOR(i, nz) {                                       // inactive world: new_v = v
             gv[(size_t)w * nz + i] = masked ? gnv[(size_t)w * nz + i] : 0.0;
             gf[(size_t)w * nz + i] = 0.0;
         }
-        for (int i = lane; i < nb; i += 32) {
-            gmass[(size_t)w * nb + i] = 0.0; gfric[(size_t)w * nb + i] = 0.0; grest[(size_t)w * nb + i] = 0.0;
-        }
-        for (int i = lane; i < nb * 9; i += 32) gI[(size_t)w * nb * 9 + i] = 0.0;
-        for (int i = lane; i < maxc * 10; i += 32) ggeo[(size_t)w * maxc * 10 + i] = 0.0;
-        if (lane == 0) gdt[w] = 0.0;
+        TFOR(i, nb) { gmass[(size_t)w * nb + i] = 0.0; gfric[(size_t)w * nb + i] = 0.0; grest[(size_t)w * nb + i] = 0.0; }
+        TFOR(i, nb * 9) gI[(size_t)w * nb * 9 + i] = 0.0;
+        TFOR(i, maxc * 10) ggeo[(size_t)w * maxc * 10 + i] = 0.0;
+        if (Team::rank() == 0) gdt[w] = 0.0;
         return;
     }
-    __shared__ double s_mu[64], s_e[64], s_h[64];
+    DynCtx c = dyn_ctx(smd, Team::kContactsInSmem ? smd + L.body : work + (size_t)w * L.contact, L);
     const double dtw = dt[w];
-    dyn_load(c, w, p, v, mass, Ibody, fric, rest, f, dtw, count, cbody, cgeo, eq_rows, maxc, fd, s_mu, s_e, s_h);
+    dyn_load<Team>(c, w, p, v, mass, Ibody, fric, rest, f, dtw, count, cbody, cgeo, eq_rows, maxc, fd);
     const int ni = c.ni, nc = c.nc;
     const double* vw = v + (size_t)w * nz;
     double *lam = c.vec(DV_Z), *d = c.vec(DV_D), *dl = c.vec(DV_DZ), *ds = c.vec(DV_DS);
     double *g = c.sv(DS_RXY), *dxy = c.sv(DS_DXY), *zh = c.sv(DS_XY);
-    for (int i = lane; i < nq; i += 32) { g[i] = i < nz ? -gnv[(size_t)w * nz + i] : 0.0; zh[i] = i < nz ? xs[(size_t)w * nz + i] : 0.0; }
-    for (int r = lane; r < ni; r += 32) {
+    TFOR(i, nq) { g[i] = i < nz ? -gnv[(size_t)w * nz + i] : 0.0; zh[i] = i < nz ? xs[(size_t)w * nz + i] : 0.0; }
+    TFOR(r, ni) {
         const int rr = ref_row(r / per, r % per, nc, fd);
         lam[r] = lams[(size_t)w * niCap + rr];
         d[r] = fmax(lam[r], 1e-8) / fmax(ss[(size_t)w * niCap + rr], 1e-8);
     }
-    __syncwarp();
-    dyn_factor(c, d, s_mu, fd);
-    dyn_solve(c, d, s_mu, fd, g, nullptr, nullptr, dxy, ds, dl);      // dx = dxy[:nz], dlam = dl
+    Team::sync();
+    dyn_factor<Team>(c, d, fd);
+    dyn_solve<Team>(c, d, fd, g, nullptr, nullptr, dxy, ds, dl);      // dx = dxy[:nz], dlam = dl
     // ---- dp (= du), dh, and the outer-product gradients, contracted on the fly
     // gv = M' du + Jc' (e o dh),  dh = -dlam ; gf = dt du ; gdt = f . du
-    for (int I = lane; I < nz; I += 32) {
+    TFOR(I, nz) {
         const int b = I / 6, k = I % 6;
         double acc = 0.0;
         for (int i = 0; i < 6; ++i) acc += c.Qb[36 * b + 6 * i + k] * dxy[6 * b + i];
-        for (int cc = 0; cc < nc; ++cc) {
-            int kk;
-            if (c.cb[2 * cc] == b) kk = k; else if (c.cb[2 * cc + 1] == b) kk = 6 + k; else continue;
-            acc += c.G[(size_t)cc * L.gs + kk] * s_e[cc] * (-dl[cc * per]);
+        for (int t = c.bstart[b]; t < c.bstart[b + 1]; ++t) {
+            const int cc = c.blist[t] >> 1, kk = (c.blist[t] & 1) * 6 + k;
+            acc += c.G[(size_t)cc * L.gs + kk] * c.e[cc] * (-dl[cc * per]);
         }
         gv[(size_t)w * nz + I] = acc;
         gf[(size_t)w * nz + I] = dtw * dxy[I];
     }
     {
         double acc = 0.0;
-        for (int I = lane; I < nz; I += 32) acc += f[(size_t)w * nz + I] * dxy[I];
-        acc = wsum(acc);
-        if (lane == 0) gdt[w] = acc;
+        TFOR(I, nz) acc += f[(size_t)w * nz + I] * dxy[I];
+        acc = Team::sum(acc);
+        if (Team::rank() == 0) gdt[w] = acc;
     }
     // per body: dM = dQ + du v' with dQ = 1/2 (dx z' + z dx')
-    for (int b = lane; b < nb; b += 32) {
+    TFOR(b, nb) {
         double dMb[36];
         for (int i = 0; i < 6; ++i)
             for (int j = 0; j < 6; ++j)
@@ -622,9 +697,11 @@ dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, 
             else gI[((size_t)w * nb + b) * 9 + seed - 4] = acc;
         }
         gp[((size_t)w * nb + b) * 7 + 4] = 0.0; gp[((size_t)w * nb + b) * 7 + 5] = 0.0; gp[((size_t)w * nb + b) * 7 + 6] = 0.0;
+    }
+    TFOR(b, nb) {                        // a pass of its own: keeps the one-warp loop above free of spills
         double gfr = 0.0, gre = 0.0;
-        for (int cc = 0; cc < nc; ++cc) {
-            if (c.cb[2 * cc] != b && c.cb[2 * cc + 1] != b) continue;
+        for (int t = c.bstart[b]; t < c.bstart[b + 1]; ++t) {
+            const int cc = c.blist[t] >> 1;
             // dF[cone row, normal col] = dlam_cone * lam_normal
             gfr += 0.5 * dl[cc * per + per - 1] * lam[cc * per];
             double jv = 0.0;
@@ -635,7 +712,7 @@ dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, 
         grest[(size_t)w * nb + b] = gre;
     }
     // contact geometry: dG row = dlam_r z' + lam_r dx'  (+ dh e v' on normal rows)
-    for (int t = lane; t < maxc * 10; t += 32) {
+    TFOR(t, maxc * 10) {
         const int cc = t / 10, comp = t % 10;
         double acc = 0.0;
         if (cc < nc && comp < 9) {
@@ -648,7 +725,7 @@ dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, 
                 const double dlr = dl[cc * per], lr = lam[cc * per], dh = -dlr;
                 for (int k = 0; k < 12; ++k) {
                     const int I = c.gidx(cc, k);
-                    acc += (dlr * zh[I] + lr * dxy[I] + dh * s_e[cc] * vw[I]) * row[k].d;
+                    acc += (dlr * zh[I] + lr * dxy[I] + dh * c.e[cc] * vw[I]) * row[k].d;
                 }
             }
             if (!stop_friction_grad) {
@@ -672,22 +749,78 @@ dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, 
 
 using namespace dsdf;
 
-extern "C" {
-
-size_t dsdf_dynamics_solve_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs) {
-    return dyn_layout(nb, neq, ncontacts, fric_dirs).bytes;
-}
-
-static int dyn_check(int W, int nb, int neq, int maxc, int* C, int fd, size_t* smem) {
-    if (W <= 0 || nb <= 0 || neq < 0 || maxc <= 0 || (fd != 8 && fd != 4)) return -1;
+// Argument checks of both launchers: clamps *C to maxc and returns the launch's dynamic shared memory in *smem.
+// The one-warp kernel takes at most 64 contacts per world; more go to the one-CTA kernel, which needs a workspace.
+template <class Team> static int dyn_check(int W, int nb, int neq, int maxc, int* C, int fd, const double* work,
+                                           size_t* smem) {
+    if (W <= 0 || nb <= 0 || neq < 0 || maxc <= 0 || (fd != 8 && fd != 4) || (!Team::kContactsInSmem && !work))
+        return -1;
     if (*C <= 0 || *C > maxc) *C = maxc;
-    if (*C > 64) return -2;
-    *smem = dyn_layout(nb, neq, *C, fd).bytes;
+    if (Team::kContactsInSmem && *C > 64) return -2;
+    const DynLayout L = dyn_layout(nb, neq, *C, fd);
+    *smem = (L.body + (Team::kContactsInSmem ? L.contact : 0)) * sizeof(double);
     if (*smem > 227 * 1024) return -2;
     return 0;
 }
 
-static size_t g_fwd_smem = 0, g_bwd_smem = 0;
+template <class Team>
+static int dyn_launch_forward(const double* p, const double* v, const double* mass, const double* Ibody,
+                              const double* fric, const double* rest, const double* f, const double* dt,
+                              const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
+                              const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts, int fric_dirs,
+                              double eps, int not_improved_lim, int max_iter,
+                              double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status,
+                              int32_t* iters, const int32_t* vmap, int32_t* ctrl, int count_min, int last_class,
+                              double* work, void* stream) {
+    static size_t granted = 0;
+    size_t smem;
+    int C = ncontacts;
+    int rc = dyn_check<Team>(W, nb, neq, maxc, &C, fric_dirs, work, &smem);
+    if (rc) return rc;
+    cudaError_t e = ensure_smem(dyn_forward_kernel<Team>, smem, &granted);
+    if (e != cudaSuccess) return (int)e;
+    dyn_forward_kernel<Team><<<W, Team::kThreads, smem, (cudaStream_t)stream>>>(
+        p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, nb, neq, maxc, C, fric_dirs, eps,
+        not_improved_lim, max_iter, x, new_v, nu, lam, s, status, iters, vmap, ctrl, count_min, last_class, work);
+    return (int)cudaGetLastError();
+}
+
+template <class Team>
+static int dyn_launch_backward(const double* p, const double* v, const double* mass, const double* Ibody,
+                               const double* fric, const double* rest, const double* f, const double* dt,
+                               const unsigned char* active, const int32_t* count, const int32_t* cbody,
+                               const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
+                               int ncontacts, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
+                               const double* x, const double* lam, const double* s, const double* g_new_v,
+                               double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
+                               double* gf, double* gdt, double* ggeo, int count_min, int last_class,
+                               double* work, void* stream) {
+    static size_t granted = 0;
+    size_t smem;
+    int C = ncontacts;
+    int rc = dyn_check<Team>(W, nb, neq, maxc, &C, fric_dirs, work, &smem);
+    if (rc) return rc;
+    cudaError_t e = ensure_smem(dyn_backward_kernel<Team>, smem, &granted);
+    if (e != cudaSuccess) return (int)e;
+    dyn_backward_kernel<Team><<<W, Team::kThreads, smem, (cudaStream_t)stream>>>(
+        p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, nb, neq, maxc, C, fric_dirs,
+        stop_contact_grad, stop_friction_grad, x, lam, s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo,
+        count_min, last_class, work);
+    return (int)cudaGetLastError();
+}
+
+extern "C" {
+
+size_t dsdf_dynamics_solve_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs) {
+    const DynLayout L = dyn_layout(nb, neq, ncontacts, fric_dirs);
+    return (L.body + L.contact) * sizeof(double);
+}
+size_t dsdf_dynamics_big_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs) {
+    return dyn_layout(nb, neq, ncontacts, fric_dirs).body * sizeof(double);
+}
+size_t dsdf_dynamics_big_workspace_bytes(int W, int nb, int neq, int ncontacts, int fric_dirs) {
+    return (size_t)W * dyn_layout(nb, neq, ncontacts, fric_dirs).contact * sizeof(double);
+}
 
 int dsdf_dynamics_solve_loop(const double* p, const double* v, const double* mass, const double* Ibody,
                              const double* fric, const double* rest, const double* f, const double* dt,
@@ -696,17 +829,9 @@ int dsdf_dynamics_solve_loop(const double* p, const double* v, const double* mas
                              double eps, int not_improved_lim, int max_iter,
                              double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
                              const int32_t* vmap, int32_t* ctrl, int count_min, int last_class, void* stream) {
-    size_t smem;
-    int C = ncontacts_smem;
-    int rc = dyn_check(W, nb, neq, maxc, &C, fric_dirs, &smem);
-    if (rc) return rc;
-    cudaError_t e = ensure_smem(dyn_forward_kernel, smem, &g_fwd_smem);
-    if (e != cudaSuccess) return (int)e;
-    dyn_forward_kernel<<<W, 32, smem, (cudaStream_t)stream>>>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody,
-                                                              cgeo, eq_rows, nb, neq, maxc, C, fric_dirs, eps,
-                                                              not_improved_lim, max_iter, x, new_v, nu, lam, s, status, iters,
-                                                              vmap, ctrl, count_min, last_class);
-    return (int)cudaGetLastError();
+    return dyn_launch_forward<WarpTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
+                                        neq, maxc, ncontacts_smem, fric_dirs, eps, not_improved_lim, max_iter, x, new_v,
+                                        nu, lam, s, status, iters, vmap, ctrl, count_min, last_class, nullptr, stream);
 }
 
 int dsdf_dynamics_solve(const double* p, const double* v, const double* mass, const double* Ibody,
@@ -721,6 +846,19 @@ int dsdf_dynamics_solve(const double* p, const double* v, const double* mass, co
                                     status, iters, nullptr, nullptr, -1, 1, stream);
 }
 
+int dsdf_dynamics_big_solve(const double* p, const double* v, const double* mass, const double* Ibody,
+                            const double* fric, const double* rest, const double* f, const double* dt,
+                            const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
+                            const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts, int fric_dirs,
+                            double eps, int not_improved_lim, int max_iter,
+                            double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
+                            const int32_t* vmap, int32_t* ctrl, int count_min, int last_class, double* workspace,
+                            void* stream) {
+    return dyn_launch_forward<CtaTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
+                                       neq, maxc, ncontacts, fric_dirs, eps, not_improved_lim, max_iter, x, new_v, nu,
+                                       lam, s, status, iters, vmap, ctrl, count_min, last_class, workspace, stream);
+}
+
 int dsdf_dynamics_solve_backward_loop(const double* p, const double* v, const double* mass, const double* Ibody,
                                       const double* fric, const double* rest, const double* f, const double* dt,
                                       const unsigned char* active, const int32_t* count, const int32_t* cbody,
@@ -729,18 +867,10 @@ int dsdf_dynamics_solve_backward_loop(const double* p, const double* v, const do
                                       const double* x, const double* lam, const double* s, const double* g_new_v,
                                       double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
                                       double* gf, double* gdt, double* ggeo, int count_min, int last_class, void* stream) {
-    size_t smem;
-    int C = ncontacts_smem;
-    int rc = dyn_check(W, nb, neq, maxc, &C, fric_dirs, &smem);
-    if (rc) return rc;
-    cudaError_t e = ensure_smem(dyn_backward_kernel, smem, &g_bwd_smem);
-    if (e != cudaSuccess) return (int)e;
-    dyn_backward_kernel<<<W, 32, smem, (cudaStream_t)stream>>>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody,
-                                                               cgeo, eq_rows, nb, neq, maxc, C, fric_dirs,
-                                                               stop_contact_grad, stop_friction_grad, x, lam, s, g_new_v, gp,
-                                                               gv, gmass, gI, gfric, grest, gf, gdt, ggeo, count_min,
-                                                               last_class);
-    return (int)cudaGetLastError();
+    return dyn_launch_backward<WarpTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
+                                         neq, maxc, ncontacts_smem, fric_dirs, stop_contact_grad, stop_friction_grad, x,
+                                         lam, s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, count_min,
+                                         last_class, nullptr, stream);
 }
 
 int dsdf_dynamics_solve_backward(const double* p, const double* v, const double* mass, const double* Ibody,
@@ -755,6 +885,21 @@ int dsdf_dynamics_solve_backward(const double* p, const double* v, const double*
                                              nb, neq, maxc, ncontacts_smem, fric_dirs, stop_contact_grad,
                                              stop_friction_grad, x, lam, s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf,
                                              gdt, ggeo, -1, 1, stream);
+}
+
+int dsdf_dynamics_big_solve_backward(const double* p, const double* v, const double* mass, const double* Ibody,
+                                     const double* fric, const double* rest, const double* f, const double* dt,
+                                     const unsigned char* active, const int32_t* count, const int32_t* cbody,
+                                     const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
+                                     int ncontacts, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
+                                     const double* x, const double* lam, const double* s, const double* g_new_v,
+                                     double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
+                                     double* gf, double* gdt, double* ggeo, int count_min, int last_class,
+                                     double* workspace, void* stream) {
+    return dyn_launch_backward<CtaTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
+                                        neq, maxc, ncontacts, fric_dirs, stop_contact_grad, stop_friction_grad, x, lam,
+                                        s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, count_min,
+                                        last_class, workspace, stream);
 }
 
 }  // extern "C"

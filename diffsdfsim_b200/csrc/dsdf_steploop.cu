@@ -314,7 +314,7 @@ int dsdf_step_rounds(const dsdf_step_args* a, int n_rounds, int ncontacts_small,
         { PhaseTimer t(PHASE_PREP, st); step_prep_kernel<<<(W + 255) / 256, 256, 0, st>>>(*a); }
         PhaseTimer* td = new PhaseTimer(PHASE_DYN, st);
         // contact-count classes: worlds with <= ncontacts_small contacts, and (if any) the rest; worlds with many bodies,
-        // or more contacts than the one-warp kernel holds, go to the one-CTA kernel (dsdf_dynsolve_big.cu)
+        // or more contacts than the one-warp kernel holds, go to the one-CTA kernel (dsdf_dynsolve.cu, CtaTeam)
         int rc = 0;
         auto warp_class = [&](int C, int cmin, int last) {
             return dsdf_dynamics_solve_loop(a->p, a->v, a->mass, a->Ibody, a->fric, a->rest, a->f, a->dt_used_v, nullptr,

@@ -361,7 +361,7 @@ def mixed16_floor(seed=0, steps=6, spacing=1.5, floor=(8.0, 1.0, 8.0), floor_tri
     pinned floor slab (4 x 4 layout, ``gap`` above it), gravity on, small random drift.  Boxes rest on 4 + 4 corner
     contacts, lying cylinders on line contacts, spheres on point contacts: ~80-100 simultaneous contacts per world
     (nz = 102, 6 equality rows) -- beyond the 64-contact cap of the one-warp dynamics kernel, so this scene runs on
-    dsdf_dynsolve_big.cu.  Body 0 is the floor; per-world masses / velocities via 'mass_all' / 'vel_all' (17 rows)."""
+    the one-CTA kernel of dsdf_dynsolve.cu.  Body 0 is the floor; per-world masses / velocities via 'mass_all' / 'vel_all' (17 rows)."""
     rng = np.random.RandomState(seed)
     bodies = [body('box', [0, -floor[1] / 2, 0], dims=list(floor), pinned=True, fric_coeff=0.3, restitution=0.2,
                    max_tri_length=floor_tri)]

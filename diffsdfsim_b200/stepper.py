@@ -218,7 +218,7 @@ class DeviceStepper:
         self.iters_v = torch.zeros(V, dtype=I32, device=dev)
         self.cs_v = ContactSet(V, self.maxc, dev)
         # dynamics kernel selection (csrc/dsdf_dynsolve.cu: one warp per world, <= 64 contacts, small worlds;
-        # csrc/dsdf_dynsolve_big.cu: one CTA per world, any contact count, up to ~120 free velocity components)
+        # or one CTA per world, any contact count, up to ~120 free velocity components)
         L = _lib.lib()
         neq, fd = world.num_constraints, world.fric_dirs
         warp_fits = L.dsdf_dynamics_solve_smem_bytes(nb, neq, 16, fd) <= 48 * 1024

@@ -275,7 +275,7 @@ int dsdf_dynamics_solve_backward(const double* p, const double* v, const double*
  * what scales with the bodies (free block of the reduced KKT matrix, <= ~120 free velocity components), a caller-provided
  * global workspace of dsdf_dynamics_big_workspace_bytes(W, ...) bytes holds what scales with the contacts (no cap on
  * their number), per-body contact lists exploit the body-pair block sparsity of G Q^-1 G'.  Same arguments and semantics
- * as dsdf_dynamics_solve_loop / dsdf_dynamics_solve_backward_loop (csrc/dsdf_dynsolve_big.cu). */
+ * as dsdf_dynamics_solve_loop / dsdf_dynamics_solve_backward_loop (csrc/dsdf_dynsolve.cu, CtaTeam instantiation). */
 size_t dsdf_dynamics_big_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs);
 size_t dsdf_dynamics_big_workspace_bytes(int W, int nb, int neq, int ncontacts, int fric_dirs);
 int dsdf_dynamics_big_solve(const double* p, const double* v, const double* mass, const double* Ibody,

@@ -49,8 +49,9 @@ def test_fused_engine_has_no_contact_limit_of_the_dense_kernel():
 
 
 def test_one_cta_kernel_matches_one_warp_kernel():
-    """dsdf_dynsolve_big.cu (one CTA per world, per-contact data in a global workspace, per-body contact lists) solves
-    the same Newton systems as the one-warp kernel: identical attempts / contact sets, states and gradients to round-off."""
+    """The one-CTA instantiation of the solver (per-contact data in a global workspace, block-wide reductions and LU)
+    solves the same Newton systems as the one-warp kernel: identical attempts / contact sets, states and gradients to
+    round-off."""
     from diffsdfsim_b200.stepper import DeviceStepper
     steps, W = 8, 16
     ta, ga, wa = _rollout('PdipmEngine', steps, W)
