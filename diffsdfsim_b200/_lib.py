@@ -21,35 +21,23 @@ SIGNATURES = {
     'dsdf_lcp_smem_bytes': (c_sz, [c_i, c_i, c_i]),
     'dsdf_lcp_forward': (c_i, [c_p] * 8 + [c_i] * 5 + [c_d, c_i, c_i, c_i] + [c_p] * 8),
     'dsdf_lcp_backward': (c_i, [c_p] * 10 + [c_i] * 5 + [c_p] * 10),
-    'dsdf_sdf_query': (c_i, [c_i, c_p, c_p, c_i, c_ll, c_p, c_i, c_i, c_i, c_p, c_p, c_p]),
-    'dsdf_sdf_query_backward': (c_i, [c_i, c_p, c_p, c_i, c_ll, c_p, c_i, c_i, c_p, c_p, c_p, c_p]),
-    'dsdf_sdf_query_ex': (c_i, [c_i, c_p, c_d, c_d, c_p, c_i, c_ll, c_p, c_i, c_i, c_i, c_p, c_p, c_p]),
-    'dsdf_sdf_query_backward_ex': (c_i, [c_i, c_p, c_d, c_d, c_p, c_i, c_ll, c_p, c_i, c_i, c_p, c_p, c_p, c_p]),
+    'dsdf_sdf_query': (c_i, [c_i, c_p, c_d, c_d, c_p, c_i, c_ll, c_p, c_i, c_i, c_i, c_p, c_p, c_p]),
+    'dsdf_sdf_query_backward': (c_i, [c_i, c_p, c_d, c_d, c_p, c_i, c_ll, c_p, c_i, c_i, c_p, c_p, c_p, c_p]),
     'dsdf_integrate': (c_i, [c_p, c_p, c_p, c_p, c_i, c_i, c_p, c_p]),
     'dsdf_integrate_backward': (c_i, [c_p, c_p, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p]),
     'dsdf_contacts_detect': (c_i, [c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_d, c_d, c_d, c_d, c_i, c_i, c_i]
-                             + [c_p] * 9),
+                             + [c_p] * 11),
     'dsdf_contacts_phase_cycles': (c_i, [c_p, c_i]),
     'dsdf_filter_contacts': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_p, c_p, c_p]),
-    'dsdf_contact_geometry_backward': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_i, c_i] + [c_p] * 7),
-    'dsdf_contact_geometry_backward_rows': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_i, c_i] + [c_p] * 8),
-    'dsdf_contact_geometry_backward_full': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_i, c_i] + [c_p] * 10),
+    'dsdf_contact_geometry_backward': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_i, c_i] + [c_p] * 10),
     'dsdf_dynamics_assemble': (c_i, [c_p] * 12 + [c_i] * 4 + [c_p] * 7),
     'dsdf_dynamics_assemble_backward': (c_i, [c_p] * 12 + [c_i] * 6 + [c_p] * 17),
-    'dsdf_dynamics_solve_smem_bytes': (c_sz, [c_i] * 4),
-    'dsdf_dynamics_solve': (c_i, [c_p] * 13 + [c_i] * 6 + [c_d, c_i, c_i] + [c_p] * 8),
-    'dsdf_dynamics_solve_backward': (c_i, [c_p] * 13 + [c_i] * 8 + [c_p] * 14),
+    'dsdf_dynamics_plan': (c_i, [c_i] * 7 + [c_p]),
+    'dsdf_dynamics_solve': (c_i, [c_p] * 13 + [c_i] * 8 + [c_d, c_i, c_i] + [c_p] * 11),
+    'dsdf_dynamics_solve_backward': (c_i, [c_p] * 13 + [c_i] * 10 + [c_p] * 15),
     'dsdf_toc_backward': (c_i, [c_i] * 3 + [c_p] * 9 + [c_d] + [c_p] * 7),
     'dsdf_contactset_move': (c_i, [c_i, c_i] + [c_p] * 16),
     'dsdf_attempt_commit': (c_i, [c_i] * 3 + [c_p] * 4 + [c_d, c_i, c_i] + [c_p] * 21),
-    'dsdf_dynamics_solve_loop': (c_i, [c_p] * 13 + [c_i] * 6 + [c_d, c_i, c_i] + [c_p] * 9 + [c_i, c_i, c_p]),
-    'dsdf_dynamics_solve_backward_loop': (c_i, [c_p] * 13 + [c_i] * 8 + [c_p] * 13 + [c_i, c_i, c_p]),
-    'dsdf_contacts_detect_loop': (c_i, [c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_d, c_d, c_d, c_d, c_i, c_i, c_i]
-                                  + [c_p] * 11),
-    'dsdf_dynamics_big_smem_bytes': (c_sz, [c_i] * 4),
-    'dsdf_dynamics_big_workspace_bytes': (c_sz, [c_i] * 5),
-    'dsdf_dynamics_big_solve': (c_i, [c_p] * 13 + [c_i] * 6 + [c_d, c_i, c_i] + [c_p] * 9 + [c_i, c_i, c_p, c_p]),
-    'dsdf_dynamics_big_solve_backward': (c_i, [c_p] * 13 + [c_i] * 8 + [c_p] * 13 + [c_i, c_i, c_p, c_p]),
     'dsdf_step_begin': (c_i, [c_p, c_p]),
     'dsdf_step_resume': (c_i, [c_p, c_p]),
     'dsdf_step_rounds': (c_i, [c_p, c_i, c_i, c_i, c_p]),
@@ -79,16 +67,8 @@ def lib():
     return _lib
 
 
-# CUDA kernels launched by one call of each entry point (for bench.py's gpu_launches claim)
-KERNELS_PER_CALL = {
-    'dsdf_lcp_forward': 1, 'dsdf_lcp_backward': 1, 'dsdf_sdf_query': 1, 'dsdf_sdf_query_backward': 1, 'dsdf_sdf_query_ex': 1, 'dsdf_sdf_query_backward_ex': 1,
-    'dsdf_integrate': 1, 'dsdf_integrate_backward': 1, 'dsdf_contacts_detect': 1,
-    'dsdf_contact_geometry_backward': 1, 'dsdf_dynamics_assemble': 1, 'dsdf_dynamics_assemble_backward': 1,
-    'dsdf_dynamics_solve': 1, 'dsdf_dynamics_solve_backward': 1, 'dsdf_attempt_commit': 1, 'dsdf_toc_backward': 1, 'dsdf_contactset_move': 1,
-    'dsdf_step_begin': 1, 'dsdf_step_resume': 1, 'dsdf_step_rounds': 0, 'dsdf_dynamics_solve_backward_loop': 1, 'dsdf_dynamics_big_solve': 1, 'dsdf_dynamics_big_solve_backward': 1, 'dsdf_contact_geometry_backward_rows': 1, 'dsdf_contact_geometry_backward_full': 1,      # rounds: counted by the stepper (5 per round)
-}
 PROFILE = None      # set to {} to record (start, end) CUDA events around every entry-point call
-LAUNCHES = {}       # name -> number of calls since reset_counters()
+LAUNCHES = {}       # name -> CUDA kernels its calls launched since reset_counters() (for bench.py's gpu_launches claim)
 
 
 def reset_counters(profile=False):
@@ -98,13 +78,14 @@ def reset_counters(profile=False):
 
 
 def kernel_launches():
-    return sum(KERNELS_PER_CALL.get(k, 1) * n for k, n in LAUNCHES.items())
+    return sum(LAUNCHES.values())
 
 
-def call(name, *args):
-    """Invoke an entry point of the library (counts launches; optionally brackets it with CUDA events)."""
+def call(name, *args, kernels=1):
+    """Invoke an entry point of the library that launches ``kernels`` CUDA kernels (counted; optionally bracketed with
+    CUDA events)."""
     fn = getattr(lib(), name)
-    LAUNCHES[name] = LAUNCHES.get(name, 0) + 1
+    LAUNCHES[name] = LAUNCHES.get(name, 0) + kernels
     if PROFILE is None:
         return fn(*args)
     s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -119,6 +100,18 @@ def profile_summary():
     """name -> (calls, total ms) from the recorded events (synchronises)."""
     torch.cuda.synchronize()
     return {k: (len(v), sum(s.elapsed_time(e) for s, e in v)) for k, v in (PROFILE or {}).items()}
+
+
+def dynamics_plan(W, nb, neq, fric_dirs, ncontacts_small, ncontacts_large, force_cta=False):
+    """(kernel launches, workspace bytes) of one dsdf_dynamics_solve / dsdf_dynamics_solve_backward call."""
+    ws = ctypes.c_size_t(0)
+    n = lib().dsdf_dynamics_plan(W, nb, neq, fric_dirs, ncontacts_small, ncontacts_large, int(force_cta),
+                                 ctypes.byref(ws))
+    if n == -2:
+        raise DsdfLibraryError('world too large for the dynamics kernels: %d bodies' % nb)
+    if n < 0:
+        raise DsdfLibraryError('dsdf_dynamics_plan failed with status %d' % n)
+    return n, ws.value
 
 
 def ptr(t):

@@ -219,7 +219,7 @@ class ContactDetector:
                        _lib.ptr(shape), _lib.ptr(active), out.W, self.nb, eps, tol, fd_eps, body_eps, int(detach_b2),
                        self.capK, self.maxc, _lib.ptr(out.count), _lib.ptr(out.body), _lib.ptr(out.face),
                        _lib.ptr(out.abc), _lib.ptr(out.geo), _lib.ptr(out.status), _lib.ptr(out.pre_ids),
-                       _lib.ptr(out.pre_cnt), _lib.stream())
+                       _lib.ptr(out.pre_cnt), None, None, _lib.stream())
         _lib.check(rc, 'dsdf_contacts_detect')
         return out
 
@@ -233,7 +233,7 @@ def geometry_vjp(table, p, shape, count, body, face, abc, ggeo, fd_eps, detach_b
     gshape = torch.empty(R, nb, 4, dtype=F64, device=p.device) if want_shape else None
     gctri = torch.empty(R, maxc, 3, dtype=F64, device=p.device) if want_shape else None
     ggeo = ggeo.contiguous()
-    rc = _lib.call('dsdf_contact_geometry_backward_full', table.ptr(), _lib.ptr(p), _lib.ptr(shape), R, nb, fd_eps,
+    rc = _lib.call('dsdf_contact_geometry_backward', table.ptr(), _lib.ptr(p), _lib.ptr(shape), R, nb, fd_eps,
                    int(detach_b2), maxc, _lib.ptr(count), _lib.ptr(body), _lib.ptr(face), _lib.ptr(abc), _lib.ptr(ggeo),
                    _lib.ptr(gp), _lib.ptr(wmap), _lib.ptr(gshape), _lib.ptr(gctri), _lib.stream())
     _lib.check(rc, 'dsdf_contact_geometry_backward')

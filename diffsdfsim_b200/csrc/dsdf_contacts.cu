@@ -1281,12 +1281,12 @@ extern "C" {
 
 static size_t g_contacts_smem = 0, g_filter_smem = 0;
 
-int dsdf_contacts_detect_loop(const dsdf_body_geom* geom, const int32_t* pairs, int npairs, const double* p,
-                              const double* shape, const unsigned char* active,
-                              int W, int nb, double eps, double tol, double fd_eps, double body_eps, int detach_b2,
-                              int capK, int maxc, int32_t* count, int32_t* cbody, int32_t* cface, double* cabc, double* cgeo,
-                              int32_t* wstatus, int32_t* pre_ids, int32_t* pre_cnt, const int32_t* vmap, const int32_t* ctrl,
-                              void* stream) {
+int dsdf_contacts_detect(const dsdf_body_geom* geom, const int32_t* pairs, int npairs, const double* p,
+                         const double* shape, const unsigned char* active,
+                         int W, int nb, double eps, double tol, double fd_eps, double body_eps, int detach_b2,
+                         int capK, int maxc, int32_t* count, int32_t* cbody, int32_t* cface, double* cabc, double* cgeo,
+                         int32_t* wstatus, int32_t* pre_ids, int32_t* pre_cnt, const int32_t* vmap, const int32_t* ctrl,
+                         void* stream) {
     if (W <= 0 || nb <= 0 || npairs < 0 || capK < 32 || capK > 1024 || (capK & 3) || maxc <= 0) return -1;
     static_assert(sizeof(BodyGeom) == sizeof(dsdf_body_geom), "BodyGeom must mirror dsdf_body_geom");
     cudaStream_t st = (cudaStream_t)stream;
@@ -1298,16 +1298,6 @@ int dsdf_contacts_detect_loop(const dsdf_body_geom* geom, const int32_t* pairs, 
                                           eps, tol, fd_eps, body_eps, detach_b2, capK, maxc, count, cbody, cface, cabc,
                                           cgeo, wstatus, pre_ids, pre_cnt, vmap, ctrl);
     return (int)cudaGetLastError();
-}
-
-int dsdf_contacts_detect(const dsdf_body_geom* geom, const int32_t* pairs, int npairs, const double* p,
-                         const double* shape, const unsigned char* active,
-                         int W, int nb, double eps, double tol, double fd_eps, double body_eps, int detach_b2,
-                         int capK, int maxc, int32_t* count, int32_t* cbody, int32_t* cface, double* cabc, double* cgeo,
-                         int32_t* wstatus, int32_t* pre_ids, int32_t* pre_cnt, void* stream) {
-    return dsdf_contacts_detect_loop(geom, pairs, npairs, p, shape, active, W, nb, eps, tol, fd_eps, body_eps, detach_b2,
-                                     capK, maxc, count, cbody, cface, cabc, cgeo, wstatus, pre_ids, pre_cnt, nullptr,
-                                     nullptr, stream);
 }
 
 int dsdf_filter_contacts(const double* normals, const double* p1, const int32_t* n, int W, int capK, double eps,

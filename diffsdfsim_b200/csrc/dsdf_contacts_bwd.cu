@@ -103,11 +103,10 @@ using namespace dsdf;
 
 extern "C" {
 
-int dsdf_contact_geometry_backward_full(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
-                                        double fd_eps, int detach_b2, int maxc, const int32_t* count,
-                                        const int32_t* cbody, const int32_t* cface, const double* cabc,
-                                        const double* ggeo, double* gp, const int32_t* wmap, double* gshape,
-                                        double* gctri, void* stream) {
+int dsdf_contact_geometry_backward(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
+                                   double fd_eps, int detach_b2, int maxc, const int32_t* count, const int32_t* cbody,
+                                   const int32_t* cface, const double* cabc, const double* ggeo, double* gp,
+                                   const int32_t* wmap, double* gshape, double* gctri, void* stream) {
     if (W <= 0 || nb <= 0 || maxc <= 0 || ((gshape == nullptr) != (gctri == nullptr))) return -1;
     const size_t smem = (size_t)maxc * (gshape ? GEO_ALL_SEEDS : GEO_POSE_SEEDS) * sizeof(double);
     static size_t granted = 0;
@@ -120,21 +119,6 @@ int dsdf_contact_geometry_backward_full(const dsdf_body_geom* geom, const double
                                                                     fd_eps, detach_b2, maxc, count, cbody, cface, cabc,
                                                                     ggeo, gp, wmap, gshape, gctri);
     return (int)cudaGetLastError();
-}
-
-int dsdf_contact_geometry_backward_rows(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
-                                        double fd_eps, int detach_b2, int maxc, const int32_t* count,
-                                        const int32_t* cbody, const int32_t* cface, const double* cabc,
-                                        const double* ggeo, double* gp, const int32_t* wmap, void* stream) {
-    return dsdf_contact_geometry_backward_full(geom, p, shape, W, nb, fd_eps, detach_b2, maxc, count, cbody, cface, cabc,
-                                               ggeo, gp, wmap, nullptr, nullptr, stream);
-}
-
-int dsdf_contact_geometry_backward(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
-                                   double fd_eps, int detach_b2, int maxc, const int32_t* count, const int32_t* cbody,
-                                   const int32_t* cface, const double* cabc, const double* ggeo, double* gp, void* stream) {
-    return dsdf_contact_geometry_backward_rows(geom, p, shape, W, nb, fd_eps, detach_b2, maxc, count, cbody, cface, cabc,
-                                               ggeo, gp, nullptr, stream);
 }
 
 }  // extern "C"

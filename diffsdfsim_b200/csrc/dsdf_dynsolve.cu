@@ -749,18 +749,51 @@ dyn_backward_kernel(const double* __restrict__ p, const double* __restrict__ v, 
 
 using namespace dsdf;
 
+// ---- host dispatch ---------------------------------------------------------------------------------------------
+// The one-warp kernel holds a whole world in shared memory: at most 64 contacts, and only for worlds whose layout at 16
+// contacts fits in 48 KB (several CTAs per SM).  Every other world runs on the one-CTA kernel.
+static constexpr int kWarpMaxContacts = 64;
+static constexpr size_t kWarpSmemBytes = 48 * 1024, kMaxSmemBytes = 227 * 1024;
+
+// dynamic shared memory of a launch sized for C contacts
+static size_t dyn_smem(bool contacts_in_smem, int nb, int neq, int C, int fd) {
+    const DynLayout L = dyn_layout(nb, neq, C, fd);
+    return (L.body + (contacts_in_smem ? L.contact : 0)) * sizeof(double);
+}
+
 // Argument checks of both launchers: clamps *C to maxc and returns the launch's dynamic shared memory in *smem.
-// The one-warp kernel takes at most 64 contacts per world; more go to the one-CTA kernel, which needs a workspace.
 template <class Team> static int dyn_check(int W, int nb, int neq, int maxc, int* C, int fd, const double* work,
                                            size_t* smem) {
     if (W <= 0 || nb <= 0 || neq < 0 || maxc <= 0 || (fd != 8 && fd != 4) || (!Team::kContactsInSmem && !work))
         return -1;
     if (*C <= 0 || *C > maxc) *C = maxc;
-    if (Team::kContactsInSmem && *C > 64) return -2;
-    const DynLayout L = dyn_layout(nb, neq, *C, fd);
-    *smem = (L.body + (Team::kContactsInSmem ? L.contact : 0)) * sizeof(double);
-    if (*smem > 227 * 1024) return -2;
+    if (Team::kContactsInSmem && *C > kWarpMaxContacts) return -2;
+    *smem = dyn_smem(Team::kContactsInSmem, nb, neq, *C, fd);
+    if (*smem > kMaxSmemBytes) return -2;
     return 0;
+}
+
+// One launch of a plan: sized for C contacts, it solves the worlds with count_min < count <= C (and, if last_class,
+// reports those above C as DSDF_LCP_TOO_LARGE).
+struct DynLaunch { bool cta; int C, count_min, last_class; };
+
+// The contact-count classes that cover a batch whose worlds have at most ncontacts_large contacts, most of them at most
+// ncontacts_small: one-warp launches for both classes (capped at 64 contacts) and a one-CTA launch for the worlds above
+// 64.  Worlds too large for the one-warp kernel, or force_cta, run on the one-CTA kernel in one class.  Returns the
+// number of launches (<= 3), or -1.
+static int dyn_plan(int nb, int neq, int fd, int small, int large, int force_cta, DynLaunch* out) {
+    if (small <= 0 || large <= 0) return -1;
+    if (force_cta || dyn_smem(true, nb, neq, 16, fd) > kWarpSmemBytes) {
+        out[0] = {true, large, -1, 1};
+        return 1;
+    }
+    const int wl = large < kWarpMaxContacts ? large : kWarpMaxContacts, ws = small < wl ? small : wl;
+    const bool two = wl > ws, beyond = large > kWarpMaxContacts;
+    int n = 0;
+    out[n++] = {false, ws, -1, (two || beyond) ? 0 : 1};
+    if (two) out[n++] = {false, wl, ws, beyond ? 0 : 1};
+    if (beyond) out[n++] = {true, large, kWarpMaxContacts, 1};
+    return n;
 }
 
 template <class Team>
@@ -811,95 +844,63 @@ static int dyn_launch_backward(const double* p, const double* v, const double* m
 
 extern "C" {
 
-size_t dsdf_dynamics_solve_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs) {
-    const DynLayout L = dyn_layout(nb, neq, ncontacts, fric_dirs);
-    return (L.body + L.contact) * sizeof(double);
-}
-size_t dsdf_dynamics_big_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs) {
-    return dyn_layout(nb, neq, ncontacts, fric_dirs).body * sizeof(double);
-}
-size_t dsdf_dynamics_big_workspace_bytes(int W, int nb, int neq, int ncontacts, int fric_dirs) {
-    return (size_t)W * dyn_layout(nb, neq, ncontacts, fric_dirs).contact * sizeof(double);
-}
-
-int dsdf_dynamics_solve_loop(const double* p, const double* v, const double* mass, const double* Ibody,
-                             const double* fric, const double* rest, const double* f, const double* dt,
-                             const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
-                             const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts_smem, int fric_dirs,
-                             double eps, int not_improved_lim, int max_iter,
-                             double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
-                             const int32_t* vmap, int32_t* ctrl, int count_min, int last_class, void* stream) {
-    return dyn_launch_forward<WarpTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
-                                        neq, maxc, ncontacts_smem, fric_dirs, eps, not_improved_lim, max_iter, x, new_v,
-                                        nu, lam, s, status, iters, vmap, ctrl, count_min, last_class, nullptr, stream);
+int dsdf_dynamics_plan(int W, int nb, int neq, int fric_dirs, int ncontacts_small, int ncontacts_large, int force_cta,
+                       size_t* workspace_bytes) {
+    if (W <= 0 || nb <= 0 || neq < 0 || (fric_dirs != 8 && fric_dirs != 4)) return -1;
+    DynLaunch plan[3];
+    const int n = dyn_plan(nb, neq, fric_dirs, ncontacts_small, ncontacts_large, force_cta, plan);
+    if (n < 0) return n;
+    size_t ws = 0;
+    for (int i = 0; i < n; ++i) {
+        if (dyn_smem(!plan[i].cta, nb, neq, plan[i].C, fric_dirs) > kMaxSmemBytes) return -2;
+        if (plan[i].cta) ws = (size_t)W * dyn_layout(nb, neq, plan[i].C, fric_dirs).contact * sizeof(double);
+    }
+    if (workspace_bytes) *workspace_bytes = ws;
+    return n;
 }
 
 int dsdf_dynamics_solve(const double* p, const double* v, const double* mass, const double* Ibody,
                         const double* fric, const double* rest, const double* f, const double* dt,
                         const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
-                        const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts_smem, int fric_dirs,
-                        double eps, int not_improved_lim, int max_iter,
-                        double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
-                        void* stream) {
-    return dsdf_dynamics_solve_loop(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb, neq,
-                                    maxc, ncontacts_smem, fric_dirs, eps, not_improved_lim, max_iter, x, new_v, nu, lam, s,
-                                    status, iters, nullptr, nullptr, -1, 1, stream);
-}
-
-int dsdf_dynamics_big_solve(const double* p, const double* v, const double* mass, const double* Ibody,
-                            const double* fric, const double* rest, const double* f, const double* dt,
-                            const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
-                            const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts, int fric_dirs,
-                            double eps, int not_improved_lim, int max_iter,
-                            double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
-                            const int32_t* vmap, int32_t* ctrl, int count_min, int last_class, double* workspace,
-                            void* stream) {
-    return dyn_launch_forward<CtaTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
-                                       neq, maxc, ncontacts, fric_dirs, eps, not_improved_lim, max_iter, x, new_v, nu,
-                                       lam, s, status, iters, vmap, ctrl, count_min, last_class, workspace, stream);
-}
-
-int dsdf_dynamics_solve_backward_loop(const double* p, const double* v, const double* mass, const double* Ibody,
-                                      const double* fric, const double* rest, const double* f, const double* dt,
-                                      const unsigned char* active, const int32_t* count, const int32_t* cbody,
-                                      const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
-                                      int ncontacts_smem, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
-                                      const double* x, const double* lam, const double* s, const double* g_new_v,
-                                      double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
-                                      double* gf, double* gdt, double* ggeo, int count_min, int last_class, void* stream) {
-    return dyn_launch_backward<WarpTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
-                                         neq, maxc, ncontacts_smem, fric_dirs, stop_contact_grad, stop_friction_grad, x,
-                                         lam, s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, count_min,
-                                         last_class, nullptr, stream);
+                        const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts_small,
+                        int ncontacts_large, int force_cta, int fric_dirs, double eps, int not_improved_lim,
+                        int max_iter, double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status,
+                        int32_t* iters, const int32_t* vmap, int32_t* ctrl, double* workspace, void* stream) {
+    DynLaunch plan[3];
+    const int n = dyn_plan(nb, neq, fric_dirs, ncontacts_small, ncontacts_large, force_cta, plan);
+    if (n < 0) return n;
+    for (int i = 0; i < n; ++i) {
+        const DynLaunch& d = plan[i];
+        const int rc = (d.cta ? dyn_launch_forward<CtaTeam> : dyn_launch_forward<WarpTeam>)(
+            p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb, neq, maxc, d.C, fric_dirs,
+            eps, not_improved_lim, max_iter, x, new_v, nu, lam, s, status, iters, vmap, ctrl, d.count_min,
+            d.last_class, workspace, stream);
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 int dsdf_dynamics_solve_backward(const double* p, const double* v, const double* mass, const double* Ibody,
                                  const double* fric, const double* rest, const double* f, const double* dt,
                                  const unsigned char* active, const int32_t* count, const int32_t* cbody,
                                  const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
-                                 int ncontacts_smem, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
+                                 int ncontacts_small, int ncontacts_large, int force_cta, int fric_dirs,
+                                 int stop_contact_grad, int stop_friction_grad,
                                  const double* x, const double* lam, const double* s, const double* g_new_v,
                                  double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
-                                 double* gf, double* gdt, double* ggeo, void* stream) {
-    return dsdf_dynamics_solve_backward_loop(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W,
-                                             nb, neq, maxc, ncontacts_smem, fric_dirs, stop_contact_grad,
-                                             stop_friction_grad, x, lam, s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf,
-                                             gdt, ggeo, -1, 1, stream);
-}
-
-int dsdf_dynamics_big_solve_backward(const double* p, const double* v, const double* mass, const double* Ibody,
-                                     const double* fric, const double* rest, const double* f, const double* dt,
-                                     const unsigned char* active, const int32_t* count, const int32_t* cbody,
-                                     const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
-                                     int ncontacts, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
-                                     const double* x, const double* lam, const double* s, const double* g_new_v,
-                                     double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
-                                     double* gf, double* gdt, double* ggeo, int count_min, int last_class,
-                                     double* workspace, void* stream) {
-    return dyn_launch_backward<CtaTeam>(p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb,
-                                        neq, maxc, ncontacts, fric_dirs, stop_contact_grad, stop_friction_grad, x, lam,
-                                        s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, count_min,
-                                        last_class, workspace, stream);
+                                 double* gf, double* gdt, double* ggeo, double* workspace, void* stream) {
+    DynLaunch plan[3];
+    const int n = dyn_plan(nb, neq, fric_dirs, ncontacts_small, ncontacts_large, force_cta, plan);
+    if (n < 0) return n;
+    for (int i = 0; i < n; ++i) {
+        const DynLaunch& d = plan[i];
+        const int rc = (d.cta ? dyn_launch_backward<CtaTeam> : dyn_launch_backward<WarpTeam>)(
+            p, v, mass, Ibody, fric, rest, f, dt, active, count, cbody, cgeo, eq_rows, W, nb, neq, maxc, d.C, fric_dirs,
+            stop_contact_grad, stop_friction_grad, x, lam, s, g_new_v, gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo,
+            d.count_min, d.last_class, workspace, stream);
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 }  // extern "C"

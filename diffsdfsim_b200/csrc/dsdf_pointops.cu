@@ -273,9 +273,9 @@ using namespace dsdf;
 
 extern "C" {
 
-int dsdf_sdf_query_ex(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
-                      long long grid_world_stride, const double* pts, int W, int N, int want_dir, double* sdf, double* dir,
-                      void* stream) {
+int dsdf_sdf_query(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
+                   long long grid_world_stride, const double* pts, int W, int N, int want_dir, double* sdf, double* dir,
+                   void* stream) {
     if (W <= 0 || N < 0 || kind < 0 || kind > DSDF_SDF_BOWL || (kind == DSDF_SDF_GRID && (!grid || res < 2))) return -1;
     if (N == 0) return 0;
     int bx = (N + 255) / 256;
@@ -297,14 +297,9 @@ int dsdf_sdf_query_ex(int kind, const double* shape, double extra0, double extra
     return (int)cudaGetLastError();
 }
 
-int dsdf_sdf_query(int kind, const double* shape, const double* grid, int res, long long grid_world_stride,
-                   const double* pts, int W, int N, int want_dir, double* sdf, double* dir, void* stream) {
-    return dsdf_sdf_query_ex(kind, shape, 0.0, 0.0, grid, res, grid_world_stride, pts, W, N, want_dir, sdf, dir, stream);
-}
-
-int dsdf_sdf_query_backward_ex(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
-                               long long grid_world_stride, const double* pts, int W, int N, const double* gsdf,
-                               const double* gdir, double* gpts, void* stream) {
+int dsdf_sdf_query_backward(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
+                            long long grid_world_stride, const double* pts, int W, int N, const double* gsdf,
+                            const double* gdir, double* gpts, void* stream) {
     if (W <= 0 || N < 0 || kind < 0 || kind > DSDF_SDF_BOWL || (kind == DSDF_SDF_GRID && (!grid || res < 2))) return -1;
     if (N == 0) return 0;
     int bx = (N + 255) / 256;
@@ -312,13 +307,6 @@ int dsdf_sdf_query_backward_ex(int kind, const double* shape, double extra0, dou
     sdf_query_bwd_kernel<<<dim3(bx, W), 256, 0, (cudaStream_t)stream>>>(kind, shape, grid, res, grid_world_stride, pts,
                                                                         N, gsdf, gdir, gpts, extra0, extra1);
     return (int)cudaGetLastError();
-}
-
-int dsdf_sdf_query_backward(int kind, const double* shape, const double* grid, int res, long long grid_world_stride,
-                            const double* pts, int W, int N, const double* gsdf, const double* gdir, double* gpts,
-                            void* stream) {
-    return dsdf_sdf_query_backward_ex(kind, shape, 0.0, 0.0, grid, res, grid_world_stride, pts, W, N, gsdf, gdir, gpts,
-                                      stream);
 }
 
 int dsdf_integrate(const double* p, const double* v, const double* dt, const unsigned char* active, int W, int nb,

@@ -2,11 +2,12 @@
 // (solve -> move -> find_contacts -> accept | halve dt and retry | give up below dt / 2^10 | take the remaining time |
 // time-of-contact bookkeeping) runs ON THE DEVICE, round after round, with no host decision in between.
 //
-// One ROUND = one attempt of every world that is still inside its step = five launches on one stream:
+// One ROUND = one attempt of every world that is still inside its step = these launches on one stream:
 //   step_prep_kernel      compacts the active worlds into "virtual worlds" (attempt d of world i uses dt / 2^d: a
 //                         rejected sub-step is retried from the SAME start state with half the step, world.py:344-356,
 //                         so when few worlds are left the halved retries are evaluated speculatively in one round)
 //   dyn_forward_kernel    (dsdf_dynsolve.cu, loop mode)   PdipmEngine.solve_dynamics         engines.py:31-83
+//                         one to three launches, one per contact-count class (dsdf_dynamics_plan)
 //   step_integrate_kernel                                 Body3D.move                       bodies.py:488-496
 //   contacts_kernel       (dsdf_contacts.cu, loop mode)   World.find_contacts                world.py:396-399
 //   step_commit_kernel    accept / reject bookkeeping, first accepted attempt in the reference's order wins; an accepted
@@ -313,41 +314,20 @@ int dsdf_step_rounds(const dsdf_step_args* a, int n_rounds, int ncontacts_small,
     for (int r = 0; r < n_rounds; ++r) {
         { PhaseTimer t(PHASE_PREP, st); step_prep_kernel<<<(W + 255) / 256, 256, 0, st>>>(*a); }
         PhaseTimer* td = new PhaseTimer(PHASE_DYN, st);
-        // contact-count classes: worlds with <= ncontacts_small contacts, and (if any) the rest; worlds with many bodies,
-        // or more contacts than the one-warp kernel holds, go to the one-CTA kernel (dsdf_dynsolve.cu, CtaTeam)
-        int rc = 0;
-        auto warp_class = [&](int C, int cmin, int last) {
-            return dsdf_dynamics_solve_loop(a->p, a->v, a->mass, a->Ibody, a->fric, a->rest, a->f, a->dt_used_v, nullptr,
-                                            a->count, a->body, a->geo, a->eq_rows, V, nb, (int)a->neq, (int)a->maxc, C,
-                                            (int)a->fric_dirs, 1e-12, 3, (int)a->max_iter, a->x_v, a->new_v_v, a->nu_v,
-                                            a->lam_v, a->s_v, a->lcp_status_v, a->iters_v, a->vmap, a->ctrl, cmin, last, stream);
-        };
-        auto big_class = [&](int C, int cmin) {
-            return dsdf_dynamics_big_solve(a->p, a->v, a->mass, a->Ibody, a->fric, a->rest, a->f, a->dt_used_v, nullptr,
-                                           a->count, a->body, a->geo, a->eq_rows, V, nb, (int)a->neq, (int)a->maxc, C,
-                                           (int)a->fric_dirs, 1e-12, 3, (int)a->max_iter, a->x_v, a->new_v_v, a->nu_v,
-                                           a->lam_v, a->s_v, a->lcp_status_v, a->iters_v, a->vmap, a->ctrl, cmin, 1,
-                                           a->dyn_ws, stream);
-        };
-        if (a->dyn_mode == 1) {
-            rc = big_class(ncontacts_large, -1);
-        } else {
-            const int wl = ncontacts_large > 64 ? 64 : ncontacts_large;          // largest class of the one-warp kernel
-            const int ws_ = ncontacts_small > wl ? wl : ncontacts_small;
-            const bool beyond = a->dyn_mode == 2 && ncontacts_large > 64;
-            const bool two = wl > ws_;
-            rc = warp_class(ws_, -1, (two || beyond) ? 0 : 1);
-            if (!rc && two) rc = warp_class(wl, ws_, beyond ? 0 : 1);
-            if (!rc && beyond) rc = big_class(ncontacts_large, 64);
-        }
-        if (rc) { delete td; return rc; }
+        // dsdf_dynamics_solve picks the contact-count classes of the round and the kernel of each (dsdf_dynsolve.cu)
+        int rc = dsdf_dynamics_solve(a->p, a->v, a->mass, a->Ibody, a->fric, a->rest, a->f, a->dt_used_v, nullptr, a->count,
+                                     a->body, a->geo, a->eq_rows, V, nb, (int)a->neq, (int)a->maxc, ncontacts_small,
+                                     ncontacts_large, (int)a->force_cta, (int)a->fric_dirs, 1e-12, 3, (int)a->max_iter,
+                                     a->x_v, a->new_v_v, a->nu_v, a->lam_v, a->s_v, a->lcp_status_v, a->iters_v, a->vmap,
+                                     a->ctrl, a->dyn_ws, stream);
         delete td;
+        if (rc) return rc;
         { PhaseTimer t(PHASE_MOVE, st); step_integrate_kernel<<<(V * nb + 127) / 128, 128, 0, st>>>(*a); }
         PhaseTimer* tc = new PhaseTimer(PHASE_CONTACTS, st);
-        rc = dsdf_contacts_detect_loop(a->geom, a->pairs, (int)a->npairs, a->p_try_v, a->shape, nullptr, V, nb, a->eps,
-                                       a->tol, a->fd_eps, a->body_eps, (int)a->detach_b2, (int)a->capK, (int)a->maxc,
-                                       a->count_v, a->body_v, a->face_v, a->abc_v, a->geo_v, a->status_v, nullptr, nullptr,
-                                       a->vmap, a->ctrl, stream);
+        rc = dsdf_contacts_detect(a->geom, a->pairs, (int)a->npairs, a->p_try_v, a->shape, nullptr, V, nb, a->eps, a->tol,
+                                  a->fd_eps, a->body_eps, (int)a->detach_b2, (int)a->capK, (int)a->maxc, a->count_v,
+                                  a->body_v, a->face_v, a->abc_v, a->geo_v, a->status_v, nullptr, nullptr, a->vmap,
+                                  a->ctrl, stream);
         delete tc;
         if (rc) return rc;
         { PhaseTimer t(PHASE_COMMIT, st); step_commit_kernel<<<(W + 3) / 4, 128, 0, st>>>(*a); }

@@ -93,8 +93,15 @@ class _Dynamics(torch.autograd.Function):
         return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, None, None, (dA if want_A else None), None, None, None
 
 
+def _fused_plan(W, nb, neq, fd, C, dev):
+    """Kernel launches of dsdf_dynamics_solve(_backward) for one class of C contacts and the workspace they need."""
+    n, nbytes = _lib.dynamics_plan(W, nb, neq, fd, C, C)
+    return n, (torch.empty(nbytes // 8 + 1, dtype=F64, device=dev) if nbytes else None)
+
+
 class _DynamicsFused(torch.autograd.Function):
-    """dsdf_dynamics_solve / dsdf_dynamics_solve_backward: one warp per world, structure-exploiting KKT.
+    """dsdf_dynamics_solve / dsdf_dynamics_solve_backward: structure-exploiting KKT, one class of ``nc_smem`` contacts
+    (the library picks the kernels, as for the device-resident step loop).
 
     The kernels write new_v (= -x, inactive worlds: v) and consume dL/dnew_v directly: no torch arithmetic around them.
     """
@@ -116,11 +123,14 @@ class _DynamicsFused(torch.autograd.Function):
         s = torch.empty_like(lam)
         status = torch.zeros(W, dtype=torch.int32, device=dev)
         iters = torch.zeros(W, dtype=torch.int32, device=dev)
+        C = cfg['nc_smem']
+        n, ws = _fused_plan(W, nb, neq, fd, C, dev)
         rc = _lib.call('dsdf_dynamics_solve', _lib.ptr(p), _lib.ptr(v), _lib.ptr(mass), _lib.ptr(Ibody),
                        _lib.ptr(fric), _lib.ptr(rest), _lib.ptr(f), _lib.ptr(dt), _lib.ptr(active), _lib.ptr(count),
-                       _lib.ptr(cbody), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, neq, maxc, cfg['nc_smem'], fd,
+                       _lib.ptr(cbody), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, neq, maxc, C, C, 0, fd,
                        1e-12, 3, cfg['max_iter'], _lib.ptr(x), _lib.ptr(new_v), _lib.ptr(nu), _lib.ptr(lam),
-                       _lib.ptr(s), _lib.ptr(status), _lib.ptr(iters), _lib.stream())
+                       _lib.ptr(s), _lib.ptr(status), _lib.ptr(iters), None, None, _lib.ptr(ws), _lib.stream(),
+                       kernels=n)
         _lib.check(rc, 'dsdf_dynamics_solve')
         ctx.save_for_backward(p, v, mass, Ibody, fric, rest, f, dt, geo, count, cbody, eq_rows, x, lam, s,
                               active if active is not None else p.new_empty(0))
@@ -141,13 +151,15 @@ class _DynamicsFused(torch.autograd.Function):
         gmass, gI = torch.empty_like(mass), torch.empty_like(Ibody)
         gfric, grest, gf = torch.empty_like(fric), torch.empty_like(rest), torch.empty_like(f)
         gdt, ggeo = torch.empty(W, dtype=F64, device=p.device), torch.empty_like(geo)
+        neq, C = eq_rows.shape[0], cfg['nc_smem']
+        n, ws = _fused_plan(W, nb, neq, fd, C, p.device)
         rc = _lib.call('dsdf_dynamics_solve_backward', _lib.ptr(p), _lib.ptr(v), _lib.ptr(mass), _lib.ptr(Ibody),
                        _lib.ptr(fric), _lib.ptr(rest), _lib.ptr(f), _lib.ptr(dt), _lib.ptr(active), _lib.ptr(count),
-                       _lib.ptr(cbody), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, eq_rows.shape[0], maxc,
-                       cfg['nc_smem'], fd, int(cfg['stop_contact_grad']), int(cfg['stop_friction_grad']),
+                       _lib.ptr(cbody), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, neq, maxc, C, C, 0, fd,
+                       int(cfg['stop_contact_grad']), int(cfg['stop_friction_grad']),
                        _lib.ptr(x), _lib.ptr(lam), _lib.ptr(s), _lib.ptr(gnv), _lib.ptr(gp), _lib.ptr(gv),
                        _lib.ptr(gmass), _lib.ptr(gI), _lib.ptr(gfric), _lib.ptr(grest), _lib.ptr(gf), _lib.ptr(gdt),
-                       _lib.ptr(ggeo), _lib.stream())
+                       _lib.ptr(ggeo), _lib.ptr(ws), _lib.stream(), kernels=n)
         _lib.check(rc, 'dsdf_dynamics_solve_backward')
         return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, None, None, None, None, None
 

@@ -28,7 +28,7 @@ class _SdfQuery(torch.autograd.Function):
             stride = res ** 3 if grid.dim() == 4 else 0
         sdf = torch.empty(W, N, dtype=F64, device=pts.device)
         d = torch.empty(W, N, 3, dtype=F64, device=pts.device) if want_dir else None
-        rc = _lib.call('dsdf_sdf_query_ex', kind, _lib.ptr(shape), float(extra[0]), float(extra[1]),
+        rc = _lib.call('dsdf_sdf_query', kind, _lib.ptr(shape), float(extra[0]), float(extra[1]),
                        _lib.ptr(grid) if kind == 3 else None, res, stride, _lib.ptr(pts), W, N, int(want_dir), _lib.ptr(sdf),
                        _lib.ptr(d), _lib.stream())
         _lib.check(rc, 'dsdf_sdf_query')
@@ -48,7 +48,7 @@ class _SdfQuery(torch.autograd.Function):
         gpts = torch.empty_like(pts)
         gdir = _c(gdir) if (want_dir and gdir is not None and gdir.numel()) else None
         gsdf = _c(gsdf)                  # contiguous copies stay bound to locals until the launch has been enqueued
-        rc = _lib.call('dsdf_sdf_query_backward_ex', kind, _lib.ptr(shape), float(extra[0]), float(extra[1]),
+        rc = _lib.call('dsdf_sdf_query_backward', kind, _lib.ptr(shape), float(extra[0]), float(extra[1]),
                        _lib.ptr(grid) if kind == 3 else None, res, stride, _lib.ptr(pts), W, N, _lib.ptr(gsdf), _lib.ptr(gdir),
                        _lib.ptr(gpts), _lib.stream())
         _lib.check(rc, 'dsdf_sdf_query_backward')

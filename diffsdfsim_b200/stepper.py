@@ -36,7 +36,7 @@ _SLOT_FIELDS = ['world', 'p_in', 'v_in', 'x', 'new_v', 'p_try', 'dt_raw', 'dt_us
                 'toc_mask', 'count_in', 'body_in', 'geo_in', 'count', 'body', 'face', 'abc', 'geo']
 _INT_FIELDS = ['W', 'nb', 'neq', 'maxc', 'fric_dirs', 'capK', 'npairs', 'depth', 'spec_threshold', 'depth2',
                'spec_threshold2', 'vcap', 'n_slots', 'slots_final',
-               'max_iter', 'max_rounds', 'strict', 'toc_enabled', 'fixed_dt', 'detach_b2', 'dyn_mode']
+               'max_iter', 'max_rounds', 'strict', 'toc_enabled', 'fixed_dt', 'detach_b2', 'force_cta']
 _DBL_FIELDS = ['world_dt', 'eps', 'tol', 'fd_eps', 'body_eps']
 _PTR_FIELDS = ['geom', 'pairs', 'eq_rows', 'mass', 'Ibody', 'fric', 'rest', 'f', 'shape',
                'p', 'v', 't', 'dt_try', 'end_t', 'last_dt', 'active', 'toc_flag', 'had', 'nsub', 'attempts',
@@ -170,7 +170,7 @@ class DeviceStepper:
     """Owns the per-world work buffers of the step loop of one ``World3D`` and launches its rounds."""
     INITIAL_SLOTS = 2
     TIMING = None           # set to {} to accumulate host wall-clock seconds per phase of run() (diagnostics)
-    FORCE_DYN_MODE = None   # tests: 1 = run every world through the one-CTA dynamics kernel
+    FORCE_CTA = False       # tests: run every world through the one-CTA dynamics kernel
 
     @classmethod
     def _tick(cls, name, t0):
@@ -217,20 +217,10 @@ class DeviceStepper:
         self.lcp_status_v = torch.zeros(V, dtype=I32, device=dev)
         self.iters_v = torch.zeros(V, dtype=I32, device=dev)
         self.cs_v = ContactSet(V, self.maxc, dev)
-        # dynamics kernel selection (csrc/dsdf_dynsolve.cu: one warp per world, <= 64 contacts, small worlds;
-        # or one CTA per world, any contact count, up to ~120 free velocity components)
-        L = _lib.lib()
-        neq, fd = world.num_constraints, world.fric_dirs
-        warp_fits = L.dsdf_dynamics_solve_smem_bytes(nb, neq, 16, fd) <= 48 * 1024
-        self.dyn_mode = 1 if not warp_fits else (2 if self.maxc > 64 else 0)
-        if self.FORCE_DYN_MODE is not None:
-            self.dyn_mode = self.FORCE_DYN_MODE
-        self.dyn_ws = None
-        if self.dyn_mode:
-            if L.dsdf_dynamics_big_smem_bytes(nb, neq, self.maxc, fd) > 227 * 1024:
-                raise _lib.DsdfLibraryError('world too large for the dynamics kernels: %d bodies' % nb)
-            n = L.dsdf_dynamics_big_workspace_bytes(V, nb, neq, self.maxc, fd)
-            self.dyn_ws = torch.empty(n // 8 + 1, dtype=F64, device=dev)
+        # workspace of the one-CTA dynamics kernel, if some world may run on it (csrc/dsdf_dynsolve.cu)
+        self.force_cta = bool(self.FORCE_CTA)
+        _, n = _lib.dynamics_plan(V, nb, world.num_constraints, world.fric_dirs, self.maxc, self.maxc, self.force_cta)
+        self.dyn_ws = torch.empty(n // 8 + 1, dtype=F64, device=dev) if n else None
 
     # ------------------------------------------------------------------------------------------------------------
     def _args(self, world, fixed_dt, st, tape, f):
@@ -260,7 +250,7 @@ class DeviceStepper:
         v = self.cs_v
         a.count_v, a.status_v, a.body_v, a.face_v, a.abc_v, a.geo_v = (_ptr(v.count), _ptr(v.status), _ptr(v.body),
                                                                        _ptr(v.face), _ptr(v.abc), _ptr(v.geo))
-        a.dyn_mode, a.dyn_ws = self.dyn_mode, _ptr(self.dyn_ws)
+        a.force_cta, a.dyn_ws = int(self.force_cta), _ptr(self.dyn_ws)
         a.ctrl = _ptr(self.ctrl)
         # the slot table lives in device memory (no limit from the kernel-parameter space); uploaded when it changes
         table = (StepSlot * len(tape.slots))()
@@ -275,8 +265,7 @@ class DeviceStepper:
         """Contacts the dynamics kernel sizes its shared memory for, as two classes (small, large): the bulk of the
         worlds (largest non-penetrating count so far + slack) and, if there are any, the few worlds that carry many more
         (a world that gave up halving keeps a penetrating state with dozens of contacts)."""
-        cap = world.maxc if self.dyn_mode else min(world.maxc, 64)
-        r4 = lambda c: max(4, min((c + 2 + 3) // 4 * 4, cap))
+        r4 = lambda c: max(4, min((c + 2 + 3) // 4 * 4, world.maxc))
         small, large = r4(self.max_clean), r4(self.max_count)
         return small, (large if large > small else small)
 
@@ -326,11 +315,12 @@ class DeviceStepper:
         syncs = 0
         while True:
             small, large = self._smem_contacts(world)
-            rc = _lib.call('dsdf_step_rounds', ctypes.byref(args), burst, small, large, stream)
+            n_dyn, _ = _lib.dynamics_plan(self.vcap, nb, world.num_constraints, world.fric_dirs, small, large,
+                                          self.force_cta)
+            nk = burst * (4 + n_dyn)                         # kernels of this burst
+            rc = _lib.call('dsdf_step_rounds', ctypes.byref(args), burst, small, large, stream, kernels=nk)
             _lib.check(rc, 'dsdf_step_rounds')
-            nk = burst * (6 if large > small else 5)         # kernels of this burst (bench.py's gpu_launches)
             self.launches += nk
-            _lib.LAUNCHES['step_round_kernels'] = _lib.LAUNCHES.get('step_round_kernels', 0) + nk
             t0 = self._tick('launch', t0)
             c = self._read_ctrl()
             t0 = self._tick('sync', t0)
@@ -375,7 +365,7 @@ class DeviceStepper:
         if ls & LCP_INACCURATE and getattr(world.engine, 'verbose', -1) >= 0:
             print('qpth warning: Returning an inaccurate and potentially incorrect solution.')       # batch.py:165,229
         tape.maxsub, tape.any_toc = c[CT_MAXNSUB], bool(c[CT_ANYTOC])
-        tape.maxc, tape.C, tape.rounds, tape.syncs = world.maxc, self._smem_contacts(world) + (self.dyn_mode,), c[CT_ROUNDS], syncs
+        tape.maxc, tape.C, tape.rounds, tape.syncs = world.maxc, self._smem_contacts(world) + (self.force_cta,), c[CT_ROUNDS], syncs
         tape.p_out, tape.v_out, tape.last_dt_out, tape.had = st['p'], st['v'], st['last_dt'], st['had'].bool()
         tape.final = st['cur']
         tape.geo_out = st['cur'].geo.clone()
@@ -459,36 +449,16 @@ def _dyn_bwd(cfg, p, v, mass, Ibody, fric, rest, f, dt, active, count, body, geo
     gmass, gI = torch.empty_like(mass), torch.empty_like(Ibody)
     gfric, grest, gf = torch.empty_like(fric), torch.empty_like(rest), torch.empty_like(f)
     gdt, ggeo = torch.empty(W, dtype=F64, device=p.device), torch.empty_like(geo)
-    small, large, mode = cfg['C']
-    large = min(large, maxc)
-    common = lambda C: (_ptr(p), _ptr(v), _ptr(mass), _ptr(Ibody), _ptr(fric), _ptr(rest), _ptr(f), _ptr(dt), _ptr(active),
-                        _ptr(count), _ptr(body), _ptr(geo), _ptr(cfg['eq_rows']), W, nb, cfg['neq'], maxc, C,
-                        cfg['fric_dirs'], int(cfg['stop_contact_grad']), int(cfg['stop_friction_grad']), _ptr(x), _ptr(lam),
-                        _ptr(s), _ptr(gnv), _ptr(gp), _ptr(gv), _ptr(gmass), _ptr(gI), _ptr(gfric), _ptr(grest), _ptr(gf),
-                        _ptr(gdt), _ptr(ggeo))
-    # contact-count classes, as in the forward (dsdf_step_rounds): one-warp kernel up to 64 contacts, one-CTA kernel beyond
-    # (or for every world when it has many bodies)
-    warp, big = [], None
-    if mode == 1:
-        big = (large, -1)
-    else:
-        wl = min(large, 64)
-        ws_ = min(small, wl)
-        beyond = mode == 2 and large > 64
-        warp.append((ws_, -1, 0 if (wl > ws_ or beyond) else 1))
-        if wl > ws_:
-            warp.append((wl, ws_, 0 if beyond else 1))
-        if beyond:
-            big = (large, 64)
-    for C, cmin, last in warp:
-        rc = _lib.call('dsdf_dynamics_solve_backward_loop', *common(C), cmin, last, _lib.stream())
-        _lib.check(rc, 'dsdf_dynamics_solve_backward')
-    if big is not None:
-        L = _lib.lib()
-        n = L.dsdf_dynamics_big_workspace_bytes(W, nb, cfg['neq'], big[0], cfg['fric_dirs'])
-        ws = torch.empty(n // 8 + 1, dtype=F64, device=p.device)
-        rc = _lib.call('dsdf_dynamics_big_solve_backward', *common(big[0]), big[1], 1, _ptr(ws), _lib.stream())
-        _lib.check(rc, 'dsdf_dynamics_big_solve_backward')
+    small, large, force_cta = cfg['C']             # the contact-count classes of the forward
+    n, nbytes = _lib.dynamics_plan(W, nb, cfg['neq'], cfg['fric_dirs'], small, large, force_cta)
+    ws = torch.empty(nbytes // 8 + 1, dtype=F64, device=p.device) if nbytes else None
+    rc = _lib.call('dsdf_dynamics_solve_backward', _ptr(p), _ptr(v), _ptr(mass), _ptr(Ibody), _ptr(fric), _ptr(rest),
+                   _ptr(f), _ptr(dt), _ptr(active), _ptr(count), _ptr(body), _ptr(geo), _ptr(cfg['eq_rows']), W, nb,
+                   cfg['neq'], maxc, small, large, int(force_cta), cfg['fric_dirs'], int(cfg['stop_contact_grad']),
+                   int(cfg['stop_friction_grad']), _ptr(x), _ptr(lam), _ptr(s), _ptr(gnv), _ptr(gp), _ptr(gv),
+                   _ptr(gmass), _ptr(gI), _ptr(gfric), _ptr(grest), _ptr(gf), _ptr(gdt), _ptr(ggeo), _ptr(ws),
+                   _lib.stream(), kernels=n)
+    _lib.check(rc, 'dsdf_dynamics_solve_backward')
     return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo
 
 

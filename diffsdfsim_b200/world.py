@@ -656,7 +656,6 @@ class World3D:
         return acc_w, dt_out, act_out, int(info[4])
 
     MAX_CAPK, MAX_MAXC = 1024, 512     # candidate list: shared memory of the contact kernel; contacts: tape / workspace sizes
-                                       # (the host-driven loop uses the one-warp dynamics kernel: 64 contacts)
 
     def _grow_capacity(self, bits):
         """Double the candidate (capK) and / or contact (maxc) capacity after an overflow; raises when at the limit."""

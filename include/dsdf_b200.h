@@ -86,24 +86,20 @@ int dsdf_lcp_backward(const double* Q, const double* G, const double* A, const d
  * Replaces SDF3D.query_sdfs(pts_loc, return_grads)  (sdf_physics/physics3d/bodies.py:721-760) with the
  * analytic SDFs (bodies.py:38-125) and the grid SDF (bodies.py:203-257; ev_sdf_utils.grid_interp).
  * shape (W,4) = [a,b,c,scale]: box dims/scale | sphere r/scale | cylinder r/scale,h/scale | grid: unused.
+ * extra0 / extra1: the further parameters of the kinds that need more than three (DSDF_SDF_BOX_ROUNDED / BRICK:
+ * extra0 = r/scale); 0 for the others.
  * grid: W grids of res^3 doubles, world w at grid + w*grid_world_stride (stride 0 = shared grid).
  * pts (W,N,3) body-frame points -> sdf (W,N), dir (W,N,3) unit gradient (NULL/want_dir=0 to skip).
  * Outside the cube |p| <= scale: sdf = scale, dir = 0.
  */
-int dsdf_sdf_query(int kind, const double* shape, const double* grid, int res, long long grid_world_stride,
-                   const double* pts, int W, int N, int want_dir, double* sdf, double* dir, void* stream);
+int dsdf_sdf_query(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
+                   long long grid_world_stride, const double* pts, int W, int N, int want_dir, double* sdf, double* dir,
+                   void* stream);
 /* VJP of the above w.r.t. pts with torch-autograd conventions (DiffGridSDF.backward for grids, bodies.py:253-257):
  * gpts (W,N,3) = gsdf * d sdf/d pts + gdir . d dir/d pts ; gsdf / gdir may be NULL. */
-int dsdf_sdf_query_backward(int kind, const double* shape, const double* grid, int res, long long grid_world_stride,
-                            const double* pts, int W, int N, const double* gsdf, const double* gdir, double* gpts,
-                            void* stream);
-/* The same with the extra parameters of the kinds that need more than three (DSDF_SDF_BOX_ROUNDED / BRICK: extra0 = r/scale). */
-int dsdf_sdf_query_ex(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
-                      long long grid_world_stride, const double* pts, int W, int N, int want_dir, double* sdf, double* dir,
-                      void* stream);
-int dsdf_sdf_query_backward_ex(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
-                               long long grid_world_stride, const double* pts, int W, int N, const double* gsdf,
-                               const double* gdir, double* gpts, void* stream);
+int dsdf_sdf_query_backward(int kind, const double* shape, double extra0, double extra1, const double* grid, int res,
+                            long long grid_world_stride, const double* pts, int W, int N, const double* gsdf,
+                            const double* gdir, double* gpts, void* stream);
 
 /* ----------------------------------------------------------- integrator ----
  * Replaces Body3D.move (sdf_physics/physics3d/bodies.py:488-496): q <- standardize(quat(expmap(w dt)) * q),
@@ -164,12 +160,16 @@ typedef struct dsdf_body_geom {
  *   cabc (W,maxc,3) barycentrics; cgeo (W,maxc,10) = [normal(3), p1(3), p2(3), pen]; wstatus (W).
  *   pre_ids (W,2*npairs,capK) / pre_cnt (W,2*npairs): PRE-filter contact face ids per direction (parity
  *   evidence; -1 = direction not searched); both may be NULL.
+ * vmap / ctrl (both NULL outside the device-resident step loop below): CTA w works on VIRTUAL world w (poses p[w],
+ * outputs at [w]) with the shapes and per-world geometry of the real world vmap[w]; ctrl = the loop's control block
+ * (every CTA returns at once when the loop is idle).
  */
 int dsdf_contacts_detect(const dsdf_body_geom* geom, const int32_t* pairs, int npairs, const double* p,
                          const double* shape, const unsigned char* active,
                          int W, int nb, double eps, double tol, double fd_eps, double body_eps, int detach_b2,
                          int capK, int maxc, int32_t* count, int32_t* cbody, int32_t* cface, double* cabc, double* cgeo,
-                         int32_t* wstatus, int32_t* pre_ids, int32_t* pre_cnt, void* stream);
+                         int32_t* wstatus, int32_t* pre_ids, int32_t* pre_cnt, const int32_t* vmap, const int32_t* ctrl,
+                         void* stream);
 /* Replaces _filter_contacts (sdf_physics/physics3d/contacts.py:97-158) as a stand-alone operator: W independent contact
  * lists, list w = the first n[w] rows of normals / p1 (W,capK,3).  keep (W,capK) <- 1 for the contacts the reference keeps:
  * zero normals dropped, greedy clustering by angle < 1e-2 rad to the first remaining normal, per cluster the vertices of the
@@ -182,28 +182,17 @@ int dsdf_filter_contacts(const double* normals, const double* p1, const int32_t*
  * was built with -DDSDF_PHASE_PROFILE (DSDF_PHASE_PROFILE=1 python -m diffsdfsim_b200.build). Host pointer out8. */
 int dsdf_contacts_phase_cycles(unsigned long long* out8, int reset);
 /* VJP of cgeo w.r.t. the poses (the reference's grad-enabled second _compute_contacts, contacts.py:262-264):
- * gp (W,nb,7) from ggeo (W,maxc,10). */
-int dsdf_contact_geometry_backward(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
-                                   double fd_eps, int detach_b2, int maxc, const int32_t* count, const int32_t* cbody,
-                                   const int32_t* cface, const double* cabc, const double* ggeo, double* gp, void* stream);
-
-/* Same for a compact batch of rows: row w carries the poses / contacts of world wmap[w], whose shapes and per-world
- * meshes / grids are used (wmap == NULL: row = world). */
-int dsdf_contact_geometry_backward_rows(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
-                                        double fd_eps, int detach_b2, int maxc, const int32_t* count,
-                                        const int32_t* cbody, const int32_t* cface, const double* cabc,
-                                        const double* ggeo, double* gp, const int32_t* wmap, void* stream);
-
-/* The same with the gradients w.r.t. the SHAPES as well (radius / dimension fitting: the reference's grad-enabled
+ * gp (W,nb,7) from ggeo (W,maxc,10).  wmap (W) or NULL: row w carries the poses / contacts of world wmap[w], whose
+ * shapes and per-world meshes / grids are used (a compact batch of rows; NULL: row = world).
+ * With gshape / gctri the gradients w.r.t. the SHAPES as well (radius / dimension fitting: the reference's grad-enabled
  * _compute_contacts differentiates through the SDF parameters, the scale and the mesh vertices):
  * gshape (W,nb,4) = d/d[a,b,c,scale] of every body, gctri (W,maxc,3) = gradient w.r.t. the body-frame point
  * sum(abc * vertices of the face) on the mesh body of each contact (the caller scatters it onto the vertices with the
  * weights cabc).  gshape == gctri == NULL: pose gradients only. */
-int dsdf_contact_geometry_backward_full(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
-                                        double fd_eps, int detach_b2, int maxc, const int32_t* count,
-                                        const int32_t* cbody, const int32_t* cface, const double* cabc,
-                                        const double* ggeo, double* gp, const int32_t* wmap, double* gshape,
-                                        double* gctri, void* stream);
+int dsdf_contact_geometry_backward(const dsdf_body_geom* geom, const double* p, const double* shape, int W, int nb,
+                                   double fd_eps, int detach_b2, int maxc, const int32_t* count, const int32_t* cbody,
+                                   const int32_t* cface, const double* cabc, const double* ggeo, double* gp,
+                                   const int32_t* wmap, double* gshape, double* gctri, void* stream);
 
 /* ------------------------------------------------------------- dynamics ----
  * Replaces the matrix assembly of PdipmEngine.solve_dynamics (lcp_physics/physics/engines.py:31-79) with
@@ -239,62 +228,53 @@ int dsdf_dynamics_assemble_backward(const double* p, const double* v, const doub
                                     double* gf, double* gdt, double* ggeo, void* stream);
 
 /* ------------------------------------------------- fused contact dynamics ----
- * Replaces PdipmEngine.solve_dynamics (lcp_physics/physics/engines.py:31-83) end to end, one warp per world:
+ * Replaces PdipmEngine.solve_dynamics (lcp_physics/physics/engines.py:31-83) end to end:
  * assembly (as dsdf_dynamics_assemble) + the PDIPM of lcp_physics/lcp/solvers/batch.py:70-237 with the Newton
  * systems reduced through the per-contact block structure of F + D^-1 (closed-form block inverse, pivoted LU of
- * the (6 nb + neq)^2 reduced KKT matrix in shared memory) instead of the dense nineq^2 factorisation.
+ * the free block of the (6 nb + neq)^2 reduced KKT matrix) instead of the dense nineq^2 factorisation.
  * Same iterates as dsdf_lcp_forward on the assembled matrices up to round-off.
  * eq_rows (neq,2) int32 = [body, velocity component] of each equality row (rows of Je are 0/1 selections:
- * sdf_physics/physics3d/constraints.py:32-145).  ncontacts_smem (0 = maxc): contacts the launch sizes its shared
- * memory for (<= 64); worlds with more get DSDF_LCP_TOO_LARGE.
+ * sdf_physics/physics3d/constraints.py:32-145).
  * Outputs x (W,6nb), new_v (W,6nb) = -x (engines.py:81-82; inactive worlds: v passed through; may be NULL),
  * nu (W,neq), lam / s (W, maxc (2+fric_dirs)) in the reference's row order [normal | friction | cone], status (W),
  * iters (W).
+ *
+ * One call runs one to three kernel launches, one per contact-count class: a launch sized for C contacts solves the
+ * worlds with count_min < count <= C, and the last class reports the worlds above its C as DSDF_LCP_TOO_LARGE.
+ * ncontacts_small (> 0): contacts of the bulk of the worlds; ncontacts_large: of the few worlds with many more
+ * (ncontacts_large <= ncontacts_small: one class); both are clamped to maxc.  Two kernels run the classes:
+ *   one warp per world, the whole world in shared memory: up to 64 contacts, small worlds (the default);
+ *   one CTA of 256 threads per world for many bodies (up to ~120 free velocity components) and / or more than 64
+ *   contacts: shared memory holds what scales with the bodies, a global workspace holds what scales with the contacts
+ *   (no cap on their number).
+ * force_cta = 1 runs every world on the one-CTA kernel.  dsdf_dynamics_plan returns the number of launches of a call
+ * (or -2: the world does not fit the one-CTA kernel's shared memory) and the bytes of the workspace it needs, 0 when no
+ * world goes to the one-CTA kernel (workspace may then be NULL).
+ * vmap / ctrl (both NULL outside the device-resident step loop below): CTA w solves VIRTUAL world w (its own dt[w],
+ * outputs at [w]) with the state, parameters and current contacts of the real world vmap[w]; ctrl = the loop's
+ * control block (every CTA returns at once when the loop is idle).
  */
-size_t dsdf_dynamics_solve_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs);
+int dsdf_dynamics_plan(int W, int nb, int neq, int fric_dirs, int ncontacts_small, int ncontacts_large, int force_cta,
+                       size_t* workspace_bytes);
 int dsdf_dynamics_solve(const double* p, const double* v, const double* mass, const double* Ibody,
                         const double* fric, const double* rest, const double* f, const double* dt,
                         const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
-                        const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts_smem, int fric_dirs,
-                        double eps, int not_improved_lim, int max_iter,
-                        double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
-                        void* stream);
+                        const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts_small,
+                        int ncontacts_large, int force_cta, int fric_dirs, double eps, int not_improved_lim,
+                        int max_iter, double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status,
+                        int32_t* iters, const int32_t* vmap, int32_t* ctrl, double* workspace, void* stream);
 /* Replaces LCPFunctionFn.backward (lcp_physics/lcp/lcp.py:156-213) + the autograd of the assembly, fused: from
  * g_new_v = dL/dnew_v (W,6nb) straight to the gradients of the physical inputs (no dense dG / dF is materialised).
- * Inactive worlds pass g_new_v through to gv. */
+ * Inactive worlds pass g_new_v through to gv.  Contact-count classes, kernels and workspace as in the forward. */
 int dsdf_dynamics_solve_backward(const double* p, const double* v, const double* mass, const double* Ibody,
                                  const double* fric, const double* rest, const double* f, const double* dt,
                                  const unsigned char* active, const int32_t* count, const int32_t* cbody,
                                  const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
-                                 int ncontacts_smem, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
+                                 int ncontacts_small, int ncontacts_large, int force_cta, int fric_dirs,
+                                 int stop_contact_grad, int stop_friction_grad,
                                  const double* x, const double* lam, const double* s, const double* g_new_v,
                                  double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
-                                 double* gf, double* gdt, double* ggeo, void* stream);
-
-/* The same solver for LARGE worlds -- many bodies and / or hundreds of contacts -- one CTA per world: shared memory holds
- * what scales with the bodies (free block of the reduced KKT matrix, <= ~120 free velocity components), a caller-provided
- * global workspace of dsdf_dynamics_big_workspace_bytes(W, ...) bytes holds what scales with the contacts (no cap on
- * their number), per-body contact lists exploit the body-pair block sparsity of G Q^-1 G'.  Same arguments and semantics
- * as dsdf_dynamics_solve_loop / dsdf_dynamics_solve_backward_loop (csrc/dsdf_dynsolve.cu, CtaTeam instantiation). */
-size_t dsdf_dynamics_big_smem_bytes(int nb, int neq, int ncontacts, int fric_dirs);
-size_t dsdf_dynamics_big_workspace_bytes(int W, int nb, int neq, int ncontacts, int fric_dirs);
-int dsdf_dynamics_big_solve(const double* p, const double* v, const double* mass, const double* Ibody,
-                            const double* fric, const double* rest, const double* f, const double* dt,
-                            const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
-                            const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts, int fric_dirs,
-                            double eps, int not_improved_lim, int max_iter,
-                            double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
-                            const int32_t* vmap, int32_t* ctrl, int count_min, int last_class, double* workspace,
-                            void* stream);
-int dsdf_dynamics_big_solve_backward(const double* p, const double* v, const double* mass, const double* Ibody,
-                                     const double* fric, const double* rest, const double* f, const double* dt,
-                                     const unsigned char* active, const int32_t* count, const int32_t* cbody,
-                                     const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
-                                     int ncontacts, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
-                                     const double* x, const double* lam, const double* s, const double* g_new_v,
-                                     double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
-                                     double* gf, double* gdt, double* ggeo, int count_min, int last_class,
-                                     double* workspace, void* stream);
+                                 double* gf, double* gdt, double* ggeo, double* workspace, void* stream);
 
 /* ------------------------------------------------------ step bookkeeping ----
  * Replaces the accept / reject / halve-dt / remaining-time / time-of-contact control flow of World.step_dt and
@@ -341,37 +321,6 @@ int dsdf_contactset_move(int n, int maxc, const long long* idx, const long long*
                          int32_t* count_d, int32_t* status_d, int32_t* body_d, int32_t* face_d,
                          double* abc_d, double* geo_d, void* stream);
 
-/* Loop-mode variants of dsdf_dynamics_solve / dsdf_contacts_detect used by the device-resident step loop below:
- * CTA w works on VIRTUAL world w (its own dt[w] / poses p[w], outputs at [w]) but reads the state, parameters, current
- * contacts, shapes and per-world geometry of the real world vmap[w]; ctrl = the loop's control block (every CTA returns
- * at once when the loop is idle).  vmap == NULL && ctrl == NULL: identical to the plain entry points. */
-int dsdf_dynamics_solve_loop(const double* p, const double* v, const double* mass, const double* Ibody,
-                             const double* fric, const double* rest, const double* f, const double* dt,
-                             const unsigned char* active, const int32_t* count, const int32_t* cbody, const double* cgeo,
-                             const int32_t* eq_rows, int W, int nb, int neq, int maxc, int ncontacts_smem, int fric_dirs,
-                             double eps, int not_improved_lim, int max_iter,
-                             double* x, double* new_v, double* nu, double* lam, double* s, int32_t* status, int32_t* iters,
-                             const int32_t* vmap, int32_t* ctrl, int count_min, int last_class, void* stream);
-/* count_min / last_class: contact-count classes.  A launch sized for ncontacts_smem contacts solves the worlds with
- * count_min < count <= ncontacts_smem and leaves the others untouched (last_class = 1: worlds above ncontacts_smem are
- * reported DSDF_LCP_TOO_LARGE instead), so a batch is covered by a launch for the typical count plus one for the few
- * worlds with many contacts.  (-1, 1) = every world, the plain entry points' behaviour.  In the backward, masked
- * (inactive) worlds are written by the count_min < 0 launch only. */
-int dsdf_dynamics_solve_backward_loop(const double* p, const double* v, const double* mass, const double* Ibody,
-                                      const double* fric, const double* rest, const double* f, const double* dt,
-                                      const unsigned char* active, const int32_t* count, const int32_t* cbody,
-                                      const double* cgeo, const int32_t* eq_rows, int W, int nb, int neq, int maxc,
-                                      int ncontacts_smem, int fric_dirs, int stop_contact_grad, int stop_friction_grad,
-                                      const double* x, const double* lam, const double* s, const double* g_new_v,
-                                      double* gp, double* gv, double* gmass, double* gI, double* gfric, double* grest,
-                                      double* gf, double* gdt, double* ggeo, int count_min, int last_class, void* stream);
-int dsdf_contacts_detect_loop(const dsdf_body_geom* geom, const int32_t* pairs, int npairs, const double* p,
-                              const double* shape, const unsigned char* active,
-                              int W, int nb, double eps, double tol, double fd_eps, double body_eps, int detach_b2,
-                              int capK, int maxc, int32_t* count, int32_t* cbody, int32_t* cface, double* cabc, double* cgeo,
-                              int32_t* wstatus, int32_t* pre_ids, int32_t* pre_cnt, const int32_t* vmap, const int32_t* ctrl,
-                              void* stream);
-
 /* ------------------------------------------------- device-resident step ----
  * World.step / World.step_dt (lcp_physics/physics/world.py:119-139, 241-379) as a state machine that lives on the
  * device: the host launches ROUNDS (one attempt of every world still inside its step: prep -> solve -> move ->
@@ -386,7 +335,7 @@ int dsdf_contacts_detect_loop(const dsdf_body_geom* geom, const int32_t* pairs, 
 /* bits of ctrl[0] (abort word): what the host must do before launching further rounds */
 #define DSDF_STEP_CAPK        1   /* a paused world overflowed the candidate list: enlarge capK          */
 #define DSDF_STEP_MAXC        2   /* a paused world found more than maxc contacts: enlarge maxc           */
-#define DSDF_STEP_DYN_SMEM    4   /* a world has more contacts than ncontacts_smem: round voided           */
+#define DSDF_STEP_DYN_SMEM    4   /* a world has more contacts than ncontacts_large: round voided          */
 #define DSDF_STEP_TAPE        8   /* a paused world found its tape slot missing or full: add / enlarge slots (the host
                                      clamps the slot's row counter to its capacity before resuming)           */
 #define DSDF_STEP_MAX_ROUNDS 16   /* max_rounds reached with worlds still active                           */
@@ -424,8 +373,7 @@ typedef struct dsdf_step_args {
                                         leaves the step early (its time stays behind) and DSDF_CON_STALLED is reported */
     int64_t max_iter, max_rounds;
     int64_t strict, toc_enabled, fixed_dt, detach_b2;
-    int64_t dyn_mode;                /* 0: one-warp dynamics kernel only (<= 64 contacts); 1: the one-CTA kernel for every
-                                        world (many bodies); 2: one-warp kernel up to 64 contacts, one-CTA kernel above */
+    int64_t force_cta;               /* 1: every world on the one-CTA dynamics kernel; 0: dsdf_dynamics_solve chooses */
     double world_dt, eps, tol, fd_eps, body_eps;
     const dsdf_body_geom* geom; const int32_t* pairs; const int32_t* eq_rows;
     const double *mass, *Ibody, *fric, *rest, *f, *shape;              /* (W,nb..) constant during the step */
@@ -445,8 +393,8 @@ typedef struct dsdf_step_args {
 int dsdf_step_begin(const dsdf_step_args* a, void* stream);
 /* Clear the abort word after the host enlarged a buffer (a may carry new pointers / sizes from here on). */
 int dsdf_step_resume(const dsdf_step_args* a, void* stream);
-/* Launch n_rounds rounds (5-6 kernels each) without any host synchronisation.  ncontacts_small / ncontacts_large:
- * contacts the dynamics kernel sizes its shared memory for, in two classes (large <= small: one launch).
+/* Launch n_rounds rounds (4 kernels + the 1-3 of dsdf_dynamics_solve each) without any host synchronisation.
+ * ncontacts_small / ncontacts_large: the contact-count classes of dsdf_dynamics_solve (large <= small: one class).
  * a is a HOST pointer; it is passed to the kernels by value. */
 int dsdf_step_rounds(const dsdf_step_args* a, int n_rounds, int ncontacts_small, int ncontacts_large, void* stream);
 /* Diagnostics: per-kernel device time of the rounds.  dsdf_step_profile(1) makes dsdf_step_rounds bracket every launch

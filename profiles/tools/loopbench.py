@@ -33,8 +33,8 @@ res = {}
 from diffsdfsim_b200 import stepper as _st
 _st.DeviceStepper.TIMING = {}
 import os
-if os.environ.get('DYN_MODE'):
-    _st.DeviceStepper.FORCE_DYN_MODE = int(os.environ['DYN_MODE'])
+if os.environ.get('FORCE_CTA'):
+    _st.DeviceStepper.FORCE_CTA = os.environ['FORCE_CTA'] == '1'
 for mode in modes:
     World3D.device_loop = mode == 'dev'
     for _ in range(2):

@@ -40,27 +40,28 @@ def test_fused_engine_matches_dense_engine():
         np.testing.assert_allclose(a.cpu().numpy(), ref, rtol=1e-4, atol=1e-5 * max(1e-9, np.abs(ref).max()))
 
 
-def test_fused_engine_has_no_contact_limit_of_the_dense_kernel():
-    """16+ contacts per world exceed the dense kernel's shared memory; the fused kernel takes them."""
+def test_fused_plan_has_no_contact_limit_of_the_dense_kernel():
+    """16+ contacts per world exceed the dense kernel's shared memory; the fused kernel takes them (one launch of the
+    one-warp kernel, no workspace)."""
     from diffsdfsim_b200 import _lib
     L = _lib.lib()
     assert L.dsdf_lcp_smem_bytes(12, 6, 170) > 227 * 1024
-    assert L.dsdf_dynamics_solve_smem_bytes(2, 6, 32, 8) < 227 * 1024
+    assert _lib.dynamics_plan(1, 2, 6, 8, 32, 32) == (1, 0)
 
 
-def test_one_cta_kernel_matches_one_warp_kernel():
+def test_forced_one_cta_kernel_matches_one_warp_kernel():
     """The one-CTA instantiation of the solver (per-contact data in a global workspace, block-wide reductions and LU)
     solves the same Newton systems as the one-warp kernel: identical attempts / contact sets, states and gradients to
     round-off."""
     from diffsdfsim_b200.stepper import DeviceStepper
     steps, W = 8, 16
     ta, ga, wa = _rollout('PdipmEngine', steps, W)
-    DeviceStepper.FORCE_DYN_MODE = 1
+    DeviceStepper.FORCE_CTA = True
     try:
         tb, gb, wb = _rollout('PdipmEngine', steps, W)
-        assert wb._stepper.dyn_mode == 1
+        assert wb._stepper.force_cta and wb._stepper.dyn_ws is not None
     finally:
-        DeviceStepper.FORCE_DYN_MODE = None
+        DeviceStepper.FORCE_CTA = False
     assert torch.equal(wa.stats['attempts'], wb.stats['attempts'])
     for (pa, va, ca), (pb, vb, cb) in zip(ta, tb):
         assert torch.equal(ca, cb)
@@ -71,10 +72,11 @@ def test_one_cta_kernel_matches_one_warp_kernel():
         np.testing.assert_allclose(a.cpu().numpy(), ref, rtol=1e-7, atol=1e-9 * max(1e-9, np.abs(ref).max()))
 
 
-def test_more_than_64_contacts_per_world():
+def test_more_than_64_contacts_per_world_on_the_one_cta_kernel():
     """Config 3, gravity + floor variant (16 primitives resting on a pinned floor): ~80-100 simultaneous contacts per
     world, beyond the one-warp kernel's 64 -- runs on the one-CTA kernel, forward and backward, finite and consistent
     between a batch and a single world."""
+    from diffsdfsim_b200 import _lib
     spec = scenes.mixed16_floor(seed=0, steps=5)
     outs = []
     for W in (1, 3):
@@ -85,7 +87,9 @@ def test_more_than_64_contacts_per_world():
             world.step(fixed_dt=True)
             loss = loss + (world.state.p[:, 1:, 4:] ** 2).sum()
         loss.backward()
-        assert world._stepper.dyn_mode == 1
+        # 16 bodies: every world runs on the one-CTA kernel, which needs a workspace even for one contact
+        assert world._stepper.dyn_ws is not None
+        assert _lib.dynamics_plan(W, world.nb, world.num_constraints, world.fric_dirs, 1, 1)[1] > 0
         assert int(world.contact_set.count.max()) > 64, 'the scene must exceed 64 contacts'
         assert torch.isfinite(vel.grad).all() and float(vel.grad.abs().sum()) > 0
         outs.append((world.state.p.detach()[0].clone(), vel.grad[0].clone(), world.contact_set.count[0].clone()))

@@ -132,3 +132,19 @@ def test_undo_step_after_contact_count_change():
         b.step(fixed_dt=True)
         assert torch.equal(a.get_p(), b.get_p()) and torch.equal(a.v, b.v)
         assert torch.equal(a.contact_set.count, b.contact_set.count)
+
+
+def test_many_contacts_identical_to_host_loop():
+    """16 bodies resting on a floor with more than 64 contacts per world: the library picks the one-CTA dynamics kernel
+    for both loops, so they run the same kernels on the same attempts."""
+    W, steps = 3, 4
+    spec = scenes.mixed16_floor(seed=0, steps=steps)
+    gen = torch.Generator().manual_seed(7)
+    vel = torch.tensor([b['vel'] for b in spec['bodies']], dtype=F64).repeat(W, 1, 1)
+    drift = 0.1 * (torch.rand(W, vel.shape[1] - 1, 3, generator=gen, dtype=F64) - 0.5)
+    vel[:, 1:, 3:] += drift * torch.tensor([1.0, 0.0, 1.0], dtype=F64)           # per-world horizontal drift
+    mk = lambda: dict(vel_all=vel.cuda().requires_grad_(True))
+    lf = lambda w: (w.state.p[:, 1:, 4:] ** 2).sum()
+    dev = _rollout(spec, mk, steps, True, lf, maxc=128)
+    host = _rollout(spec, mk, steps, False, lf, maxc=128)
+    assert _same(dev, host) > 64, 'the scene must exceed 64 contacts'
