@@ -36,7 +36,6 @@ SIGNATURES = {
     'dsdf_dynamics_solve': (c_i, [c_p] * 13 + [c_i] * 8 + [c_d, c_i, c_i] + [c_p] * 11),
     'dsdf_dynamics_solve_backward': (c_i, [c_p] * 13 + [c_i] * 10 + [c_p] * 15),
     'dsdf_toc_backward': (c_i, [c_i] * 3 + [c_p] * 9 + [c_d] + [c_p] * 7),
-    'dsdf_contactset_move': (c_i, [c_i, c_i] + [c_p] * 16),
     'dsdf_attempt_commit': (c_i, [c_i] * 3 + [c_p] * 4 + [c_d, c_i, c_i] + [c_p] * 21),
     'dsdf_step_begin': (c_i, [c_p, c_p]),
     'dsdf_step_resume': (c_i, [c_p, c_p]),

@@ -167,24 +167,13 @@ class ContactSet:
         c.pre_ids, c.pre_cnt = self.pre_ids, self.pre_cnt
         return c
 
-    def _segs(self):
-        return [_lib.ptr(getattr(self, k)) for k in ('count', 'status', 'body', 'face', 'abc', 'geo')]
-
-    def gathered(self, src):
-        """New set of len(src) worlds whose world w holds the contacts of world src[w] (src: int64 device tensor)."""
-        n = int(src.numel())
-        c = ContactSet(n, self.maxc, self.flat.device)
-        rc = _lib.call('dsdf_contactset_move', n, self.maxc, _lib.ptr(src), None, None, *self._segs(), *c._segs(),
-                       _lib.stream())
-        _lib.check(rc, 'dsdf_contactset_move')
+    def where(self, mask, other):
+        """New set with the contacts of ``other`` in the worlds where ``mask`` ((W,) bool), else those of ``self``."""
+        c = self.clone()
+        for k in ('count', 'status', 'body', 'face', 'abc', 'geo'):
+            a = getattr(c, k)
+            a.copy_(torch.where(mask.reshape((-1,) + (1,) * (a.dim() - 1)), getattr(other, k), a))
         return c
-
-    def scatter_from(self, other, dst_worlds, src_rows, mask):
-        """self[dst_worlds[i]] = other[src_rows[i]] where mask[i] (int64 / int64 / uint8 device tensors), in place."""
-        rc = _lib.call('dsdf_contactset_move', int(dst_worlds.numel()), self.maxc, _lib.ptr(dst_worlds),
-                       _lib.ptr(src_rows), _lib.ptr(mask), *other._segs(), *self._segs(), _lib.stream())
-        _lib.check(rc, 'dsdf_contactset_move')
-        return self
 
     def clone(self):
         c = ContactSet(self.W, self.maxc, self.flat.device, self.flat.clone())

@@ -9,6 +9,7 @@
 // One thread per world; everything a host loop needs afterwards comes back in four int32 flags (one D2H copy).
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "dsdf_steploop.cuh"
 #include "../../include/dsdf_b200.h"
 
 namespace dsdf {
@@ -30,9 +31,8 @@ attempt_commit_kernel(int W, int nb, int maxc, const unsigned char* __restrict__
     const bool act = active[w] != 0;
     const int st = status_n[w];
     const bool clean = act && !(st & DSDF_CON_PENETRATION);
-    bool accept = clean;
     const double dtw = dt_try[w];
-    if (!strict) accept = clean || (act && dtw < world_dt / 1024.0);                 // world.py:345-347
+    const bool accept = act && attempt_accepted(clean, strict, dtw, world_dt);
     int bad = 0;                                   // bit 0: candidate list overflow (capK), bit 1: contact overflow (maxc)
     if (act && (st & DSDF_CON_CAND_OVERFLOW)) bad |= 1;
     if (accept && (st & DSDF_CON_OVERFLOW)) bad |= 2;
@@ -49,17 +49,8 @@ attempt_commit_kernel(int W, int nb, int maxc, const unsigned char* __restrict__
     const int cn = min(count_n[w], maxc), co = min(count_o[w], maxc);
     if (toc_enabled) {
         for (int k = 0; k < maxc; ++k) {
-            unsigned char m = 0;
-            if (clean && k < cn) {
-                const int a = body_n[((size_t)w * maxc + k) * 2], b = body_n[((size_t)w * maxc + k) * 2 + 1];
-                const int pid = min(a, b) * nb + max(a, b);
-                bool seen = false;
-                for (int j = 0; j < co; ++j) {
-                    const int a2 = body_o[((size_t)w * maxc + j) * 2], b2 = body_o[((size_t)w * maxc + j) * 2 + 1];
-                    seen = seen || (min(a2, b2) * nb + max(a2, b2) == pid);
-                }
-                m = seen ? 0 : 1;
-            }
+            const unsigned char m = clean && k < cn &&
+                                    new_body_pair(body_n + ((size_t)w * maxc + k) * 2, body_o + (size_t)w * maxc * 2, co, nb);
             toc_mask[(size_t)w * maxc + k] = m;
             any_toc |= m;
         }
@@ -89,44 +80,7 @@ attempt_commit_kernel(int W, int nb, int maxc, const unsigned char* __restrict__
     atomicMax(&flags[3], cnt_after);
 }
 
-// Row gather / masked row scatter of a contact set (count, status, body, face, abc, geo) between two batches:
-//   mask == NULL:  dst[i]          = src[idx[i]]                 for i < n   (gather into a compact batch)
-//   mask != NULL:  dst[idx[i]]     = src[sel[i]]  where mask[i]  for i < n   (commit the winning virtual worlds)
-__global__ void __launch_bounds__(128)
-contactset_move_kernel(int n, int maxc, const long long* __restrict__ idx, const long long* __restrict__ sel,
-                       const unsigned char* __restrict__ mask,
-                       const int* __restrict__ count_s, const int* __restrict__ status_s, const int* __restrict__ body_s,
-                       const int* __restrict__ face_s, const double* __restrict__ abc_s, const double* __restrict__ geo_s,
-                       int* __restrict__ count_d, int* __restrict__ status_d, int* __restrict__ body_d,
-                       int* __restrict__ face_d, double* __restrict__ abc_d, double* __restrict__ geo_d) {
-    const int i = blockIdx.x;
-    if (i >= n) return;
-    size_t s, d;
-    if (mask) { if (!mask[i]) return; s = (size_t)sel[i]; d = (size_t)idx[i]; }
-    else { s = (size_t)idx[i]; d = (size_t)i; }
-    if (threadIdx.x == 0) { count_d[d] = count_s[s]; status_d[d] = status_s[s]; }
-    const int nc = min(count_s[s], maxc);
-    for (int t = threadIdx.x; t < nc * 2; t += blockDim.x) body_d[d * maxc * 2 + t] = body_s[s * maxc * 2 + t];
-    for (int t = threadIdx.x; t < nc; t += blockDim.x) face_d[d * maxc + t] = face_s[s * maxc + t];
-    for (int t = threadIdx.x; t < nc * 3; t += blockDim.x) abc_d[d * maxc * 3 + t] = abc_s[s * maxc * 3 + t];
-    for (int t = threadIdx.x; t < nc * 10; t += blockDim.x) geo_d[d * maxc * 10 + t] = geo_s[s * maxc * 10 + t];
-}
-
 }  // namespace dsdf
-
-extern "C" int dsdf_contactset_move(int n, int maxc, const long long* idx, const long long* sel,
-                                    const unsigned char* mask,
-                                    const int32_t* count_s, const int32_t* status_s, const int32_t* body_s,
-                                    const int32_t* face_s, const double* abc_s, const double* geo_s,
-                                    int32_t* count_d, int32_t* status_d, int32_t* body_d, int32_t* face_d,
-                                    double* abc_d, double* geo_d, void* stream) {
-    if (n < 0 || maxc <= 0 || !idx || (mask && !sel)) return -1;
-    if (n == 0) return 0;
-    dsdf::contactset_move_kernel<<<n, 128, 0, (cudaStream_t)stream>>>(n, maxc, idx, sel, mask, count_s, status_s, body_s,
-                                                                     face_s, abc_s, geo_s, count_d, status_d, body_d,
-                                                                     face_d, abc_d, geo_d);
-    return (int)cudaGetLastError();
-}
 
 extern "C" int dsdf_attempt_commit(int W, int nb, int maxc, const unsigned char* active, const double* dt_try,
                                    const double* t, const double* end_t, double world_dt, int strict, int toc_enabled,

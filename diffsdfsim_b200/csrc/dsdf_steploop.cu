@@ -128,8 +128,7 @@ step_commit_kernel(const __grid_constant__ Args a) {
         for (int d = 0; d < deff; ++d) {
             const int vv = d * n + i;
             const int st = a.status_v[vv];
-            const bool clean = !(st & DSDF_CON_PENETRATION);
-            const bool acc = clean || (!a.strict && a.dt_raw_v[vv] < a.world_dt / 1024.0);     // world.py:345-347
+            const bool acc = attempt_accepted(!(st & DSDF_CON_PENETRATION), a.strict, a.dt_raw_v[vv], a.world_dt);
             if (st & DSDF_CON_CAND_OVERFLOW) pause |= DSDF_STEP_CAPK;
             if (acc && (st & DSDF_CON_OVERFLOW)) pause |= DSDF_STEP_MAXC;
             if (acc && win < 0) win = d;
@@ -172,17 +171,9 @@ step_commit_kernel(const __grid_constant__ Args a) {
             // time-of-contact set (world.py:273-274): contacts whose body pair had no contact at the start of the sub-step
             int any_toc = 0;
             for (int kk = lane; kk < maxc; kk += 32) {
-                unsigned char m = 0;
-                if (a.toc_enabled && clean && kk < cn) {
-                    const int b1 = a.body_v[((size_t)vv * maxc + kk) * 2], b2 = a.body_v[((size_t)vv * maxc + kk) * 2 + 1];
-                    const int pid = min(b1, b2) * nb + max(b1, b2);
-                    bool seen = false;
-                    for (int j = 0; j < co; ++j) {
-                        const int o1 = a.body[((size_t)w * maxc + j) * 2], o2 = a.body[((size_t)w * maxc + j) * 2 + 1];
-                        seen = seen || (min(o1, o2) * nb + max(o1, o2) == pid);
-                    }
-                    m = seen ? 0 : 1;
-                }
+                const unsigned char m = a.toc_enabled && clean && kk < cn &&
+                                        new_body_pair(a.body_v + ((size_t)vv * maxc + kk) * 2, a.body + (size_t)w * maxc * 2,
+                                                      co, nb);
                 S.toc_mask[r * maxc + kk] = m;
                 any_toc |= m;
             }

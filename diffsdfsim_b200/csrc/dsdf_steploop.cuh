@@ -24,4 +24,24 @@ enum {
 };
 // true when this launch has nothing to do (a previous kernel asked the host for help, or every world is done)
 __device__ __forceinline__ bool loop_idle(const int* ctrl) { return ctrl[CT_ABORT] != 0 || ctrl[CT_NACT] == 0; }
+
+// The two rules of the reference that both commit kernels (step_commit_kernel here, attempt_commit_kernel of the
+// host-driven loop in dsdf_step.cu) apply to an attempt.
+//
+// world.py:345-347: a sub-step is accepted when its state does not penetrate (clean), or, when not strict, once its dt
+// fell below world_dt / 2^10 (give up halving).
+__device__ __forceinline__ bool attempt_accepted(bool clean, bool strict, double dt, double world_dt) {
+    return clean || (!strict && dt < world_dt / 1024.0);
+}
+// world.py:273-274: the contact with body pair `pair` (2 ints) is new when none of the n_old contacts of the set at
+// the start of the sub-step (old_pairs, 2 ints each) joins the same two bodies.
+__device__ __forceinline__ bool new_body_pair(const int* pair, const int* old_pairs, int n_old, int nb) {
+    const int pid = min(pair[0], pair[1]) * nb + max(pair[0], pair[1]);
+    bool seen = false;
+    for (int j = 0; j < n_old; ++j) {
+        const int a = old_pairs[2 * j], b = old_pairs[2 * j + 1];
+        seen = seen || (min(a, b) * nb + max(a, b) == pid);
+    }
+    return !seen;
+}
 }  // namespace dsdf

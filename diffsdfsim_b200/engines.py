@@ -191,18 +191,8 @@ class PdipmEngine(Engine):
             new_v = self.solve(world, dt, active).reshape(world.W, -1)
         return new_v if world.batched else new_v[0]
 
-    def solve(self, world, dt, active=None, inputs=None):
-        """dt: (W,) tensor (may carry grad).  Returns new_v (W,nb,6).  ``inputs`` (optional) replaces the world's own
-        state by explicit per-slot tensors: dict(p, v, mass, Ibody, fric, rest, f, geo, count, body)."""
-        if inputs is not None:
-            cfg = dict(fric_dirs=world.fric_dirs, max_iter=self.max_iter, stop_contact_grad=world.stop_contact_grad,
-                       stop_friction_grad=world.stop_friction_grad,
-                       ni_smem=max(world.max_nc, 1) * (2 + world.fric_dirs), nc_smem=max(world.max_nc, 1))
-            i = inputs
-            new_v, status = _DynamicsFused.apply(i['p'], i['v'], i['mass'], i['Ibody'], i['fric'], i['rest'], i['f'], dt,
-                                                 i['geo'], i['count'], i['body'], world.eq_rows, active, cfg)
-            self.last_status = status
-            return new_v
+    def solve(self, world, dt, active=None):
+        """dt: (W,) tensor (may carry grad).  Returns new_v (W,nb,6)."""
         st = world.state
         f = world.step_forces()
         cfg = dict(fric_dirs=world.fric_dirs, max_iter=self.max_iter, stop_contact_grad=world.stop_contact_grad,

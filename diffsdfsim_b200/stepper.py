@@ -171,6 +171,12 @@ class DeviceStepper:
     INITIAL_SLOTS = 2
     TIMING = None           # set to {} to accumulate host wall-clock seconds per phase of run() (diagnostics)
     FORCE_CTA = False       # tests: run every world through the one-CTA dynamics kernel
+    # speculative halving (W >= 64): the retries dt, dt/2, ... of the few still-active worlds run in ONE round as virtual
+    # worlds, the first accepted attempt in the reference's order wins (step_prep_kernel / step_commit_kernel).
+    # False: one halving per round, the same results in more rounds.
+    SPECULATE = True
+    SPEC_DEPTH = 3          # halvings tried at once when <= W/8 worlds are still active
+    SPEC_DEPTH2 = 6         # ... when <= W/32 worlds are still active
 
     @classmethod
     def _tick(cls, name, t0):
@@ -182,11 +188,11 @@ class DeviceStepper:
         _lib.lib()
         self.W, self.nb, self.dev = world.W, world.nb, world.device
         W, dev = self.W, self.dev
-        self.depth = world.SPEC_DEPTH if world.speculate else 1
-        self.spec_threshold = W // 8 if (world.speculate and W >= 64) else 0
+        self.depth = self.SPEC_DEPTH if self.SPECULATE else 1
+        self.spec_threshold = W // 8 if (self.SPECULATE and W >= 64) else 0
         # second level: when hardly any world is left, try six halvings at once (a world that ends up giving up at
         # dt / 2^10 then needs two rounds instead of four)
-        self.depth2 = world.SPEC_DEPTH2 if (world.speculate and world.SPEC_DEPTH2 > self.depth) else 0
+        self.depth2 = self.SPEC_DEPTH2 if (self.SPECULATE and self.SPEC_DEPTH2 > self.depth) else 0
         self.spec_threshold2 = W // 32 if (self.depth2 and W >= 64) else 0
         self.vcap = max(W, self.depth * self.spec_threshold, self.depth2 * self.spec_threshold2)
         self.ctrl = torch.zeros(CT_WORDS, dtype=I32, device=dev)

@@ -101,9 +101,6 @@ class TimeOfContactNative(torch.autograd.Function):
 
 class World3D:
     max_rounds_per_step = 256
-    speculate = True       # evaluate dt, dt/2, dt/4 of the few still-active worlds in ONE round (see _attempt_speculative)
-    SPEC_DEPTH = 3
-    SPEC_DEPTH2 = 6        # device loop only: halvings tried at once when <= W/32 worlds are still active
     toc_native = True      # False: the torch-autograd restatement of World.H (TimeOfContact) on the affected worlds
     device_loop = True     # the per-world step state machine runs on the device (stepper.py / csrc/dsdf_steploop.cu);
                            # False: the host-driven round loop below (one synchronisation per round)
@@ -187,7 +184,6 @@ class World3D:
         # contact detection set-up (replaces the py3ode HashSpace of world.py:69-72)
         self.table = GeometryTable(self.bodies, W, dev)
         self.vert_leaves = [self.bodies[i].verts.to(dev) for i in self.table.vert_leaf_ids]   # differentiable meshes
-        self._shared_geometry = bool((self.table.rows['vstride'] == 0).all() and (self.table.rows['gstride'] == 0).all())
         self.pairs = [(i, j) for i in range(nb) for j in range(i + 1, nb)
                       if self.bodies[j] not in self.bodies[i].no_contact]
         self.detector = ContactDetector(self.table, self.pairs, W, nb, dev, capK=capK, maxc=maxc,
@@ -410,7 +406,7 @@ class World3D:
         dt_try = torch.full((W,), float(self.dt), dtype=F64, device=dev)
         active = torch.ones(W, dtype=torch.uint8, device=dev)
         had = torch.zeros(W, dtype=torch.bool, device=dev)
-        rounds, n_active = 0, W
+        rounds = 0
         while True:
             rounds += 1
             if rounds > self.max_rounds_per_step:
@@ -420,11 +416,8 @@ class World3D:
                 raise RuntimeError('step did not complete in %d attempts: worlds %s keep penetrating (dt < %.3g); '
                                    'use strict_no_penetration=False or a smaller dt'
                                    % (self.max_rounds_per_step, stuck, float(dt_try.min())))
-            if self._use_speculation(n_active):
-                accept, dt_try, active, n_active = self._attempt_speculative(active, dt_try, end_t)
-            else:
-                self.stats['attempts'] += active
-                accept, dt_try, active, n_active = self._attempt(active, dt_try, end_t)
+            self.stats['attempts'] += active
+            accept, dt_try, active, n_active = self._attempt(active, dt_try, end_t)
             had |= accept.bool() & (self.contact_set.count > 0)
             if not n_active:
                 break
@@ -451,9 +444,7 @@ class World3D:
             m3 = m[:, None, None]
             st.p, st.v = torch.where(m3, p0, st.p), torch.where(m3, v0, st.v)
             self.contact_geo = torch.where(m3, geo, self.contact_geo)
-            idx = torch.arange(self.W, device=self.device)
-            with self._on_device():
-                self.contact_set = self.contact_set.clone().scatter_from(cs, idx, idx, m.to(torch.uint8))
+            self.contact_set = self.contact_set.where(m, cs)
             self.t = torch.where(m, t0, self.t)
             self.toc_flag = torch.where(m, toc0, self.toc_flag)
             self.last_dt = torch.where(m, last0, self.last_dt)
@@ -560,100 +551,6 @@ class World3D:
         self.contact_geo = torch.where(a3, geo, self.contact_geo)
         self.contact_set = cs
         self.max_nc = max(int(self.max_nc), int(cs.count.max()))
-
-    def _use_speculation(self, n_active):
-        """Speculate when few worlds are still active (their slots are plentiful) and no body has per-world geometry
-        (the contact kernels address per-world meshes / grids by slot index)."""
-        return (self.speculate and self.W >= 64 and 0 < n_active <= self.W // 8 and self._shared_geometry
-                and self.shape_t is None and not self.vert_leaves and not self.post_stab and not self._general_joints)
-
-    def _attempt_speculative(self, active, dt_try, end_t):
-        """One round that tries dt, dt/2 and dt/4 of every still-active world AT ONCE.
-
-        The reference retries a rejected sub-step with half the time step from the same start state (world.py:344-356),
-        so the attempts of one world are independent of each other: the few still-active worlds are gathered into a
-        compact batch of SPEC_DEPTH x n virtual worlds (attempt d of world i uses dt / 2^d), the same kernels run on that
-        small batch, and the FIRST accepted attempt in the reference's order is committed -- the same state, contacts,
-        time-of-contact flags and attempt count as trying them one after the other, in a third of the (latency-bound,
-        nearly empty) rounds.  Two host synchronisations per round.
-        """
-        st = self.state
-        nb, dev, D = self.nb, self.device, self.SPEC_DEPTH
-        toc = self.time_of_contact_diff
-        act_idx = active.nonzero().flatten()                          # (n,) still-active worlds            [sync 1]
-        n = act_idx.numel()
-        V = D * n                                                      # virtual worlds: attempt-major (d * n + i)
-        src = act_idx.repeat(D)
-        g = lambda x: x.index_select(0, src)
-        scale = torch.repeat_interleave(0.5 ** torch.arange(D, dtype=F64, device=dev), n)
-        dt_v = g(dt_try) * scale                                       # dt, dt/2, dt/4 (exact: powers of two)
-        act_v = torch.ones(V, dtype=torch.uint8, device=dev)
-        old = self.contact_set.gathered(src)
-        geo_in, p_in, v_in, f_in = g(self.contact_geo), g(st.p), g(st.v), g(self.step_forces())
-        t_in, last_dt_in, mass_in, shape_in = g(self.t), g(self.last_dt), g(st.mass), g(self.shape)
-        end_in = g(end_t) if end_t is not None else None
-        toc_flag = g(self.toc_flag) if toc else torch.zeros(V, dtype=torch.uint8, device=dev)
-        dt_ = dt_v
-        if toc and self._any_toc_flag:
-            dt_ = torch.where(toc_flag.bool(), -last_dt_in + (last_dt_in.detach() + dt_v), dt_v)
-        inputs = dict(p=p_in, v=v_in, mass=mass_in, Ibody=g(st.Ibody), fric=g(st.fric), rest=g(st.rest), f=f_in,
-                      geo=geo_in, count=old.count, body=old.body)
-        new_v = self.engine.solve(self, dt_, act_v, inputs=inputs)
-        p_try = ops.integrate(p_in, new_v, dt_, act_v)
-        cs = old.clone()
-        self.detector.detect(p_try.detach(), shape_in, cs, act_v, eps=self.eps, tol=self.tol,
-                             fd_eps=Defaults3D.EPSILON, body_eps=self.body_eps, detach_b2=self.detach_contact_b2)
-        geo = differentiable_geometry(p_try, shape_in, cs, self.table, Defaults3D.EPSILON, self.detach_contact_b2)
-        u8 = lambda *shape: torch.empty(*shape, dtype=torch.uint8, device=dev)
-        accept, active_next, toc_now, toc_mask = u8(V), u8(V), u8(V), u8(V, self.maxc)
-        t_new, dt_next = torch.empty_like(dt_v), torch.empty_like(dt_v)
-        flags = torch.empty(4, dtype=torch.int32, device=dev)
-        rc = _lib.call('dsdf_attempt_commit', V, nb, self.maxc, _lib.ptr(act_v), _lib.ptr(dt_v), _lib.ptr(t_in),
-                       _lib.ptr(end_in), float(self.dt), int(self.strict_no_pen), int(toc),
-                       _lib.ptr(old.count), _lib.ptr(old.status), _lib.ptr(old.body), _lib.ptr(old.face),
-                       _lib.ptr(old.abc), _lib.ptr(old.geo), _lib.ptr(cs.count), _lib.ptr(cs.status),
-                       _lib.ptr(cs.body), _lib.ptr(cs.face), _lib.ptr(cs.abc), _lib.ptr(cs.geo), _lib.ptr(toc_flag),
-                       _lib.ptr(accept), _lib.ptr(t_new), _lib.ptr(dt_next), _lib.ptr(active_next), _lib.ptr(toc_now),
-                       _lib.ptr(toc_mask), _lib.ptr(flags), _lib.stream())
-        _lib.check(rc, 'dsdf_attempt_commit')
-        # first accepted attempt of every active world, in the reference's order dt, dt/2, dt/4
-        acc = accept.reshape(D, n).bool()
-        any_acc = acc.any(0)
-        first = acc.to(torch.uint8).argmax(0)                          # first True (0 when none: masked by any_acc)
-        sel = first * n + torch.arange(n, device=dev)                  # winning virtual world of active world i
-        nxt_act = torch.where(any_acc, active_next.index_select(0, sel).bool(), torch.ones_like(any_acc))
-        cnt = torch.where(any_acc, cs.count.index_select(0, sel), self.contact_set.count.index_select(0, act_idx))
-        info = torch.cat([flags, torch.stack([nxt_act.sum(), cnt.max()]).to(torch.int32)]).tolist()             # [sync 2]
-        if info[0]:
-            # an overflow in ANY virtual world (even a discarded one) grows the buffers; nothing has been committed yet
-            self._grow_capacity(info[0])
-            return self._attempt_speculative(active, dt_try, end_t)
-        if toc and info[2]:
-            dt_h = TimeOfContactNative.apply(dt_, p_try, new_v, geo, f_in, mass_in, toc_mask, cs.body)
-            p_redo = ops.integrate(p_in, new_v, dt_h, toc_now)
-            tn = toc_now.bool()
-            p_try = torch.where(tn[:, None, None], p_redo, p_try)
-            last_dt_in = torch.where(tn, dt_h, last_dt_in)
-            self._any_toc_flag = True
-        self.stats['attempts'][act_idx] += torch.where(any_acc, first + 1, torch.full_like(first, D))
-        # commit: world i takes the outputs of its winning attempt, or stays as it was and goes on halving
-        # (fixed-shape masked updates of the n active rows: no data-dependent shapes, hence no hidden synchronisation)
-        def put(cur, new_rows):
-            keep = any_acc.reshape((n,) + (1,) * (cur.dim() - 1))
-            return cur.index_copy(0, act_idx, torch.where(keep, new_rows.index_select(0, sel),
-                                                          cur.index_select(0, act_idx)))
-        st.p, st.v, self.contact_geo = put(st.p, p_try), put(st.v, new_v), put(self.contact_geo, geo)
-        self.contact_set = self.contact_set.clone().scatter_from(cs, act_idx, sel, any_acc.to(torch.uint8))
-        self.t = put(self.t, t_new)
-        if toc:
-            self.last_dt, self.toc_flag = put(self.last_dt, last_dt_in), put(self.toc_flag, toc_flag)
-        dt_act = dt_try.index_select(0, act_idx)
-        dt_out = dt_try.index_copy(0, act_idx, torch.where(any_acc, dt_next.index_select(0, sel), dt_act / (2 ** D)))
-        act_out = torch.zeros_like(active).index_copy(0, act_idx, nxt_act.to(torch.uint8))
-        acc_w = torch.zeros_like(active).index_copy(0, act_idx, any_acc.to(torch.uint8))
-        # the dynamics kernel sizes its shared memory by the largest contact count over ALL worlds
-        self.max_nc = max(int(info[5]), int(self.max_nc))      # (an upper bound: the other worlds did not change)
-        return acc_w, dt_out, act_out, int(info[4])
 
     MAX_CAPK, MAX_MAXC = 1024, 512     # candidate list: shared memory of the contact kernel; contacts: tape / workspace sizes
 

@@ -312,15 +312,6 @@ int dsdf_toc_backward(int W, int nb, int maxc, const double* dt, const unsigned 
                       const double* f, const double* mass, const double* g_dt_h, double base_tol,
                       double* g_dt, double* gp, double* gv, double* ggeo, double* gf, double* gmass, void* stream);
 
-/* Row gather / masked row scatter of a contact set between two batches (host-side scheduling aid: the still-active
- * worlds of a step are retried as a compact batch).  mask == NULL: dst[i] = src[idx[i]], i < n.
- * mask != NULL: dst[idx[i]] = src[sel[i]] where mask[i].  idx / sel are int64 device arrays. */
-int dsdf_contactset_move(int n, int maxc, const long long* idx, const long long* sel, const unsigned char* mask,
-                         const int32_t* count_s, const int32_t* status_s, const int32_t* body_s,
-                         const int32_t* face_s, const double* abc_s, const double* geo_s,
-                         int32_t* count_d, int32_t* status_d, int32_t* body_d, int32_t* face_d,
-                         double* abc_d, double* geo_d, void* stream);
-
 /* ------------------------------------------------- device-resident step ----
  * World.step / World.step_dt (lcp_physics/physics/world.py:119-139, 241-379) as a state machine that lives on the
  * device: the host launches ROUNDS (one attempt of every world still inside its step: prep -> solve -> move ->

@@ -40,6 +40,29 @@ def test_fused_engine_matches_dense_engine():
         np.testing.assert_allclose(a.cpu().numpy(), ref, rtol=1e-4, atol=1e-5 * max(1e-9, np.abs(ref).max()))
 
 
+def test_dense_engine_runs_the_dense_operator_in_every_round():
+    """64 spheres dropped from heights spread over 2 m: at every step only a few worlds touch the floor and retry with
+    a halved dt, so most retry rounds have a handful of active worlds.  Every round of the dense engine, forward and
+    backward, still goes through the dense LCP kernels and never through the fused solver."""
+    from diffsdfsim_b200 import _lib
+    W, steps = 64, 14
+    gen = torch.Generator().manual_seed(3)
+    pos = torch.zeros(W, 3, dtype=F64)
+    pos[:, 1] = 0.62 + 2.0 * torch.rand(W, generator=gen, dtype=F64)
+    pos = pos.cuda().requires_grad_(True)
+    spec = scenes.bouncing_sphere(floor=(6.0, 1.0, 6.0), steps=steps, floor_tri=0.2, subdivisions=3)
+    world = scenes.build_world(spec, device='cuda', params=dict(pos=pos), engine='DensePdipmEngine', maxc=12)
+    _lib.reset_counters()
+    loss = 0.
+    for _ in range(steps):
+        world.step(fixed_dt=True)
+        loss = loss + (world.bodies[-1].pos ** 2).sum()
+    loss.backward()
+    assert int(world.stats['attempts'].max()) > steps, 'the scene must reject and retry sub-steps'
+    assert 'dsdf_dynamics_solve' not in _lib.LAUNCHES and 'dsdf_dynamics_solve_backward' not in _lib.LAUNCHES
+    assert 'dsdf_lcp_forward' in _lib.LAUNCHES
+
+
 def test_fused_plan_has_no_contact_limit_of_the_dense_kernel():
     """16+ contacts per world exceed the dense kernel's shared memory; the fused kernel takes them (one launch of the
     one-warp kernel, no workspace)."""

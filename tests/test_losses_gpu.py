@@ -109,3 +109,57 @@ def test_run_world_fixed_dt_matches_the_reference_function(flag):
     for name, leaf in (('gpos', pos), ('gvel', vel)):
         ref = g[k + '_' + name]
         np.testing.assert_allclose(leaf.grad.cpu().numpy().reshape(-1), ref, rtol=1e-4, atol=1e-5 * max(1e-9, np.abs(ref).max()))
+
+
+def test_batched_detach_2nd_bounce_matches_each_world_alone():
+    """run_world_fixed_dt(detach_2nd_bounce=True) on a batch of spheres dropped from different heights: the masked
+    undo_step / detach_state fire at different steps in different worlds, and every world ends bit for bit where it
+    ends alone.  A batch steps in lock-step on the host clock, so 'alone' is that world stepped as many times, with the
+    same rule applied through the unmasked undo_step() / detach_state() (the single-world path the reference golden
+    above pins)."""
+    from diffsdfsim_b200 import scenes
+    from diffsdfsim_b200.losses import run_world_fixed_dt
+    heights = [0.62, 0.75, 0.9, 1.05]
+    W = len(heights)
+    spec = scenes.bouncing_sphere(floor=(4.0, 1.0, 4.0), steps=0, floor_tri=0.2, subdivisions=3)
+    pos0 = torch.tensor([[0.0, h, 0.0] for h in heights], dtype=F64)
+    vel0 = torch.tensor([[0.0, 0.0, 0.0, 1.0, 0.0, 0.3]] * W, dtype=F64)
+    term = lambda world: (world.bodies[-1].pos ** 2).sum(-1) + 0.1 * (world.bodies[-1].v ** 2).sum(-1)
+
+    pos, vel = pos0.cuda().requires_grad_(True), vel0.cuda().requires_grad_(True)
+    batch = scenes.build_world(spec, device='cuda', params=dict(pos=pos, vel=vel))
+    terms, step = [], batch.step
+
+    def recording_step(fixed_dt=False):
+        had = step(fixed_dt=fixed_dt)
+        terms.append(term(batch))
+        return had
+    batch.step = recording_step
+    n_steps = run_world_fixed_dt(batch, 0.9, detach_2nd_bounce=True)
+    sum(terms).sum().backward()
+
+    fired = []
+    for w in range(W):
+        pw, vw = pos0[w:w + 1].cuda().requires_grad_(True), vel0[w:w + 1].cuda().requires_grad_(True)
+        world = scenes.build_world(spec, device='cuda', params=dict(pos=pw, vel=vw))
+        loss, contact_steps, fired_w = 0., 0, []
+        for k in range(n_steps):
+            had = world.step(fixed_dt=True)
+            loss = loss + term(world).sum()
+            contact_steps += int(had)
+            if had and contact_steps > 1:
+                world.undo_step()
+                world.detach_state()
+                contact_steps = 0
+                fired_w.append(k)
+        loss.backward()
+        fired.append(fired_w)
+        assert torch.equal(batch.get_p()[w], world.get_p()), w
+        assert torch.equal(batch.v[w], world.v), w
+        assert torch.equal(batch.t[w:w + 1], world.t), w
+        assert torch.equal(batch.contact_set.count[w:w + 1], world.contact_set.count), w
+        for leaf, lw in ((pos, pw), (vel, vw)):
+            np.testing.assert_allclose(leaf.grad[w].cpu().numpy(), lw.grad[0].cpu().numpy(), rtol=1e-12,
+                                       atol=1e-14, err_msg='world %d' % w)
+    assert sum(1 for f in fired if f) >= 2 and len({tuple(f) for f in fired}) > 1, \
+        'the undo must fire in several worlds, at different steps: %s' % fired

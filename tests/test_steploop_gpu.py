@@ -61,7 +61,9 @@ def test_box_on_plane_batch_identical_to_host_loop():
     lf = lambda w: (w.bodies[-1].pos ** 2).sum() + 0.1 * (w.bodies[-1].v ** 2).sum()
     dev, host = _rollout(spec, mk, steps, True, lf), _rollout(spec, mk, steps, False, lf)
     assert _same(dev, host) >= 4
-    assert dev['rounds'] <= host['rounds'] + 6, 'same speculation policy: about the same number of rounds'
+    # the device loop speculates, the host loop retries one halving at a time; a round in which worlds of the device loop
+    # pause for buffer growth (tape slots, contact capacity) counts as a round too
+    assert dev['rounds'] <= host['rounds'] + 6, 'device loop rounds %d, host loop rounds %d' % (dev['rounds'], host['rounds'])
     assert dev['syncs'] <= 2 * steps, 'host synchronisations: one per step + one per buffer growth (%d for %d steps)' % (dev['syncs'], steps)
 
 

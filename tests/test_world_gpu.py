@@ -406,11 +406,11 @@ def test_gradient_stopping_flags_match_oracle(flag):
                                        err_msg=f'{flag}: world {w} grad {k}')
 
 
-def test_speculative_halving_is_bitwise_identical_to_sequential_retries():
-    """Trying dt, dt/2, dt/4 of the few still-active worlds in one round (borrowed slots, first accepted attempt in
-    the reference's order wins) gives the same states, contacts, gradients AND attempt counts as retrying one after
-    the other -- with fewer rounds."""
-    from diffsdfsim_b200.world import World3D
+def test_device_loop_speculative_halving_is_bitwise_identical_to_sequential_retries():
+    """Device loop (DeviceStepper.SPECULATE): trying dt, dt/2, dt/4 of the few still-active worlds in one round (borrowed
+    slots, first accepted attempt in the reference's order wins) gives the same states, contacts, gradients AND attempt
+    counts as retrying one after the other -- with fewer rounds."""
+    from diffsdfsim_b200.stepper import DeviceStepper
     W, steps = 4096, 24
     gen = torch.Generator().manual_seed(0)
     mass = 0.9 + 0.2 * torch.rand(W, generator=gen, dtype=F64)
@@ -419,7 +419,7 @@ def test_speculative_halving_is_bitwise_identical_to_sequential_retries():
     spec = scenes.box_on_plane(steps=steps)
     out = {}
     for flag in (False, True):
-        World3D.speculate = flag
+        DeviceStepper.SPECULATE = flag
         try:
             params = dict(mass=mass.cuda().requires_grad_(True), fric_coeff=fric.cuda().requires_grad_(True),
                           push=push.cuda().requires_grad_(True))
@@ -433,7 +433,7 @@ def test_speculative_halving_is_bitwise_identical_to_sequential_retries():
                          world.stats['attempts'].clone(), {k: v.grad.clone() for k, v in params.items()},
                          sum(world.stats['rounds']), world.t.clone())
         finally:
-            World3D.speculate = True
+            DeviceStepper.SPECULATE = True
     a, b = out[False], out[True]
     assert b[5] < a[5], 'speculation must save rounds (%d vs %d)' % (b[5], a[5])
     assert torch.equal(a[3], b[3]), 'attempt counts'
