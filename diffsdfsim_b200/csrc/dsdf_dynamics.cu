@@ -10,55 +10,15 @@
 // inputs (poses, velocities, masses, inertias, friction, restitution, forces, dt, contact geometry) using
 // forward-mode duals of the same row-construction code.
 #include "dsdf_math.cuh"
+#include "dsdf_contact_rows.cuh"
 #include "../../include/dsdf_b200.h"
 
 namespace dsdf {
-
-// e_k x n with k = argmin |n_k| (first on ties)   physics3d/utils.py:247-256
-template <class S> __device__ __forceinline__ V3<S> tangent_seed(V3<S> n) {
-    const double ax = fabs(val(n.x)), ay = fabs(val(n.y)), az = fabs(val(n.z));
-    int k = 0;
-    double m = ax;
-    if (ay < m) { m = ay; k = 1; }
-    if (az < m) { k = 2; }
-    S one = cst(n.x, 1.0), zero = cst(n.x, 0.0);
-    V3<S> e = v3<S>(k == 0 ? one : zero, k == 1 ? one : zero, k == 2 ? one : zero);
-    return cross(e, n);
-}
-
-// friction directions (world.py:84-94): fd = 8 -> [d1,d2,d3,d4,-d1..-d4]; fd = 4 -> [d1,d2,-d1,-d2]
-template <class S> __device__ __forceinline__ void friction_dirs(V3<S> n, int fd, V3<S>* dirs) {
-    V3<S> d1 = normalize3(tangent_seed(n));
-    V3<S> d2 = normalize3(cross(d1, n));
-    const int half = fd / 2;
-    dirs[0] = d1; dirs[1] = d2;
-    if (fd == 8) {
-        V3<S> d3 = normalize3(d1 + d2);
-        V3<S> d4 = normalize3(cross(d3, n));
-        dirs[2] = d3; dirs[3] = d4;
-    }
-    for (int r = 0; r < half; ++r) dirs[half + r] = neg(dirs[r]);
-}
 
 // Row blocks of one direction d at contact point pt: [pt x d, d]
 template <class S> __device__ __forceinline__ void jac_block(V3<S> pt, V3<S> d, S* out6) {
     V3<S> c = cross(pt, d);
     out6[0] = c.x; out6[1] = c.y; out6[2] = c.z; out6[3] = d.x; out6[4] = d.y; out6[5] = d.z;
-}
-
-// world-frame inertia block R I R^T
-template <class S> __device__ __forceinline__ M3<S> world_inertia(Q4<S> q, const S* I9) {
-    M3<S> R = q2mat(q);
-    M3<S> I;
-#pragma unroll
-    for (int e = 0; e < 9; ++e) I.m[e] = I9[e];
-    M3<S> RI = mat_mul(R, I);
-    M3<S> Rt;
-#pragma unroll
-    for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int j = 0; j < 3; ++j) Rt.m[3 * i + j] = R.m[3 * j + i];
-    return mat_mul(RI, Rt);
 }
 
 __global__ void __launch_bounds__(128)
@@ -89,7 +49,7 @@ assemble_kernel(const double* __restrict__ p, const double* __restrict__ v, cons
     // mass matrix blocks
     for (int b = tid; b < nb; b += nt) {
         const double* pb = p + ((size_t)w * nb + b) * 7;
-        M3<double> Iw = world_inertia<double>(q4<double>(pb[0], pb[1], pb[2], pb[3]), Ibody + ((size_t)w * nb + b) * 9);
+        M3<double> Iw = winertia<double>(q4<double>(pb[0], pb[1], pb[2], pb[3]), Ibody + ((size_t)w * nb + b) * 9);
         const double m = mass[(size_t)w * nb + b];
         for (int i = 0; i < 3; ++i) {
             for (int j = 0; j < 3; ++j) Qw[(6 * b + i) * nz + 6 * b + j] = Iw.m[3 * i + j];
@@ -115,7 +75,7 @@ assemble_kernel(const double* __restrict__ p, const double* __restrict__ v, cons
         const double e = (rest[(size_t)w * nb + i1] + rest[(size_t)w * nb + i2]) / 2;
         hw[c] = jv * e;
         V3<double> dirs[8];
-        friction_dirs<double>(n, fd, dirs);
+        fdirs<double>(n, fd, dirs);
         for (int r = 0; r < fd; ++r) {
             const int row = nc + fd * c + r;
             jac_block<double>(p1, dirs[r], r1);
@@ -148,7 +108,7 @@ __device__ __forceinline__ void contact_rows(V3<S> n, V3<S> p1, V3<S> p2, int fd
     if (jc_part) { jac_block<S>(p1, n, jc1); jac_block<S>(p2, n, jc2); }
     if (jf_part) {
         V3<S> dirs[8];
-        friction_dirs<S>(n, fd, dirs);
+        fdirs<S>(n, fd, dirs);
         for (int r = 0; r < fd; ++r) { jac_block<S>(p1, dirs[r], jf1[r]); jac_block<S>(p2, dirs[r], jf2[r]); }
     }
 }
@@ -220,7 +180,7 @@ assemble_bwd_kernel(const double* __restrict__ p, const double* __restrict__ v, 
             Dual I9[9];
             for (int e = 0; e < 9; ++e) I9[e] = Dual(Ib[e], seed == 4 + e ? 1.0 : 0.0);
             Q4<Dual> q = q4<Dual>(Dual(pb[0], seed == 0), Dual(pb[1], seed == 1), Dual(pb[2], seed == 2), Dual(pb[3], seed == 3));
-            M3<Dual> Iw = world_inertia<Dual>(q, I9);
+            M3<Dual> Iw = winertia<Dual>(q, I9);
             double acc = 0.0;
             for (int i = 0; i < 3; ++i)
                 for (int j = 0; j < 3; ++j) acc += dMb[6 * i + j] * Iw.m[3 * i + j].d;

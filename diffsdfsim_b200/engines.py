@@ -7,7 +7,7 @@ Backward = dsdf_lcp_backward + dsdf_dynamics_assemble_backward.
 """
 import torch
 
-from . import _lib
+from . import _lib, ops
 from .lcp import lcp_backward_raw, lcp_solve_raw
 
 F64 = torch.float64
@@ -93,12 +93,6 @@ class _Dynamics(torch.autograd.Function):
         return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, None, None, (dA if want_A else None), None, None, None
 
 
-def _fused_plan(W, nb, neq, fd, C, dev):
-    """Kernel launches of dsdf_dynamics_solve(_backward) for one class of C contacts and the workspace they need."""
-    n, nbytes = _lib.dynamics_plan(W, nb, neq, fd, C, C)
-    return n, (torch.empty(nbytes // 8 + 1, dtype=F64, device=dev) if nbytes else None)
-
-
 class _DynamicsFused(torch.autograd.Function):
     """dsdf_dynamics_solve / dsdf_dynamics_solve_backward: structure-exploiting KKT, one class of ``nc_smem`` contacts
     (the library picks the kernels, as for the device-resident step loop).
@@ -124,7 +118,7 @@ class _DynamicsFused(torch.autograd.Function):
         status = torch.zeros(W, dtype=torch.int32, device=dev)
         iters = torch.zeros(W, dtype=torch.int32, device=dev)
         C = cfg['nc_smem']
-        n, ws = _fused_plan(W, nb, neq, fd, C, dev)
+        n, ws = ops.dynamics_workspace(W, nb, neq, fd, C, C, False, dev)
         rc = _lib.call('dsdf_dynamics_solve', _lib.ptr(p), _lib.ptr(v), _lib.ptr(mass), _lib.ptr(Ibody),
                        _lib.ptr(fric), _lib.ptr(rest), _lib.ptr(f), _lib.ptr(dt), _lib.ptr(active), _lib.ptr(count),
                        _lib.ptr(cbody), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, neq, maxc, C, C, 0, fd,
@@ -142,26 +136,11 @@ class _DynamicsFused(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gv_new, _gstatus):
         (p, v, mass, Ibody, fric, rest, f, dt, geo, count, cbody, eq_rows, x, lam, s, active) = ctx.saved_tensors
-        active = active if active.numel() else None
-        cfg = ctx.cfg
-        W, nb = p.shape[0], p.shape[1]
-        maxc, fd = geo.shape[1], cfg['fric_dirs']
-        gnv = gv_new.contiguous()
-        gp, gv = torch.empty_like(p), torch.empty_like(v)
-        gmass, gI = torch.empty_like(mass), torch.empty_like(Ibody)
-        gfric, grest, gf = torch.empty_like(fric), torch.empty_like(rest), torch.empty_like(f)
-        gdt, ggeo = torch.empty(W, dtype=F64, device=p.device), torch.empty_like(geo)
-        neq, C = eq_rows.shape[0], cfg['nc_smem']
-        n, ws = _fused_plan(W, nb, neq, fd, C, p.device)
-        rc = _lib.call('dsdf_dynamics_solve_backward', _lib.ptr(p), _lib.ptr(v), _lib.ptr(mass), _lib.ptr(Ibody),
-                       _lib.ptr(fric), _lib.ptr(rest), _lib.ptr(f), _lib.ptr(dt), _lib.ptr(active), _lib.ptr(count),
-                       _lib.ptr(cbody), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, neq, maxc, C, C, 0, fd,
-                       int(cfg['stop_contact_grad']), int(cfg['stop_friction_grad']),
-                       _lib.ptr(x), _lib.ptr(lam), _lib.ptr(s), _lib.ptr(gnv), _lib.ptr(gp), _lib.ptr(gv),
-                       _lib.ptr(gmass), _lib.ptr(gI), _lib.ptr(gfric), _lib.ptr(grest), _lib.ptr(gf), _lib.ptr(gdt),
-                       _lib.ptr(ggeo), _lib.ptr(ws), _lib.stream(), kernels=n)
-        _lib.check(rc, 'dsdf_dynamics_solve_backward')
-        return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo, None, None, None, None, None
+        cfg, C = ctx.cfg, ctx.cfg['nc_smem']
+        grads = ops.dynamics_solve_backward(p, v, mass, Ibody, fric, rest, f, dt, active if active.numel() else None,
+                                            count, cbody, geo, eq_rows, C, C, False, cfg['fric_dirs'],
+                                            cfg['stop_contact_grad'], cfg['stop_friction_grad'], x, lam, s, gv_new)
+        return grads + (None,) * 5
 
 
 class Engine:

@@ -1,9 +1,11 @@
-"""torch.autograd wrappers over the C-ABI kernels (thin: pointer marshalling only, no arithmetic)."""
+"""Thin wrappers over the C-ABI kernels (pointer marshalling only, no arithmetic): torch.autograd functions, and the
+plain backward calls they share with the reverse sweep of the device step loop (stepper.py)."""
 import torch
 
 from . import _lib
 
 F64 = torch.float64
+BASE_TOL = 1e-6      # lcp_physics/physics/utils.py:43 -- the TOL read by World.H.backward (world.py:204)
 KIND = {'box': 0, 'sphere': 1, 'cylinder': 2, 'grid': 3, 'box_rounded': 4, 'brick': 5, 'bowl': 6}
 
 
@@ -81,22 +83,69 @@ class _Integrate(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
-        L = _lib.lib()
         p, v, dt, active = ctx.saved_tensors
-        active = active if active.numel() else None
-        W, nb = p.shape[0], p.shape[1]
-        gp, gv = torch.empty_like(p), torch.empty_like(v)
-        gdt = torch.empty(W, nb, dtype=F64, device=p.device)
-        g = _c(g)
-        rc = _lib.call('dsdf_integrate_backward', _lib.ptr(p), _lib.ptr(v), _lib.ptr(dt), _lib.ptr(active), W, nb,
-                                       _lib.ptr(g), _lib.ptr(gp), _lib.ptr(gv), _lib.ptr(gdt), _lib.stream())
-        _lib.check(rc, 'dsdf_integrate_backward')
-        return gp, gv, gdt.sum(1), None
+        return integrate_backward(p, v, dt, active if active.numel() else None, g) + (None,)
 
 
 def integrate(p, v, dt, active=None):
     """active: optional uint8 (W) mask; inactive worlds pass their pose through."""
     return _Integrate.apply(p, v, dt, active)
+
+
+def integrate_backward(p, v, dt, active, g):
+    """dsdf_integrate_backward: (gp, gv, gdt) for dL/d(integrate) = g; gdt (W) is summed over the bodies."""
+    W, nb = p.shape[0], p.shape[1]
+    gp, gv = torch.empty_like(p), torch.empty_like(v)
+    gdt = torch.empty(W, nb, dtype=F64, device=p.device)
+    g = _c(g)
+    rc = _lib.call('dsdf_integrate_backward', _lib.ptr(p), _lib.ptr(v), _lib.ptr(dt), _lib.ptr(active), W, nb,
+                   _lib.ptr(g), _lib.ptr(gp), _lib.ptr(gv), _lib.ptr(gdt), _lib.stream())
+    _lib.check(rc, 'dsdf_integrate_backward')
+    return gp, gv, gdt.sum(1)
+
+
+def toc_backward(dt, toc_mask, body, p, v, geo, f, mass, gh):
+    """dsdf_toc_backward: the backward of World.H and its gather (world.py:141-237, 275-327) for all worlds, given
+    dL/dh = gh.  Returns (g_dt, gp, gv, ggeo, gf, gmass); worlds without a new contact pass gh through to g_dt."""
+    W, nb, maxc = p.shape[0], p.shape[1], geo.shape[1]
+    # contiguous copies stay bound to locals until the launch has been enqueued
+    dt, toc_mask, body, p, v, geo, f, mass, gh = [_c(t) for t in (dt, toc_mask, body, p, v, geo, f, mass, gh)]
+    g_dt, gp, gv = torch.empty_like(dt), torch.empty_like(p), torch.empty_like(v)
+    ggeo, gf, gm = torch.empty_like(geo), torch.empty_like(f), torch.empty_like(mass)
+    rc = _lib.call('dsdf_toc_backward', W, nb, maxc, _lib.ptr(dt), _lib.ptr(toc_mask), _lib.ptr(body), _lib.ptr(p),
+                   _lib.ptr(v), _lib.ptr(geo), _lib.ptr(f), _lib.ptr(mass), _lib.ptr(gh), BASE_TOL, _lib.ptr(g_dt),
+                   _lib.ptr(gp), _lib.ptr(gv), _lib.ptr(ggeo), _lib.ptr(gf), _lib.ptr(gm), _lib.stream())
+    _lib.check(rc, 'dsdf_toc_backward')
+    return g_dt, gp, gv, ggeo, gf, gm
+
+
+def dynamics_workspace(W, nb, neq, fric_dirs, small, large, force_cta, device):
+    """(kernel launches, one-CTA workspace or None) of one dsdf_dynamics_solve / dsdf_dynamics_solve_backward call
+    with contact-count classes ``small`` and ``large``."""
+    n, nbytes = _lib.dynamics_plan(W, nb, neq, fric_dirs, small, large, force_cta)
+    return n, (torch.empty(nbytes // 8 + 1, dtype=F64, device=device) if nbytes else None)
+
+
+def dynamics_solve_backward(p, v, mass, Ibody, fric, rest, f, dt, active, count, body, geo, eq_rows, small, large,
+                            force_cta, fric_dirs, stop_contact_grad, stop_friction_grad, x, lam, s, gnv):
+    """dsdf_dynamics_solve_backward with the classes (``small``, ``large``, ``force_cta``) of the forward solve.
+    Returns (gp, gv, gmass, gIbody, gfric, grest, gf, gdt, ggeo)."""
+    W, nb = p.shape[0], p.shape[1]
+    neq, maxc = eq_rows.shape[0], geo.shape[1]
+    gnv = _c(gnv)
+    gp, gv = torch.empty_like(p), torch.empty_like(v)
+    gmass, gI = torch.empty_like(mass), torch.empty_like(Ibody)
+    gfric, grest, gf = torch.empty_like(fric), torch.empty_like(rest), torch.empty_like(f)
+    gdt, ggeo = torch.empty(W, dtype=F64, device=p.device), torch.empty_like(geo)
+    n, ws = dynamics_workspace(W, nb, neq, fric_dirs, small, large, force_cta, p.device)
+    rc = _lib.call('dsdf_dynamics_solve_backward', _lib.ptr(p), _lib.ptr(v), _lib.ptr(mass), _lib.ptr(Ibody),
+                   _lib.ptr(fric), _lib.ptr(rest), _lib.ptr(f), _lib.ptr(dt), _lib.ptr(active), _lib.ptr(count),
+                   _lib.ptr(body), _lib.ptr(geo), _lib.ptr(eq_rows), W, nb, neq, maxc, small, large, int(force_cta),
+                   fric_dirs, int(stop_contact_grad), int(stop_friction_grad), _lib.ptr(x), _lib.ptr(lam), _lib.ptr(s),
+                   _lib.ptr(gnv), _lib.ptr(gp), _lib.ptr(gv), _lib.ptr(gmass), _lib.ptr(gI), _lib.ptr(gfric),
+                   _lib.ptr(grest), _lib.ptr(gf), _lib.ptr(gdt), _lib.ptr(ggeo), _lib.ptr(ws), _lib.stream(), kernels=n)
+    _lib.check(rc, 'dsdf_dynamics_solve_backward')
+    return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo
 
 
 def filter_contacts(normals, p1, eps=1e-3, count=None):

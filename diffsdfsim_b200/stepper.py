@@ -16,13 +16,12 @@ import time
 
 import torch
 
-from . import _lib
+from . import _lib, ops
 from .contacts import ContactSet, geometry_vjp, scatter_vertex_grads
 
 F64 = torch.float64
 U8 = torch.uint8
 I32 = torch.int32
-BASE_TOL = 1e-6      # lcp_physics/physics/utils.py:43 (World.H.backward, world.py:204)
 
 MAX_SLOTS = 64
 STEP_CAPK, STEP_MAXC, STEP_DYN_SMEM, STEP_TAPE, STEP_MAX_ROUNDS = 1, 2, 4, 8, 16
@@ -225,8 +224,8 @@ class DeviceStepper:
         self.cs_v = ContactSet(V, self.maxc, dev)
         # workspace of the one-CTA dynamics kernel, if some world may run on it (csrc/dsdf_dynsolve.cu)
         self.force_cta = bool(self.FORCE_CTA)
-        _, n = _lib.dynamics_plan(V, nb, world.num_constraints, world.fric_dirs, self.maxc, self.maxc, self.force_cta)
-        self.dyn_ws = torch.empty(n // 8 + 1, dtype=F64, device=dev) if n else None
+        _, self.dyn_ws = ops.dynamics_workspace(V, nb, world.num_constraints, world.fric_dirs, self.maxc, self.maxc,
+                                                self.force_cta, dev)
 
     # ------------------------------------------------------------------------------------------------------------
     def _args(self, world, fixed_dt, st, tape, f):
@@ -340,10 +339,7 @@ class DeviceStepper:
                 self.active.zero_()
                 break
             if ab & STEP_MAX_ROUNDS:
-                stuck = self.active.nonzero().flatten().tolist()[:8]
-                raise RuntimeError('step did not complete in %d attempts: worlds %s keep penetrating (dt < %.3g); '
-                                   'use strict_no_penetration=False or a smaller dt'
-                                   % (world.max_rounds_per_step, stuck, float(self.dt_try.min())))
+                raise world._incomplete_step_error(self.active, self.dt_try)
             if ab:
                 self._grow(world, ab, tape, st, per, c)
                 args = self._args(world, fixed_dt, st, tape, f)
@@ -391,21 +387,13 @@ class DeviceStepper:
 
     def _grow(self, world, bits, tape, st, per, c):
         """Enlarge what the paused worlds ran out of (the worlds themselves are untouched and still active)."""
-        if bits & STEP_CAPK:
-            capK = world.detector.capK
-            if capK >= world.MAX_CAPK:
-                raise RuntimeError('contact candidate capacity exceeded at the kernel limit capK=%d (mesh too fine '
-                                   'for the one-CTA-per-world contact kernel)' % capK)
-            world._set_capacity(min(world.MAX_CAPK, 2 * capK), world.maxc)
-        if bits & STEP_MAXC:
-            maxc = world.maxc
-            if maxc >= world.MAX_MAXC:
-                raise RuntimeError('more than %d contacts in one world: beyond the dynamics kernel limit' % maxc)
-            new = min(world.MAX_MAXC, 2 * maxc)
-            world._set_capacity(world.detector.capK, new)
-            st['cur'] = st['cur'].resized(new)
-            tape.slots = [sl.regrown(sl.cap, new) for sl in tape.slots]
-            self._alloc_virtual(world)
+        if bits & (STEP_CAPK | STEP_MAXC):
+            capK, maxc = world._next_capacity(bits)          # STEP_CAPK / STEP_MAXC are its bits 0 / 1
+            world._set_capacity(capK, maxc)
+            if bits & STEP_MAXC:
+                st['cur'] = st['cur'].resized(maxc)
+                tape.slots = [sl.regrown(sl.cap, maxc) for sl in tape.slots]
+                self._alloc_virtual(world)
         if bits & STEP_TAPE:
             # a paused world found its slot missing or full: double the full slots (their row counters overshot by the
             # number of paused worlds: clamp them), and add slots up to the deepest sub-step index seen + 1
@@ -424,48 +412,6 @@ class DeviceStepper:
                                for k in range(len(tape.slots), n)]
         # STEP_DYN_SMEM needs no buffer: max_count was refreshed from the control block, so the next burst sizes the
         # dynamics launches for it (_smem_contacts)
-
-
-# ---------------------------------------------------------------------------------------------------- raw VJP calls
-def _integrate_bwd(p, v, dt, active, g):
-    W, nb = p.shape[0], p.shape[1]
-    gp, gv = torch.empty_like(p), torch.empty_like(v)
-    gdt = torch.empty(W, nb, dtype=F64, device=p.device)
-    rc = _lib.call('dsdf_integrate_backward', _ptr(p), _ptr(v), _ptr(dt), _ptr(active), W, nb, _ptr(g), _ptr(gp),
-                   _ptr(gv), _ptr(gdt), _lib.stream())
-    _lib.check(rc, 'dsdf_integrate_backward')
-    return gp, gv, gdt.sum(1)
-
-
-def _toc_bwd(dt, toc_mask, body, p, v, geo, f, mass, gh):
-    W, nb, maxc = p.shape[0], p.shape[1], geo.shape[1]
-    g_dt, gp, gv = torch.empty_like(dt), torch.empty_like(p), torch.empty_like(v)
-    ggeo, gf, gm = torch.empty_like(geo), torch.empty_like(f), torch.empty_like(mass)
-    rc = _lib.call('dsdf_toc_backward', W, nb, maxc, _ptr(dt), _ptr(toc_mask), _ptr(body), _ptr(p), _ptr(v), _ptr(geo),
-                   _ptr(f), _ptr(mass), _ptr(gh), BASE_TOL, _ptr(g_dt), _ptr(gp), _ptr(gv), _ptr(ggeo), _ptr(gf), _ptr(gm),
-                   _lib.stream())
-    _lib.check(rc, 'dsdf_toc_backward')
-    return g_dt, gp, gv, ggeo, gf, gm
-
-
-def _dyn_bwd(cfg, p, v, mass, Ibody, fric, rest, f, dt, active, count, body, geo, x, lam, s, gnv):
-    W, nb = p.shape[0], p.shape[1]
-    maxc = geo.shape[1]
-    gp, gv = torch.empty_like(p), torch.empty_like(v)
-    gmass, gI = torch.empty_like(mass), torch.empty_like(Ibody)
-    gfric, grest, gf = torch.empty_like(fric), torch.empty_like(rest), torch.empty_like(f)
-    gdt, ggeo = torch.empty(W, dtype=F64, device=p.device), torch.empty_like(geo)
-    small, large, force_cta = cfg['C']             # the contact-count classes of the forward
-    n, nbytes = _lib.dynamics_plan(W, nb, cfg['neq'], cfg['fric_dirs'], small, large, force_cta)
-    ws = torch.empty(nbytes // 8 + 1, dtype=F64, device=p.device) if nbytes else None
-    rc = _lib.call('dsdf_dynamics_solve_backward', _ptr(p), _ptr(v), _ptr(mass), _ptr(Ibody), _ptr(fric), _ptr(rest),
-                   _ptr(f), _ptr(dt), _ptr(active), _ptr(count), _ptr(body), _ptr(geo), _ptr(cfg['eq_rows']), W, nb,
-                   cfg['neq'], maxc, small, large, int(force_cta), cfg['fric_dirs'], int(cfg['stop_contact_grad']),
-                   int(cfg['stop_friction_grad']), _ptr(x), _ptr(lam), _ptr(s), _ptr(gnv), _ptr(gp), _ptr(gv),
-                   _ptr(gmass), _ptr(gI), _ptr(gfric), _ptr(grest), _ptr(gf), _ptr(gdt), _ptr(ggeo), _ptr(ws),
-                   _lib.stream(), kernels=n)
-    _lib.check(rc, 'dsdf_dynamics_solve_backward')
-    return gp, gv, gmass, gI, gfric, grest, gf, gdt, ggeo
 
 
 class _StepFn(torch.autograd.Function):
@@ -487,7 +433,7 @@ class _StepFn(torch.autograd.Function):
         ctx.tape = tape
         ctx.params = (mass, Ibody, fric, rest, f)
         ctx.geo_in_maxc = geo.shape[1]
-        ctx.cfg = dict(eq_rows=world.eq_rows, neq=world.num_constraints, C=tape.C, fric_dirs=world.fric_dirs,
+        ctx.cfg = dict(eq_rows=world.eq_rows, fric_dirs=world.fric_dirs,
                        stop_contact_grad=world.stop_contact_grad, stop_friction_grad=world.stop_friction_grad,
                        table=world.table, shape=world.shape, detach_b2=world.detach_contact_b2,
                        want_shape=shape_t is not None,
@@ -508,6 +454,7 @@ class _StepFn(torch.autograd.Function):
         mass, Ibody, fric, rest, f = ctx.params
         W = mass.shape[0]
         maxc = tape.maxc
+        small, large, force_cta = tape.C                   # the contact-count classes of the forward
         gp, gv, glast = gp.clone(), gv.clone(), glast.clone()
         if ggeo.shape[1] != maxc:
             ggeo = torch.cat([ggeo, ggeo.new_zeros(W, maxc - ggeo.shape[1], 10)], 1)
@@ -539,10 +486,10 @@ class _StepFn(torch.autograd.Function):
             if tape.any_toc:
                 # new contacts: p' = move(p, new_v, H(dt_)); H = dsdf_toc_backward (world.py:141-237, 275-341)
                 tn = S.toc_now.bool()
-                gpA, gvA, gdtA = _integrate_bwd(S.p_in, S.new_v, S.dt_used, S.toc_now, a_gp)
+                gpA, gvA, gdtA = ops.integrate_backward(S.p_in, S.new_v, S.dt_used, S.toc_now, a_gp)
                 gh = torch.where(tn, gdtA + a_glast, zero_n)
-                g_dt_B, gp_B, gv_B, ggeo_B, gf_B, gm_B = _toc_bwd(S.dt_used, S.toc_mask, S.body, S.p_try, S.new_v, S.geo,
-                                                                   pf, pm, gh)
+                g_dt_B, gp_B, gv_B, ggeo_B, gf_B, gm_B = ops.toc_backward(S.dt_used, S.toc_mask, S.body, S.p_try,
+                                                                          S.new_v, S.geo, pf, pm, gh)
                 tn3 = tn[:, None, None]
                 gp_in_acc = torch.where(tn3, gpA, torch.zeros_like(gpA))
                 gnv_acc = torch.where(tn3, gvA + gv_B, torch.zeros_like(gvA))
@@ -563,11 +510,12 @@ class _StepFn(torch.autograd.Function):
                 if leaves:
                     scatter_vertex_grads(gverts, leaves, cfg['table'], gctri_k, S.count, S.body, S.face, S.abc,
                                          None if k == 0 else idx)
-            gp2, gv2, gdt2 = _integrate_bwd(S.p_in, S.new_v, S.dt_used, None, gptry.contiguous())
+            gp2, gv2, gdt2 = ops.integrate_backward(S.p_in, S.new_v, S.dt_used, None, gptry)
             gnv = a_gv + gv2 if gnv_acc is None else a_gv + gv2 + gnv_acc
-            gp3, gv3, gm3, gI3, gfr3, gre3, gf3, gdt3, ggeo3 = _dyn_bwd(cfg, S.p_in, S.v_in, pm, pI, pfr, pre, pf,
-                                                                       S.dt_used, None, S.count_in, S.body_in, S.geo_in,
-                                                                       S.x, S.lam, S.s, gnv.contiguous())
+            gp3, gv3, gm3, gI3, gfr3, gre3, gf3, gdt3, ggeo3 = ops.dynamics_solve_backward(
+                S.p_in, S.v_in, pm, pI, pfr, pre, pf, S.dt_used, None, S.count_in, S.body_in, S.geo_in, cfg['eq_rows'],
+                small, large, force_cta, cfg['fric_dirs'], cfg['stop_contact_grad'], cfg['stop_friction_grad'], S.x,
+                S.lam, S.s, gnv)
             gp_new = gp2 + gp3 if gp_in_acc is None else gp2 + gp3 + gp_in_acc
             gdt_tot = gdt_acc + gdt2 + gdt3
             glast_new = glast_pass + torch.where(S.toc_flag_in.bool(), -gdt_tot, zero_n)

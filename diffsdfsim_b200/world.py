@@ -21,7 +21,6 @@ from .transforms import quaternion_to_matrix, so3_exponential_map
 from .utils import Defaults3D, default_device, get_instance
 
 F64 = torch.float64
-BASE_TOL = 1e-6      # lcp_physics/physics/utils.py:43 -- the TOL read by World.H.backward (world.py:204)
 
 
 class WorldState:
@@ -63,7 +62,7 @@ class TimeOfContact(torch.autograd.Function):
             D = TimeOfContact.gap(hk, *ins)
             grads = torch.autograd.grad((D * mask).sum(), [hk] + ins)
         dD_dh = grads[0] * mask
-        dD_dh = torch.where(dD_dh < BASE_TOL / h.detach()[:, None], torch.zeros_like(dD_dh), dD_dh)
+        dD_dh = torch.where(dD_dh < ops.BASE_TOL / h.detach()[:, None], torch.zeros_like(dD_dh), dD_dh)
         den = (dD_dh ** 2).sum(1, keepdim=True)
         inv = torch.where(den > 1e-5, dD_dh / torch.where(den > 1e-5, den, torch.ones_like(den)), torch.zeros_like(dD_dh))
         outs = [gh, None]
@@ -85,18 +84,7 @@ class TimeOfContactNative(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gh):
         dt_, p_try, new_v, geo, f, mass, toc_mask, cbody = ctx.saved_tensors
-        W, nb, maxc = p_try.shape[0], p_try.shape[1], geo.shape[1]
-        # contiguous copies stay bound to locals until the launch has been enqueued
-        dt_, toc_mask, cbody, p_try, new_v, geo, f, mass, gh = [t.contiguous() for t in
-                                                                (dt_, toc_mask, cbody, p_try, new_v, geo, f, mass, gh)]
-        g_dt, gp, gv = torch.empty_like(dt_), torch.empty_like(p_try), torch.empty_like(new_v)
-        ggeo, gf, gm = torch.empty_like(geo), torch.empty_like(f), torch.empty_like(mass)
-        rc = _lib.call('dsdf_toc_backward', W, nb, maxc, _lib.ptr(dt_), _lib.ptr(toc_mask), _lib.ptr(cbody),
-                       _lib.ptr(p_try), _lib.ptr(new_v), _lib.ptr(geo), _lib.ptr(f), _lib.ptr(mass),
-                       _lib.ptr(gh), BASE_TOL, _lib.ptr(g_dt), _lib.ptr(gp), _lib.ptr(gv), _lib.ptr(ggeo),
-                       _lib.ptr(gf), _lib.ptr(gm), _lib.stream())
-        _lib.check(rc, 'dsdf_toc_backward')
-        return g_dt, gp, gv, ggeo, gf, gm, None, None
+        return ops.toc_backward(dt_, toc_mask, cbody, p_try, new_v, geo, f, mass, gh) + (None, None)
 
 
 class World3D:
@@ -410,12 +398,7 @@ class World3D:
         while True:
             rounds += 1
             if rounds > self.max_rounds_per_step:
-                # strict_no_penetration=True halves dt for ever in the reference too (world.py:344-348); stop instead of
-                # accumulating an unbounded autograd graph
-                stuck = active.nonzero().flatten().tolist()[:8]
-                raise RuntimeError('step did not complete in %d attempts: worlds %s keep penetrating (dt < %.3g); '
-                                   'use strict_no_penetration=False or a smaller dt'
-                                   % (self.max_rounds_per_step, stuck, float(dt_try.min())))
+                raise self._incomplete_step_error(active, dt_try)
             self.stats['attempts'] += active
             accept, dt_try, active, n_active = self._attempt(active, dt_try, end_t)
             had |= accept.bool() & (self.contact_set.count > 0)
@@ -423,6 +406,14 @@ class World3D:
                 break
         self.stats['rounds'].append(rounds)
         return had
+
+    def _incomplete_step_error(self, active, dt_try):
+        """strict_no_penetration=True halves dt for ever in the reference too (world.py:344-348); both step loops stop
+        after ``max_rounds_per_step`` rounds instead of accumulating an unbounded autograd graph."""
+        stuck = active.nonzero().flatten().tolist()[:8]
+        return RuntimeError('step did not complete in %d attempts: worlds %s keep penetrating (dt < %.3g); '
+                            'use strict_no_penetration=False or a smaller dt'
+                            % (self.max_rounds_per_step, stuck, float(dt_try.min())))
 
     def undo_step(self, mask=None):
         """world.py:106-116.  ``mask`` (optional (W,) bool tensor, batched extension): undo the last step only for those
@@ -554,8 +545,9 @@ class World3D:
 
     MAX_CAPK, MAX_MAXC = 1024, 512     # candidate list: shared memory of the contact kernel; contacts: tape / workspace sizes
 
-    def _grow_capacity(self, bits):
-        """Double the candidate (capK) and / or contact (maxc) capacity after an overflow; raises when at the limit."""
+    def _next_capacity(self, bits):
+        """(capK, maxc) after an overflow: bit 0 doubles the candidate capacity (capK), bit 1 the contact capacity
+        (maxc).  Raises when one of them is already at its limit.  Both step loops grow through this rule."""
         capK, maxc = self.detector.capK, self.maxc
         if bits & 1:
             if capK >= self.MAX_CAPK:
@@ -566,6 +558,12 @@ class World3D:
             if maxc >= self.MAX_MAXC:
                 raise RuntimeError('more than %d contacts in one world: beyond the dynamics kernel limit' % maxc)
             maxc = min(self.MAX_MAXC, 2 * maxc)
+        return capK, maxc
+
+    def _grow_capacity(self, bits):
+        """Grow the capacity after an overflow (_next_capacity), with the world's contact set and geometry."""
+        capK, maxc = self._next_capacity(bits)
+        if maxc != self.maxc:
             self.contact_set = self.contact_set.resized(maxc)
             pad = self.contact_geo.new_zeros(self.W, maxc - self.maxc, 10)
             self.contact_geo = torch.cat([self.contact_geo, pad], 1)
