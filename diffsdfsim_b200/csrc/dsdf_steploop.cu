@@ -225,6 +225,7 @@ step_commit_kernel(const __grid_constant__ Args a) {
                 S.count_in[r] = a.count[w];
                 S.count[r] = a.count_v[vv]; a.count[w] = a.count_v[vv]; a.status[w] = st;
                 S.dt_raw[r] = dtr; S.dt_used[r] = dtu;
+                S.t_in[r] = a.t[w];                                                   // world.py:378 stamps the start
                 S.toc_flag_in[r] = a.toc_flag[w];
                 S.toc_now[r] = (unsigned char)any_toc;
                 if (a.toc_enabled && clean) a.toc_flag[w] = (unsigned char)any_toc;   // a give-up accept leaves the flag untouched

@@ -20,10 +20,21 @@ def _stack_times(traj, W, device):
     return torch.stack(ts, 0)                                   # (S, W)
 
 
-def nearest_time_index(t, t_target):
+def _stack_valid(traj):
+    """(S, W) bool of the rows that hold a recorded state (sub-step entries of a batch carry ``valid``), or None when no
+    entry carries it."""
+    if not any(hasattr(s, 'valid') for s in traj):
+        return None
+    return torch.stack([s.valid.reshape(-1) for s in traj], 0)
+
+
+def nearest_time_index(t, t_target, valid_target=None):
     """For every recorded state (S,W) the index (S,W) of the target state (S',W) closest in time; on a tie the LATER
-    target state wins (the reference's ``diff <= min_diff`` scan in ascending time order)."""
+    target state wins (the reference's ``diff <= min_diff`` scan in ascending time order).  Target rows outside
+    ``valid_target`` (S',W) are never matched."""
     diff = (t[:, None, :] - t_target[None, :, :]).abs()         # (S, S', W)
+    if valid_target is not None:
+        diff = torch.where(valid_target[None], diff, torch.full_like(diff, float('inf')))
     Sp = t_target.shape[0]
     rev = torch.flip(diff, dims=[1])
     return Sp - 1 - rev.argmin(dim=1)                           # argmin returns the first minimum of the reversed scan
@@ -33,15 +44,21 @@ def trajectory_loss(world, world_target):
     """Mean over the recorded states of |pos_last_body - pos_last_body_target(nearest time)|^2, per world.
 
     Returns a 0-d tensor for single worlds, (W,) for a batch; differentiable w.r.t. ``world``'s trajectory (the target
-    is used as recorded, like the reference)."""
+    is used as recorded, like the reference).  Sub-step entries of a batch (``World3D(record_substeps=True)``) carry a
+    ``valid`` mask: each world averages over its own valid entries and is matched only to its valid target entries."""
     W, dev = world.W, world.device
     t = _stack_times(world.trajectory, W, dev)
     tt = _stack_times(world_target.trajectory, W, dev)
     pos = torch.stack([s[1].reshape(W, -1)[:, -3:] for s in world.trajectory], 0)               # (S, W, 3)
     pos_t = torch.stack([s[1].reshape(W, -1)[:, -3:] for s in world_target.trajectory], 0)      # (S', W, 3)
-    idx = nearest_time_index(t, tt)                                                            # (S, W)
+    valid, valid_t = _stack_valid(world.trajectory), _stack_valid(world_target.trajectory)
+    idx = nearest_time_index(t, tt, valid_t)                                                   # (S, W)
     matched = torch.gather(pos_t, 0, idx[:, :, None].expand(-1, -1, 3))
-    loss = ((pos - matched) ** 2).sum(-1).sum(0) / len(world.trajectory)
+    err = ((pos - matched) ** 2).sum(-1)
+    if valid is None:
+        loss = err.sum(0) / len(world.trajectory)
+    else:
+        loss = torch.where(valid, err, torch.zeros_like(err)).sum(0) / valid.sum(0)
     return loss if world.batched else loss[0]
 
 

@@ -31,8 +31,8 @@ CT_SLOTROWS, CT_WORDS = 16, 16 + MAX_SLOTS
 CON_HULL3D, CON_STALLED = 4, 16
 LCP_FACTOR_FAIL, LCP_INACCURATE, LCP_TOO_LARGE = 4, 8, 16
 
-_SLOT_FIELDS = ['world', 'p_in', 'v_in', 'x', 'new_v', 'p_try', 'dt_raw', 'dt_used', 'lam', 's', 'toc_flag_in', 'toc_now',
-                'toc_mask', 'count_in', 'body_in', 'geo_in', 'count', 'body', 'face', 'abc', 'geo']
+_SLOT_FIELDS = ['world', 'p_in', 'v_in', 'x', 'new_v', 'p_try', 'dt_raw', 'dt_used', 't_in', 'lam', 's', 'toc_flag_in',
+                'toc_now', 'toc_mask', 'count_in', 'body_in', 'geo_in', 'count', 'body', 'face', 'abc', 'geo']
 _INT_FIELDS = ['W', 'nb', 'neq', 'maxc', 'fric_dirs', 'capK', 'npairs', 'depth', 'spec_threshold', 'depth2',
                'spec_threshold2', 'vcap', 'n_slots', 'slots_final',
                'max_iter', 'max_rounds', 'strict', 'toc_enabled', 'fixed_dt', 'detach_b2', 'force_cta']
@@ -63,7 +63,7 @@ def _ptr(t):
 class TapeSlot:
     """Device buffers of one dsdf_step_slot: ``cap`` self-contained rows (one accepted sub-step of one world each)."""
     F64_FIELDS = dict(p_in=('nb', 7), v_in=('nb', 6), p_try=('nb', 7), x=('nz',), new_v=('nb', 6), dt_raw=(), dt_used=(),
-                      lam=('ni',), s=('ni',), geo_in=('maxc', 10), abc=('maxc', 3), geo=('maxc', 10))
+                      t_in=(), lam=('ni',), s=('ni',), geo_in=('maxc', 10), abc=('maxc', 3), geo=('maxc', 10))
     I32_FIELDS = dict(world=(), count_in=(), body_in=('maxc', 2), count=(), body=('maxc', 2), face=('maxc',))
     U8_FIELDS = dict(toc_flag_in=(), toc_now=(), toc_mask=('maxc',))
 
@@ -155,7 +155,7 @@ def release_slot(sl):
 class Tape:
     """Everything one step leaves behind for its reverse sweep."""
     __slots__ = ('slots', 'maxsub', 'any_toc', 'maxc', 'C', 'rounds', 'p_out', 'v_out', 'geo_out',
-                 'last_dt_out', 'had', 'final', 'f', 'syncs')
+                 'last_dt_out', 'had', 'final', 'f', 'syncs', 'sub_t', 'sub_valid')
 
     def __del__(self):
         for sl in getattr(self, 'slots', None) or []:
@@ -414,6 +414,29 @@ class DeviceStepper:
         # dynamics launches for it (_smem_contacts)
 
 
+def _substep_states(tape, nsub, t_end):
+    """The state after each accepted sub-step of this step, in sub-step order, gathered from the tape: start times (K,W),
+    poses (K,W,nb,7), velocities (K,W,nb,6) and valid (K,W) = k < nsub.  A row that is not valid holds the world's
+    end-of-step state."""
+    K = tape.maxsub
+    valid = torch.arange(K, device=nsub.device)[:, None] < nsub[None, :]
+    T = t_end.expand(K, -1).clone()
+    P = tape.p_out.expand(K, -1, -1, -1).clone()
+    V = tape.v_out.expand(K, -1, -1, -1).clone()
+    for k, sl in enumerate(tape.slots):
+        if k == 0:          # row = world; a world that accepted no sub-step (stalled) left its row unwritten
+            ok = valid[0]
+            T[0] = torch.where(ok, sl.t_in, T[0])
+            P[0] = torch.where(ok[:, None, None], sl.p_try, P[0])
+            V[0] = torch.where(ok[:, None, None], sl.new_v, V[0])
+        elif sl.rows:
+            idx = sl.world[:sl.rows].long()
+            T[k].index_copy_(0, idx, sl.t_in[:sl.rows])
+            P[k].index_copy_(0, idx, sl.p_try[:sl.rows])
+            V[k].index_copy_(0, idx, sl.new_v[:sl.rows])
+    return T, P, V, valid
+
+
 class _StepFn(torch.autograd.Function):
     """One ``World3D.step`` of all worlds: (p, v, contact geometry, last_dt, parameters, forces) -> the same after the step.
 
@@ -424,6 +447,9 @@ class _StepFn(torch.autograd.Function):
         geo    = contact geometry(p_try)                                    contacts.py:262-264
         new contact:  dt_h = H(dt_, p_try, new_v, geo, f, mass);  p' = move(p, new_v, dt_h);  last_dt' = dt_h
         otherwise:    p' = p_try
+
+    With ``world.record_substeps`` two more outputs: (p', new_v) of every accepted sub-step, stacked (K,W,nb,7) and
+    (K,W,nb,6) in sub-step order (``_substep_states``); the start times and the valid mask are left on the tape.
     """
 
     @staticmethod
@@ -440,6 +466,9 @@ class _StepFn(torch.autograd.Function):
                        leaves=[(i, vt) for i, vt in zip(world.table.vert_leaf_ids, verts)])
         world._last_tape = tape
         outs = (tape.p_out, tape.v_out, tape.geo_out, tape.last_dt_out, tape.had)
+        if world.record_substeps:
+            tape.sub_t, P, V, tape.sub_valid = _substep_states(tape, world._stepper.nsub, world.t)
+            outs += (P, V)
         # the tape must not keep the outputs: output -> grad_fn (this ctx) -> tape -> output would be a reference cycle
         # that only the cyclic GC frees, holding every rollout's tape alive
         tape.p_out = tape.v_out = tape.geo_out = tape.last_dt_out = tape.had = None
@@ -447,9 +476,10 @@ class _StepFn(torch.autograd.Function):
         return outs
 
     @staticmethod
-    def backward(ctx, gp, gv, ggeo, glast, _ghad):
+    def backward(ctx, gp, gv, ggeo, glast, _ghad, *gsub):
         """Reverse sweep over the tape: slot k holds one row per world that accepted a (k+1)-th sub-step in this step, so
-        slot 0 is processed in place and the later (short) slots on gathered rows of the adjoints."""
+        slot 0 is processed in place and the later (short) slots on gathered rows of the adjoints.  The gradients on the
+        recorded sub-step states (``gsub``) join the adjoints of slot k before its chain runs."""
         tape, cfg = ctx.tape, ctx.cfg
         mass, Ibody, fric, rest, f = ctx.params
         W = mass.shape[0]
@@ -480,6 +510,14 @@ class _StepFn(torch.autograd.Function):
                 sel = lambda t: t.index_select(0, idx)
                 a_gp, a_gv, a_ggeo, a_glast = sel(gp), sel(gv), sel(ggeo), sel(glast)
                 pm, pI, pfr, pre, pf = sel(mass), sel(Ibody), sel(fric), sel(rest), sel(f)
+            if gsub:
+                gP, gV = gsub[0][k], gsub[1][k]
+                if k == 0:
+                    ok = tape.sub_valid[0][:, None, None]
+                    a_gp = a_gp + torch.where(ok, gP, torch.zeros_like(gP))
+                    a_gv = a_gv + torch.where(ok, gV, torch.zeros_like(gV))
+                else:
+                    a_gp, a_gv = a_gp + sel(gP), a_gv + sel(gV)
             zero_n = torch.zeros(n, dtype=F64, device=mass.device)
             gp_in_acc = gnv_acc = dgf = dgm = None
             gdt_acc, glast_pass, ggeo_tot, gptry = zero_n, a_glast, a_ggeo, a_gp

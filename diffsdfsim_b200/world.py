@@ -87,6 +87,17 @@ class TimeOfContactNative(torch.autograd.Function):
         return ops.toc_backward(dt_, toc_mask, cbody, p_try, new_v, geo, f, mass, gh) + (None, None)
 
 
+class SubstepEntry(tuple):
+    """A trajectory entry of a batch with ``record_substeps=True``: ``(t (W,), p (W,7nb), v (W,6nb), None, None)`` for the
+    k-th accepted sub-step of one step, and ``valid`` (W,) bool: the worlds that took a k-th sub-step.  A row that is not
+    valid holds the world's end-of-step state; it is finite and receives no gradient."""
+
+    def __new__(cls, items, valid):
+        e = super().__new__(cls, items)
+        e.valid = valid
+        return e
+
+
 class World3D:
     max_rounds_per_step = 256
     toc_native = True      # False: the torch-autograd restatement of World.H (TimeOfContact) on the affected worlds
@@ -98,7 +109,10 @@ class World3D:
                  fric_dirs=Defaults3D.FRIC_DIRS, post_stab=Defaults3D.POST_STABILIZATION,
                  strict_no_penetration=True, time_of_contact_diff=True, stop_contact_grad=False,
                  stop_friction_grad=False, detach_contact_b2=False, device=None, capK=384, maxc=32,
-                 record_prefilter=False):
+                 record_prefilter=False, record_substeps=False):
+        # True: ``trajectory`` gets one entry per accepted sub-step, like the reference (world.py:372-379); False: one per
+        # step() (see INTEGRATION.md)
+        self.record_substeps = bool(record_substeps)
         self.post_stab = bool(post_stab)          # world.py:358-370; runs on the host-driven loop + the dense LCP operator
         self.engine = get_instance(engines_module, engine)
         self.contact_callback = get_instance(contacts_module, contact_callback)
@@ -365,9 +379,21 @@ class World3D:
         self._sync_bodies()
         # one entry per step(), stamped like the reference's entries with the time the step STARTED (world.py:372-379
         # appends (self.t, ...) before self.t += dt; the reference appends once per accepted sub-step, we record the
-        # state at the end of the whole step -- see INTEGRATION.md)
-        self.trajectory.append((t_start, self.get_p(), self.v, self.contact_set, None))
+        # state at the end of the whole step unless record_substeps -- see INTEGRATION.md)
+        if not self.record_substeps:
+            self.trajectory.append((t_start, self.get_p(), self.v, self.contact_set, None))
         return had if self.batched else bool(had[0])
+
+    def _append_substeps(self, T, P, V, valid):
+        """Trajectory entries of the K accepted sub-steps of this step: start times T (K,W), poses P (K,W,nb,7) and
+        velocities V (K,W,nb,6) after each sub-step, valid (K,W)."""
+        W = self.W
+        if not self.batched:
+            for t, p, v in zip(T[:, 0].tolist(), P, V):                # one device-to-host copy for the K times
+                self.trajectory.append((t, p.reshape(-1), v.reshape(-1), None, None))
+            return
+        for k in range(T.shape[0]):
+            self.trajectory.append(SubstepEntry((T[k], P[k].reshape(W, -1), V[k].reshape(W, -1), None, None), valid[k]))
 
     def _step_device(self, fixed_dt):
         """world.py:119-139 with the whole sub-step state machine on the device: one autograd node, normally one host
@@ -375,10 +401,13 @@ class World3D:
         st = self.state
         if self._stepper is None:
             self._stepper = DeviceStepper(self)
-        p, v, geo, last_dt, had = _StepFn.apply(self, fixed_dt, st.p, st.v, self.contact_geo, self.last_dt, st.mass,
-                                                st.Ibody, st.fric, st.rest, self.step_forces(), self.shape_t,
-                                                *self.vert_leaves)
+        outs = _StepFn.apply(self, fixed_dt, st.p, st.v, self.contact_geo, self.last_dt, st.mass, st.Ibody, st.fric,
+                             st.rest, self.step_forces(), self.shape_t, *self.vert_leaves)
+        p, v, geo, last_dt, had = outs[:5]
         tape = self._last_tape
+        if self.record_substeps:
+            self._append_substeps(tape.sub_t, outs[5], outs[6], tape.sub_valid)
+            tape.sub_t = None
         st.p, st.v, self.contact_geo, self.last_dt = p, v, geo, last_dt
         self.contact_set = tape.final
         self.max_nc = max(int(self.max_nc), int(self._stepper.max_count))
@@ -395,17 +424,41 @@ class World3D:
         active = torch.ones(W, dtype=torch.uint8, device=dev)
         had = torch.zeros(W, dtype=torch.bool, device=dev)
         rounds = 0
+        rec = [] if self.record_substeps else None         # per round: (time before it, committed p, v, accept)
         while True:
             rounds += 1
             if rounds > self.max_rounds_per_step:
                 raise self._incomplete_step_error(active, dt_try)
             self.stats['attempts'] += active
+            t0 = self.t
             accept, dt_try, active, n_active = self._attempt(active, dt_try, end_t)
             had |= accept.bool() & (self.contact_set.count > 0)
+            if rec is not None:
+                rec.append((t0, self.state.p, self.state.v, accept.bool()))
             if not n_active:
                 break
         self.stats['rounds'].append(rounds)
+        if rec is not None:
+            self._append_substeps(*self._substeps_of_rounds(rec))
         return had
+
+    def _substeps_of_rounds(self, rec):
+        """The host loop's rounds in sub-step order: world w's k-th accepted round becomes its entry k; the rows a world
+        did not reach hold its end-of-step state, detached (the device loop gives these rows no gradient either)."""
+        st = self.state
+        acc = torch.stack([a for *_, a in rec])
+        nsub = acc.sum(0)
+        K = int(nsub.max())
+        T, P, V = [self.t] * K, [st.p.detach()] * K, [st.v.detach()] * K
+        n = torch.zeros_like(nsub)
+        for t0, p, v, a in rec:
+            for k in range(K):
+                m = a & (n == k)
+                m3 = m[:, None, None]
+                T[k], P[k], V[k] = torch.where(m, t0, T[k]), torch.where(m3, p, P[k]), torch.where(m3, v, V[k])
+            n = n + a
+        valid = torch.arange(K, device=nsub.device)[:, None] < nsub[None, :]
+        return torch.stack(T), torch.stack(P), torch.stack(V), valid
 
     def _incomplete_step_error(self, active, dt_try):
         """strict_no_penetration=True halves dt for ever in the reference too (world.py:344-348); both step loops stop
@@ -429,7 +482,8 @@ class World3D:
         if mask is None:
             st.p, st.v, self.contact_set, self.contact_geo = p0, v0, cs, geo
             self.t, self.t_host, self.toc_flag, self.last_dt, self._any_toc_flag = t0, t_host0, toc0, last0, any_toc0
-            del self.trajectory[ntraj:]
+            if not self.record_substeps:
+                del self.trajectory[ntraj:]
         else:
             m = mask.to(self.device).bool()
             m3 = m[:, None, None]
@@ -439,7 +493,24 @@ class World3D:
             self.t = torch.where(m, t0, self.t)
             self.toc_flag = torch.where(m, toc0, self.toc_flag)
             self.last_dt = torch.where(m, last0, self.last_dt)
+        if self.record_substeps:
+            self._drop_later_substeps(t0, ntraj, mask)
         self._sync_bodies()
+
+    def _drop_later_substeps(self, t0, ntraj, mask):
+        """The reference's undo_step rule on sub-step entries (oracle/sim.py:469-476): entries stamped later than the
+        restored time go; the first entry of the undone step carries that time and stays.  A batch applies it per world
+        by clearing ``valid`` of the undone worlds' rows."""
+        if not self.batched:
+            t = float(t0[0])
+            while self.trajectory and self.trajectory[-1][0] > t:
+                self.trajectory.pop()
+            return
+        m = torch.ones(self.W, dtype=torch.bool, device=self.device) if mask is None else mask.to(self.device).bool()
+        for e in self.trajectory[ntraj:]:
+            e.valid = e.valid & ~(m & (e[0] > t0))
+        if mask is None:
+            del self.trajectory[ntraj + 1:]           # every row of these is stamped after t0 or was not valid
 
     def detach_state(self, mask=None):
         """Cut the autograd history of the poses and velocities (of the masked worlds): what the reference drivers do with

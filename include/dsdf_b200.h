@@ -347,6 +347,7 @@ typedef struct dsdf_step_slot {      /* tape of the k-th accepted sub-step of th
     double *p_in, *v_in;             /* (cap,nb,7), (cap,nb,6) state the sub-step started from                           */
     double *x, *new_v, *p_try;       /* (cap,6nb) LCP solution, (cap,nb,6) = -x, (cap,nb,7) pose after the move          */
     double *dt_raw, *dt_used;        /* (cap) sub-step length; value that entered solve / move (world.py:253-257)        */
+    double* t_in;                    /* (cap) simulated time at the start of the sub-step (the reference's trajectory stamp) */
     double *lam, *s;                 /* (cap, maxc (2+fd)) multipliers / slacks, reference row order                     */
     unsigned char *toc_flag_in, *toc_now, *toc_mask;   /* (cap), (cap), (cap,maxc)                                        */
     int32_t *count_in, *body_in; double* geo_in;       /* contacts the solve used: (cap), (cap,maxc,2), (cap,maxc,10)     */
