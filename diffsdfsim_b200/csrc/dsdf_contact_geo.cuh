@@ -36,9 +36,10 @@ __device__ __forceinline__ BodyGeom world_geom(const BodyGeom& g, int w) {
 }
 
 // One out-of-line copy of the SDF evaluation for the whole contact kernel: inlining it at ~30 call sites made the
-// kernel 575 KB of SASS, far beyond the instruction cache (ncu: 18 % of stall samples "no_instructions").
+// kernel 575 KB of SASS, far beyond the instruction cache (ncu: 18 % of stall samples "no_instructions").  The shape is
+// passed by reference: the contact kernel keeps it in shared memory, so a call passes one pointer, not eight registers.
 #ifdef DSDF_OUTLINE_MATH
-__device__ __noinline__ SdfOut<double> sdf_q(SdfShape sh, V3<double> p, bool want_n) {
+__device__ __noinline__ SdfOut<double> sdf_q(const SdfShape& sh, V3<double> p, bool want_n) {
     return sdf_query<double>(sh, p, want_n);
 }
 #define DSDF_GEO_FN __device__ __noinline__
@@ -86,7 +87,7 @@ __device__ __forceinline__ V3<Dual> lift(V3<Dual> a, Dual) { return a; }
 __device__ __forceinline__ V3<double> strip(V3<double> a) { return a; }
 __device__ __forceinline__ V3<Dual> strip(V3<Dual> a) { return v3<Dual>(Dual(a.x.v), Dual(a.y.v), Dual(a.z.v)); }
 
-DSDF_GEO_FN double laplacian_fd(SdfShape s, V3<double> c, double d0, double h) {
+DSDF_GEO_FN double laplacian_fd(const SdfShape& s, V3<double> c, double d0, double h) {
     double acc = 0.0;
 #pragma unroll
     for (int ax = 0; ax < 3; ++ax) {

@@ -194,12 +194,43 @@ __device__ __forceinline__ float pre32_dist(const Pre32& P, float cx, float cy, 
     return d * P.scale;
 }
 
+// One search direction (mesh body 1 -> SDF body 2): what every phase of it reads.  Thread 0 writes it once per direction
+// into shared memory and every thread reads it there (broadcast loads): held in registers, these values stay live
+// across every phase and every out-of-line call, and they were most of the kernel's spill traffic.
+struct DirState {
+    BodyGeom g1;                   // body 1's geometry as this world sees it
+    SdfShape s1, s2;
+    Q4<double> q1, q2, q2i, rel;   // q2i = qinv(q2), rel = qmul(q2i, q1)
+    V3<double> x1, x2;
+    CellRange cr;                  // cells of g1 that can hold a candidate face (g1.has_cells)
+    Pre32 P32;                     // (g1.has_cells)
+};
+
+__device__ __forceinline__ void load_dir_state(DirState& D, const BodyGeom* geom, const double* p, const double* shape,
+                                               int w, int wg, int nb, int i1, int i2, double eps) {
+    D.g1 = world_geom(geom[i1], wg);
+    D.s1 = body_shape(D.g1, shape, wg, nb, i1);
+    D.s2 = body_shape(geom[i2], shape, wg, nb, i2);
+    load_pose(p, w, nb, i1, D.q1, D.x1);
+    load_pose(p, w, nb, i2, D.q2, D.x2);
+    D.q2i = qinv(D.q2);
+    D.rel = qmul(D.q2i, D.q1);
+    if (D.g1.has_cells) {
+        D.cr = cube_cells(D.g1, D.q1, D.x1, D.q2, D.x2, D.s2.scale);
+        D.P32 = make_pre32(D.g1, D.s2, D.q1, D.x1, D.q2, D.x2, eps);
+    }
+}
+
 // Centroid candidate pass of one search direction into the shared list ids[0..capK) (unsorted); returns the count
 // (which may exceed capK: overflow).  s_cnt: one shared int.
-__device__ int gather_candidates(const BodyGeom& g1, int w, const SdfShape& s2, Q4<double> q1, V3<double> x1,
-                                 Q4<double> q2, V3<double> x2, double eps, int capK, int* ids, int* s_cnt) {
+__device__ int gather_candidates(const DirState& D, int w, double eps, int capK, int* ids, int* s_cnt) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
-    const Q4<double> q2i = qinv(q2);
+    const BodyGeom& g1 = D.g1;
+    const SdfShape& s2 = D.s2;
+    const Q4<double>& q1 = D.q1;
+    const Q4<double>& q2i = D.q2i;
+    const V3<double>& x1 = D.x1;
+    const V3<double>& x2 = D.x2;
     if (tid == 0) *s_cnt = 0;
     __syncthreads();
     auto push = [&](bool is_cand, int f) {
@@ -220,8 +251,8 @@ __device__ int gather_candidates(const BodyGeom& g1, int w, const SdfShape& s2, 
             push(f < g1.nfaces && face_is_candidate(g1, w, f, s2, q1, x1, q2i, x2, eps), f);
         }
     } else {
-        const CellRange cr = cube_cells(g1, q1, x1, q2, x2, s2.scale);
-        const Pre32 P32 = make_pre32(g1, s2, q1, x1, q2, x2, eps);
+        const CellRange& cr = D.cr;
+        const Pre32& P32 = D.P32;
         if (!cr.empty) {
             const int nx = cr.hi[0] - cr.lo[0] + 1, ny = cr.hi[1] - cr.lo[1] + 1, nzc = cr.hi[2] - cr.lo[2] + 1;
             const int ncell = nx * ny * nzc;
@@ -586,18 +617,23 @@ __device__ bool hull3d_vertices(const double* PX, const double* PY, const double
 }
 
 // ------------------------------------------------------------------------------------------ refine kernel
+// Work arrays of one CTA in the dynamic shared memory.  Each array's address is derived from capK where it is used:
+// eleven pointers held across the whole kernel cost registers that the kernel does not have (they were spilled).
+extern __shared__ double smraw[];
 struct RefineSmem {
-    double* P;      // [9][capK] candidate triangle in b2 frame, later GEO rows 0..8
-    double* X;      // [3][capK] FW iterate, later GEO row 9 (pen) + scratch
-    double* ABC;    // [3][capK]
-    double* HK;     // [2][capK] hull sort keys -- aliases X rows 1,2 (free once the contact geometry is computed)
-    int* ID;        // [capK] face ids
-    int* SC;        // [capK] scan / flags
-    int* CL;        // [capK] cluster id
-    int* HI;        // [capK] hull payload
-    int* KEEP;      // [capK]
-    int* TMP;       // [capK] scratch flags
-    double* red;    // [40]
+    int capK;
+    __device__ double* P() const { return smraw; }                  // [9][capK] candidate triangle in b2 frame, later GEO rows 0..8
+    __device__ double* X() const { return smraw + 9 * capK; }       // [3][capK] FW iterate, later GEO row 9 (pen) + scratch
+    __device__ double* ABC() const { return smraw + 12 * capK; }    // [3][capK]
+    __device__ double* HK() const { return smraw + 10 * capK; }     // [2][capK] hull sort keys -- aliases X rows 1,2 (free once
+                                                                    // the contact geometry is computed)
+    __device__ double* red() const { return smraw + 15 * capK; }    // [40]
+    __device__ int* ID() const { return reinterpret_cast<int*>(smraw + 15 * capK + 40); }   // [capK] face ids
+    __device__ int* SC() const { return ID() + capK; }              // [capK] scan / flags
+    __device__ int* CL() const { return ID() + 2 * capK; }          // [capK] cluster id
+    __device__ int* HI() const { return ID() + 3 * capK; }          // [capK] hull payload
+    __device__ int* KEEP() const { return ID() + 4 * capK; }        // [capK]
+    __device__ int* TMP() const { return ID() + 5 * capK; }         // [capK] scratch flags
 };
 
 __host__ __device__ inline size_t refine_smem_bytes(int capK) {
@@ -608,139 +644,174 @@ struct DirResult { int count; int valid; };
 
 // One search direction (mesh body i1 -> SDF body i2) for world w.  On return the first `count` slots of
 // GEO (=P rows 0..8 + X row 0), ABC and ID hold the pre-filter contacts in ascending face order.
-// ids: the candidate list already sitting (unsorted) in sm.ID[0..min(ncand,capK)).
-__device__ DirResult search_direction(const RefineSmem& sm, int capK, const BodyGeom& g1, const SdfShape& s1,
-                                      const SdfShape& s2, Q4<double> q1, V3<double> x1, Q4<double> q2, V3<double> x2,
-                                      int w, int ncand, double eps, double tol, double fd_eps, bool detach_b2) {
-    const int tid = threadIdx.x, nt = blockDim.x;
+// ids: the candidate list already sitting (unsorted) in sm.ID()[0..min(ncand,capK)).
+__device__ DirResult search_direction(const RefineSmem& sm, const DirState& D, int w, int ncand, double eps, double tol,
+                                      double fd_eps, bool detach_b2) {
+    const int tid = threadIdx.x, nt = blockDim.x, capK = sm.capK;
+    const BodyGeom& g1 = D.g1;
+    const SdfShape& s1 = D.s1;
+    const SdfShape& s2 = D.s2;
     const int K = min(ncand, capK);
     DirResult r; r.count = 0; r.valid = 1;
     if (K == 0) return r;
     PH_MARK(-1);
     PH_ADD(PH_CAND, K);
-    rank_sort_int(sm.ID, sm.SC, K);
-    const Q4<double> q2i = qinv(q2);
+    rank_sort_int(sm.ID(), sm.SC(), K);
     // init: vertices in b2 frame, start at the vertex with the smallest SDF (contacts.py:57-61)
     for (int k = tid; k < K; k += nt) {
-        const int f = sm.ID[k];
+        const int f = sm.ID()[k];
         double best = 0.0; int bi = 0;
 #pragma unroll
         for (int v = 0; v < 3; ++v) {
-            const V3<double> t = to_b2(load_vert(g1, w, g1.faces[3 * f + v]), q1, x1, q2i, x2);
-            sm.P[(3 * v + 0) * capK + k] = t.x; sm.P[(3 * v + 1) * capK + k] = t.y; sm.P[(3 * v + 2) * capK + k] = t.z;
+            const V3<double> t = to_b2(load_vert(g1, w, g1.faces[3 * f + v]), D.q1, D.x1, D.q2i, D.x2);
+            sm.P()[(3 * v + 0) * capK + k] = t.x; sm.P()[(3 * v + 1) * capK + k] = t.y; sm.P()[(3 * v + 2) * capK + k] = t.z;
             const double d = sdf_q(s2, t, false).d;
             if (v == 0 || d < best) { best = d; bi = v; }
         }
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            sm.X[c * capK + k] = sm.P[(3 * bi + c) * capK + k];
-            sm.ABC[c * capK + k] = c == bi ? 1.0 : 0.0;
+            sm.X()[c * capK + k] = sm.P()[(3 * bi + c) * capK + k];
+            sm.ABC()[c * capK + k] = c == bi ? 1.0 : 0.0;
         }
+        sm.KEEP()[k] = bi;                             // (free until the push; a rerun of Frank-Wolfe restarts from it)
     }
     __syncthreads();
-    // Frank-Wolfe, <= 32 iterations, PAIR-GLOBAL exit (contacts.py:63-82).  A candidate whose step is zero
-    // (|gain| <= tol) keeps its x, so re-evaluating it would reproduce the same decision: it is skipped from then on
-    // (TMP[k] = 1) -- the reference recomputes it every iteration with identical results.
-    // The still-moving candidates are kept as a compact list (two ping-pong buffers in HI / CL, free until the filter),
-    // so that from the second iteration on every thread evaluates at most one of the few dozen survivors instead of
-    // walking all K slots: the iteration latency is one SDF evaluation, not ceil(K / threads) of them.
-    __shared__ int s_nact[2];
-    int* lists[2] = {sm.HI, sm.CL};
-    for (int k = tid; k < K; k += nt) lists[0][k] = k;
-    if (tid == 0) { s_nact[0] = K; s_nact[1] = 0; }
+    // Frank-Wolfe, <= 32 iterations, PAIR-GLOBAL exit (contacts.py:63-82): every iteration ends for all candidates at the
+    // first one in which any candidate penetrates (d < -tol), or when none moves any more.  A candidate whose step is zero
+    // (|gain| <= tol) keeps its x, so re-evaluating it would reproduce the same decision: it leaves for good (the reference
+    // recomputes it every iteration with identical results).  So apart from that exit the candidates are independent.
+    // Iteration 0 is a block-wide pass over all K candidates that lists the ones still moving (HI, free until the filter).
+    // From iteration 1 on each of these few dozen survivors runs on one thread, in registers and without a barrier, until
+    // it stops or penetrates; the earliest penetration E is the pair-global exit.  A survivor that ran past E is rerun from
+    // its start up to E -- only in attempts that penetrate, which the step loop rejects and halves.  gamma = 2 / (it + 2)
+    // keeps the global iteration index, so x, abc and the iteration count have the bits of the lock-step loop.
+    auto fw_eval = [&](int k, const V3<double>& x, double& d, int& pick) {     // -> SDF value and Frank-Wolfe vertex
+        const SdfOut<double> o = sdf_q(s2, x, true);
+        double dmin = 0.0;
+        pick = 0;
+#pragma unroll
+        for (int v = 0; v < 3; ++v) {
+            const double dp = sm.P()[(3 * v) * capK + k] * o.n.x + sm.P()[(3 * v + 1) * capK + k] * o.n.y +
+                              sm.P()[(3 * v + 2) * capK + k] * o.n.z;
+            if (v == 0 || dp < dmin) { dmin = dp; pick = v; }
+        }
+        const V3<double> sv = v3<double>(sm.P()[(3 * pick) * capK + k], sm.P()[(3 * pick + 1) * capK + k],
+                                         sm.P()[(3 * pick + 2) * capK + k]);
+        d = o.d;
+        return (x.x - sv.x) * o.n.x + (x.y - sv.y) * o.n.y + (x.z - sv.z) * o.n.z;        // gain
+    };
+    auto fw_step = [&](int k, V3<double>& x, V3<double>& abc, int pick, double gamma) {
+        x.x = (1.0 - gamma) * x.x + gamma * sm.P()[(3 * pick) * capK + k];
+        x.y = (1.0 - gamma) * x.y + gamma * sm.P()[(3 * pick + 1) * capK + k];
+        x.z = (1.0 - gamma) * x.z + gamma * sm.P()[(3 * pick + 2) * capK + k];
+        abc.x *= (1.0 - gamma); abc.y *= (1.0 - gamma); abc.z *= (1.0 - gamma);
+        if (pick == 0) abc.x += gamma; else if (pick == 1) abc.y += gamma; else abc.z += gamma;
+    };
+    // a survivor from the end of iteration 0 (X / ABC as iteration 0 left them) through iterations 1 .. it_end - 1;
+    // returns the iteration it stopped in (32: it never did), *pen: it stopped because it penetrates
+    auto fw_run = [&](int k, V3<double>& x, V3<double>& abc, int it_end, bool& pen) {
+        pen = false;
+        int it = 1;
+        for (; it < it_end; ++it) {
+            double d; int pick;
+            const double gain = fw_eval(k, x, d, pick);
+            if (d < -tol) { pen = true; break; }
+            if (!(fabs(gain) > tol)) break;
+            fw_step(k, x, abc, pick, 2.0 / (it + 2.0));
+        }
+        return it;
+    };
+    __shared__ int s_nsurv, s_pen_it, s_last_it;
+    if (tid == 0) { s_nsurv = 0; s_pen_it = 32; s_last_it = 0; }
     __syncthreads();
     PH_MARK(PH_SORT_INIT);
-    for (int it = 0; it < 32; ++it) {
-        const int cur = it & 1, nxt = cur ^ 1;
-        const int nact = s_nact[cur];
-        const int* act_list = lists[cur];
-        int any_pen = 0;
-        // phase 1: evaluate (no state change until the exit test is known)
-        for (int a = tid; a < nact; a += nt) {
-            const int k = act_list[a];
-            const V3<double> x = v3<double>(sm.X[k], sm.X[capK + k], sm.X[2 * capK + k]);
-            const SdfOut<double> o = sdf_q(s2, x, true);
-            double dmin = 0.0; int pick = 0;
-#pragma unroll
-            for (int v = 0; v < 3; ++v) {
-                const double dp = sm.P[(3 * v) * capK + k] * o.n.x + sm.P[(3 * v + 1) * capK + k] * o.n.y +
-                                  sm.P[(3 * v + 2) * capK + k] * o.n.z;
-                if (v == 0 || dp < dmin) { dmin = dp; pick = v; }
-            }
-            const V3<double> s = v3<double>(sm.P[(3 * pick) * capK + k], sm.P[(3 * pick + 1) * capK + k],
-                                            sm.P[(3 * pick + 2) * capK + k]);
-            const double gain = (x.x - s.x) * o.n.x + (x.y - s.y) * o.n.y + (x.z - s.z) * o.n.z;
-            const int act = fabs(gain) > tol;
-            any_pen |= (o.d < -tol);
-            sm.SC[k] = act ? pick : -1;
-            // a candidate whose step is zero keeps its x, so re-evaluating it would reproduce the same decision: it leaves
-            // the list for good (the reference recomputes it every iteration with identical results)
-            if (act) lists[nxt][atomicAdd(&s_nact[nxt], 1)] = k;
+    int any_pen = 0;
+    for (int k = tid; k < K; k += nt) {
+        const V3<double> x = v3<double>(sm.X()[k], sm.X()[capK + k], sm.X()[2 * capK + k]);
+        double d; int pick;
+        const double gain = fw_eval(k, x, d, pick);
+        any_pen |= (d < -tol);
+        if (fabs(gain) > tol) {
+            sm.SC()[k] = pick;
+            sm.HI()[atomicAdd(&s_nsurv, 1)] = k;
         }
-        // one barrier: the penetration flag through the barrier's predicate, "anything still moving" from the length of
-        // the next list (every active candidate was appended to it before the barrier)
-        const int blk_pen = __syncthreads_or(any_pen);
-        const int blk_active = s_nact[nxt] > 0;
-        PH_ADD(PH_FW_ITERS, 1);
-        if (!blk_active || blk_pen) break;
-        const double gamma = 2.0 / (it + 2.0);
-        for (int a = tid; a < nact; a += nt) {
-            const int k = act_list[a];
-            const int pick = sm.SC[k];
-            if (pick >= 0) {
-#pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    sm.X[c * capK + k] = (1.0 - gamma) * sm.X[c * capK + k] + gamma * sm.P[(3 * pick + c) * capK + k];
-                    sm.ABC[c * capK + k] *= (1.0 - gamma);
-                }
-                sm.ABC[pick * capK + k] += gamma;
-            }
-            // dropped candidates: gamma = 0 -> x, abc unchanged (x = 1*x + 0*s, abc *= 1, += 0)
-        }
-        if (tid == 0) s_nact[cur] = 0;                 // becomes the "next" counter of the following iteration
-        __syncthreads();
     }
+    const int blk_pen = __syncthreads_or(any_pen);
+    const int nsurv = s_nsurv;
+    int iters = 1;
+    if (nsurv > 0 && !blk_pen) {
+        for (int a = tid; a < nsurv; a += nt) {
+            const int k = sm.HI()[a];
+            V3<double> x = v3<double>(sm.X()[k], sm.X()[capK + k], sm.X()[2 * capK + k]);
+            V3<double> abc = v3<double>(sm.ABC()[k], sm.ABC()[capK + k], sm.ABC()[2 * capK + k]);
+            fw_step(k, x, abc, sm.SC()[k], 2.0 / (0 + 2.0));
+            bool pen;
+            const int stop = fw_run(k, x, abc, 32, pen);
+            if (pen) atomicMin(&s_pen_it, stop);
+            atomicMax(&s_last_it, stop);
+            sm.TMP()[a] = stop;
+            sm.X()[k] = x.x; sm.X()[capK + k] = x.y; sm.X()[2 * capK + k] = x.z;
+            sm.ABC()[k] = abc.x; sm.ABC()[capK + k] = abc.y; sm.ABC()[2 * capK + k] = abc.z;
+        }
+        __syncthreads();
+        const int E = s_pen_it;
+        iters = (E < 32 ? E : s_last_it) + 1;
+        if (E < 32) {
+            for (int a = tid; a < nsurv; a += nt) {
+                if (sm.TMP()[a] <= E) continue;
+                const int k = sm.HI()[a], bi = sm.KEEP()[k];
+                V3<double> x = v3<double>(sm.P()[(3 * bi) * capK + k], sm.P()[(3 * bi + 1) * capK + k],
+                                          sm.P()[(3 * bi + 2) * capK + k]);
+                V3<double> abc = v3<double>(bi == 0 ? 1.0 : 0.0, bi == 1 ? 1.0 : 0.0, bi == 2 ? 1.0 : 0.0);
+                fw_step(k, x, abc, sm.SC()[k], 2.0 / (0 + 2.0));
+                bool pen;
+                fw_run(k, x, abc, E, pen);
+                sm.X()[k] = x.x; sm.X()[capK + k] = x.y; sm.X()[2 * capK + k] = x.z;
+                sm.ABC()[k] = abc.x; sm.ABC()[capK + k] = abc.y; sm.ABC()[2 * capK + k] = abc.z;
+            }
+        }
+    }
+    PH_ADD(PH_FW_ITERS, min(iters, 32));
     __syncthreads();
     PH_MARK(PH_FW);
     // push onto b1's surface and final threshold (contacts.py:84-91)
-    const Q4<double> rel = qmul(q2i, q1);
     for (int k = tid; k < K; k += nt) {
-        const int f = sm.ID[k];
+        const int f = sm.ID()[k];
         const V3<double> va = load_vert(g1, w, g1.faces[3 * f]), vb = load_vert(g1, w, g1.faces[3 * f + 1]),
                          vc = load_vert(g1, w, g1.faces[3 * f + 2]);
-        const double a = sm.ABC[k], b = sm.ABC[capK + k], c = sm.ABC[2 * capK + k];
+        const double a = sm.ABC()[k], b = sm.ABC()[capK + k], c = sm.ABC()[2 * capK + k];
         const V3<double> xb1 = v3<double>(va.x * a + vb.x * b + vc.x * c, va.y * a + vb.y * b + vc.y * c,
                                           va.z * a + vb.z * b + vc.z * c);
         const SdfOut<double> o1 = sdf_q(s1, xb1, true);
-        const V3<double> dir = qapply(rel, o1.n);
-        const V3<double> x = v3<double>(sm.X[k] - o1.d * dir.x, sm.X[capK + k] - o1.d * dir.y,
-                                        sm.X[2 * capK + k] - o1.d * dir.z);
+        const V3<double> dir = qapply(D.rel, o1.n);
+        const V3<double> x = v3<double>(sm.X()[k] - o1.d * dir.x, sm.X()[capK + k] - o1.d * dir.y,
+                                        sm.X()[2 * capK + k] - o1.d * dir.z);
         const double d = sdf_q(s2, x, false).d;
-        sm.SC[k] = d <= eps ? 1 : 0;
+        sm.SC()[k] = d <= eps ? 1 : 0;
         // stash the body-frame triangle point for the geometry pass
-        sm.X[k] = xb1.x; sm.X[capK + k] = xb1.y; sm.X[2 * capK + k] = xb1.z;
+        sm.X()[k] = xb1.x; sm.X()[capK + k] = xb1.y; sm.X()[2 * capK + k] = xb1.z;
     }
     int total = 0;
-    for (int k = tid; k < K; k += nt) sm.KEEP[k] = sm.SC[k];
+    for (int k = tid; k < K; k += nt) sm.KEEP()[k] = sm.SC()[k];
     __syncthreads();
-    block_exclusive_scan(sm.SC, K, &total);
+    block_exclusive_scan(sm.SC(), K, &total);
     // order-preserving compaction into the front (read everything first, then write)
     {
         const int rounds = (K + nt - 1) / nt;
         for (int rd = 0; rd < rounds; ++rd) {
             const int k = rd * nt + tid;
             double t0 = 0, t1 = 0, t2 = 0, a0 = 0, a1 = 0, a2 = 0; int id = 0, dst = -1;
-            if (k < K && sm.KEEP[k]) {
-                dst = sm.SC[k];
-                t0 = sm.X[k]; t1 = sm.X[capK + k]; t2 = sm.X[2 * capK + k];
-                a0 = sm.ABC[k]; a1 = sm.ABC[capK + k]; a2 = sm.ABC[2 * capK + k];
-                id = sm.ID[k];
+            if (k < K && sm.KEEP()[k]) {
+                dst = sm.SC()[k];
+                t0 = sm.X()[k]; t1 = sm.X()[capK + k]; t2 = sm.X()[2 * capK + k];
+                a0 = sm.ABC()[k]; a1 = sm.ABC()[capK + k]; a2 = sm.ABC()[2 * capK + k];
+                id = sm.ID()[k];
             }
             __syncthreads();
             if (dst >= 0) {      // dst <= k and all smaller k already moved in earlier rounds / this round's reads done
-                sm.X[dst] = t0; sm.X[capK + dst] = t1; sm.X[2 * capK + dst] = t2;
-                sm.ABC[dst] = a0; sm.ABC[capK + dst] = a1; sm.ABC[2 * capK + dst] = a2;
-                sm.ID[dst] = id;
+                sm.X()[dst] = t0; sm.X()[capK + dst] = t1; sm.X()[2 * capK + dst] = t2;
+                sm.ABC()[dst] = a0; sm.ABC()[capK + dst] = a1; sm.ABC()[2 * capK + dst] = a2;
+                sm.ID()[dst] = id;
             }
             __syncthreads();
         }
@@ -749,12 +820,12 @@ __device__ DirResult search_direction(const RefineSmem& sm, int capK, const Body
     // contact geometry for every pre-filter contact (the reference's no_grad _compute_contacts).  Faces that share a
     // vertex often end at the very same body-frame point (bit-identical coordinates: the barycentrics are a unit
     // vector); the geometry is a pure function of that point, so it is evaluated once per DISTINCT point and copied.
-    int* REP = sm.TMP;                 // representative (smallest index with identical coordinates)
-    int* UL = sm.HI;                   // compact list of representatives
+    int* REP = sm.TMP();                 // representative (smallest index with identical coordinates)
+    int* UL = sm.HI();                   // compact list of representatives
     {
         // open-addressing hash set over the coordinates (capK slots in CL, free until the filter): a slot holds the smallest
         // index seen so far of its key.  Replaces an O(total^2) scan (9 % of the kernel's instructions, ncu round 2).
-        int* TAB = sm.CL;
+        int* TAB = sm.CL();
         for (int k = tid; k < capK; k += nt) TAB[k] = 0x7fffffff;
         __syncthreads();
         auto slot0 = [&](double a0, double a1, double a2) {
@@ -767,7 +838,7 @@ __device__ DirResult search_direction(const RefineSmem& sm, int capK, const Body
             return (int)((unsigned)h % (unsigned)capK);
         };
         for (int k = tid; k < total; k += nt) {
-            const double a0 = sm.X[k], a1 = sm.X[capK + k], a2 = sm.X[2 * capK + k];
+            const double a0 = sm.X()[k], a1 = sm.X()[capK + k], a2 = sm.X()[2 * capK + k];
             int s_ = slot0(a0, a1, a2);
             for (int probes = 0; probes < capK; ++probes, s_ = s_ + 1 == capK ? 0 : s_ + 1) {
                 int j = TAB[s_];
@@ -776,36 +847,36 @@ __device__ DirResult search_direction(const RefineSmem& sm, int capK, const Body
                     if (j == 0x7fffffff) break;                                        // new key
                 }
                 // j indexes a contact with this slot's key (atomicMin only ever swaps in an equal-key index)
-                if (sm.X[j] == a0 && sm.X[capK + j] == a1 && sm.X[2 * capK + j] == a2) { atomicMin(&TAB[s_], k); break; }
+                if (sm.X()[j] == a0 && sm.X()[capK + j] == a1 && sm.X()[2 * capK + j] == a2) { atomicMin(&TAB[s_], k); break; }
             }
         }
         __syncthreads();
         for (int k = tid; k < total; k += nt) {
-            const double a0 = sm.X[k], a1 = sm.X[capK + k], a2 = sm.X[2 * capK + k];
+            const double a0 = sm.X()[k], a1 = sm.X()[capK + k], a2 = sm.X()[2 * capK + k];
             int rep = k;
             int s_ = slot0(a0, a1, a2);
             for (int probes = 0; probes < capK; ++probes, s_ = s_ + 1 == capK ? 0 : s_ + 1) {
                 const int j = TAB[s_];
                 if (j == 0x7fffffff) break;                                            // (NaN coordinates: own representative)
-                if (sm.X[j] == a0 && sm.X[capK + j] == a1 && sm.X[2 * capK + j] == a2) { rep = j; break; }
+                if (sm.X()[j] == a0 && sm.X()[capK + j] == a1 && sm.X()[2 * capK + j] == a2) { rep = j; break; }
             }
             REP[k] = rep;
-            sm.SC[k] = rep == k;
+            sm.SC()[k] = rep == k;
         }
     }
     int nuniq = 0;
-    block_exclusive_scan(sm.SC, total, &nuniq);
-    for (int k = tid; k < total; k += nt) if (REP[k] == k) UL[sm.SC[k]] = k;
+    block_exclusive_scan(sm.SC(), total, &nuniq);
+    for (int k = tid; k < total; k += nt) if (REP[k] == k) UL[sm.SC()[k]] = k;
     __syncthreads();
     int bad = 0;
     for (int u = tid; u < nuniq; u += nt) {
         const int k = UL[u];
-        const V3<double> ct = v3<double>(sm.X[k], sm.X[capK + k], sm.X[2 * capK + k]);
-        const ContactGeo<double> g = contact_geometry<double>(s1, s2, q1, x1, q2, x2, ct, fd_eps, detach_b2);
-        sm.P[0 * capK + k] = g.n.x; sm.P[1 * capK + k] = g.n.y; sm.P[2 * capK + k] = g.n.z;
-        sm.P[3 * capK + k] = g.p1.x; sm.P[4 * capK + k] = g.p1.y; sm.P[5 * capK + k] = g.p1.z;
-        sm.P[6 * capK + k] = g.p2.x; sm.P[7 * capK + k] = g.p2.y; sm.P[8 * capK + k] = g.p2.z;
-        sm.X[capK + k] = g.pen;                            // park pen in X row 1 until every duplicate has read row 0
+        const V3<double> ct = v3<double>(sm.X()[k], sm.X()[capK + k], sm.X()[2 * capK + k]);
+        const ContactGeo<double> g = contact_geometry<double>(s1, s2, D.q1, D.x1, D.q2, D.x2, ct, fd_eps, detach_b2);
+        sm.P()[0 * capK + k] = g.n.x; sm.P()[1 * capK + k] = g.n.y; sm.P()[2 * capK + k] = g.n.z;
+        sm.P()[3 * capK + k] = g.p1.x; sm.P()[4 * capK + k] = g.p1.y; sm.P()[5 * capK + k] = g.p1.z;
+        sm.P()[6 * capK + k] = g.p2.x; sm.P()[7 * capK + k] = g.p2.y; sm.P()[8 * capK + k] = g.p2.z;
+        sm.X()[capK + k] = g.pen;                            // park pen in X row 1 until every duplicate has read row 0
         bad |= !(g.pen <= tol);
     }
     __syncthreads();
@@ -813,11 +884,11 @@ __device__ DirResult search_direction(const RefineSmem& sm, int capK, const Body
         const int rp = REP[k];
         if (rp != k) {
 #pragma unroll
-            for (int c = 0; c < 9; ++c) sm.P[(size_t)c * capK + k] = sm.P[(size_t)c * capK + rp];
+            for (int c = 0; c < 9; ++c) sm.P()[(size_t)c * capK + k] = sm.P()[(size_t)c * capK + rp];
         }
     }
     __syncthreads();
-    for (int k = tid; k < total; k += nt) sm.X[k] = sm.X[capK + REP[k]];      // X row 0 <- pen
+    for (int k = tid; k < total; k += nt) sm.X()[k] = sm.X()[capK + REP[k]];      // X row 0 <- pen
     __syncthreads();
     r.valid = !__syncthreads_or(bad);
     r.count = total;
@@ -836,22 +907,22 @@ __device__ __forceinline__ double distround(int dim, double maxabs) {
 __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps) {
     const int tid = threadIdx.x, nt = blockDim.x;
     int status = 0;
-    for (int k = tid; k < n; k += nt) sm.KEEP[k] = 1;
+    for (int k = tid; k < n; k += nt) sm.KEEP()[k] = 1;
     __syncthreads();
     if (n <= 1) return 0;
-    const double* NX = sm.P; const double* NY = sm.P + capK; const double* NZ = sm.P + 2 * capK;
-    const double* PX = sm.P + 3 * capK; const double* PY = sm.P + 4 * capK; const double* PZ = sm.P + 5 * capK;
+    const double* NX = sm.P(); const double* NY = sm.P() + capK; const double* NZ = sm.P() + 2 * capK;
+    const double* PX = sm.P() + 3 * capK; const double* PY = sm.P() + 4 * capK; const double* PZ = sm.P() + 5 * capK;
     // zero normals are dropped; CL = -1 unassigned, -2 dropped
     for (int k = tid; k < n; k += nt) {
         const double nn = fsqrt(NX[k] * NX[k] + NY[k] * NY[k] + NZ[k] * NZ[k]);
-        sm.CL[k] = nn > 1e-12 ? -1 : -2;
-        sm.KEEP[k] = 0;
+        sm.CL()[k] = nn > 1e-12 ? -1 : -2;
+        sm.KEEP()[k] = 0;
     }
     __syncthreads();
     for (int cl = 0; cl < n; ++cl) {
         // representative = first unassigned
         int first = 0x7fffffff;
-        for (int k = tid; k < n; k += nt) if (sm.CL[k] == -1) { first = k; break; }
+        for (int k = tid; k < n; k += nt) if (sm.CL()[k] == -1) { first = k; break; }
         __shared__ int s_first;
         if (tid == 0) s_first = 0x7fffffff;
         __syncthreads();
@@ -861,44 +932,44 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
         if (rep == 0x7fffffff) break;
         const double rx = NX[rep], ry = NY[rep], rz = NZ[rep];
         for (int k = tid; k < n; k += nt) {
-            if (sm.CL[k] == -1) {
+            if (sm.CL()[k] == -1) {
                 const double dp = NX[k] * rx + NY[k] * ry + NZ[k] * rz;
-                if (acos(fmin(dp, 1.0)) < 1e-2) sm.CL[k] = cl;
+                if (acos(fmin(dp, 1.0)) < 1e-2) sm.CL()[k] = cl;
             }
         }
         __syncthreads();
         // gather members (ascending) into HI[0..m)
-        for (int k = tid; k < n; k += nt) sm.SC[k] = sm.CL[k] == cl;
+        for (int k = tid; k < n; k += nt) sm.SC()[k] = sm.CL()[k] == cl;
         int m = 0;
-        block_exclusive_scan(sm.SC, n, &m);
-        for (int k = tid; k < n; k += nt) if (sm.CL[k] == cl) sm.HI[sm.SC[k]] = k;
+        block_exclusive_scan(sm.SC(), n, &m);
+        for (int k = tid; k < n; k += nt) if (sm.CL()[k] == cl) sm.HI()[sm.SC()[k]] = k;
         __syncthreads();
-        if (m == 1) { if (tid == 0) sm.KEEP[sm.HI[0]] = 1; __syncthreads(); continue; }
+        if (m == 1) { if (tid == 0) sm.KEEP()[sm.HI()[0]] = 1; __syncthreads(); continue; }
         PH_MARK(PH_F_CLUSTER);
         // statistics: mean/variance per axis, max |coord|
         double s0 = 0, s1 = 0, s2 = 0, mx = 0;
         for (int e = tid; e < m; e += nt) {
-            const int k = sm.HI[e];
+            const int k = sm.HI()[e];
             s0 += PX[k]; s1 += PY[k]; s2 += PZ[k];
             mx = fmax(mx, fmax(fabs(PX[k]), fmax(fabs(PY[k]), fabs(PZ[k]))));
         }
         {
             double rv[4] = {s0, s1, s2, mx};
             const int ro[4] = {RED_SUM, RED_SUM, RED_SUM, RED_MAX};
-            bred_multi(rv, ro, 4, sm.red);
+            bred_multi(rv, ro, 4, sm.red());
             s0 = rv[0]; s1 = rv[1]; s2 = rv[2]; mx = rv[3];
         }
         const double m0 = s0 / m, m1 = s1 / m, m2 = s2 / m;
         double v0 = 0, v1 = 0, v2 = 0;
         for (int e = tid; e < m; e += nt) {
-            const int k = sm.HI[e];
+            const int k = sm.HI()[e];
             v0 += (PX[k] - m0) * (PX[k] - m0); v1 += (PY[k] - m1) * (PY[k] - m1); v2 += (PZ[k] - m2) * (PZ[k] - m2);
         }
         double var[3];
         {
             double rv[3] = {v0, v1, v2};
             const int ro[3] = {RED_SUM, RED_SUM, RED_SUM};
-            bred_multi(rv, ro, 3, sm.red);
+            bred_multi(rv, ro, 3, sm.red());
             var[0] = rv[0] / (m - 1); var[1] = rv[1] / (m - 1); var[2] = rv[2] / (m - 1);
         }
         // axis order: amin = first argmin (dropped first), then of the remaining two the first argmin is dropped next
@@ -911,18 +982,18 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
         const double* PA[3] = {PX, PY, PZ};
         // extremes along the 1-D axis (first min / first max index, like argmin/argmax)
         double lo = INFINITY, hi = -INFINITY;
-        for (int e = tid; e < m; e += nt) { const double c = PA[keep1][sm.HI[e]]; lo = fmin(lo, c); hi = fmax(hi, c); }
+        for (int e = tid; e < m; e += nt) { const double c = PA[keep1][sm.HI()[e]]; lo = fmin(lo, c); hi = fmax(hi, c); }
         {
             double rv[2] = {lo, hi};
             const int ro[2] = {RED_MIN, RED_MAX};
-            bred_multi(rv, ro, 2, sm.red);
+            bred_multi(rv, ro, 2, sm.red());
             lo = rv[0]; hi = rv[1];
         }
         __shared__ int s_lo, s_hi;
         if (tid == 0) { s_lo = 0x7fffffff; s_hi = 0x7fffffff; }
         __syncthreads();
         for (int e = tid; e < m; e += nt) {
-            const double c = PA[keep1][sm.HI[e]];
+            const double c = PA[keep1][sm.HI()[e]];
             if (c == lo) atomicMin(&s_lo, e);
             if (c == hi) atomicMin(&s_hi, e);
         }
@@ -930,24 +1001,24 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
         const int e_lo = s_lo, e_hi = s_hi;
         // --- is the set flat (3-D Qhull raises) ?  thickness w.r.t. the plane through a, b, c
         bool flat3 = m < 4;
-        const int ka = sm.HI[e_lo], kb = sm.HI[e_hi];
+        const int ka = sm.HI()[e_lo], kb = sm.HI()[e_hi];
         const V3<double> A = v3<double>(PX[ka], PY[ka], PZ[ka]), B = v3<double>(PX[kb], PY[kb], PZ[kb]);
         const V3<double> AB = B - A;
         const double lab = norm3(AB);
         // farthest point from line AB
         double far = -1.0;
         for (int e = tid; e < m; e += nt) {
-            const int k = sm.HI[e];
+            const int k = sm.HI()[e];
             const V3<double> AP = v3<double>(PX[k], PY[k], PZ[k]) - A;
             const double dl = lab > 0 ? fdiv(norm3(cross(AB, AP)), lab) : norm3(AP);
             far = fmax(far, dl);
         }
-        far = bred_max(far, sm.red);
+        far = bred_max(far, sm.red());
         __shared__ int s_far;
         if (tid == 0) s_far = 0x7fffffff;
         __syncthreads();
         for (int e = tid; e < m; e += nt) {
-            const int k = sm.HI[e];
+            const int k = sm.HI()[e];
             const V3<double> AP = v3<double>(PX[k], PY[k], PZ[k]) - A;
             const double dl = lab > 0 ? fdiv(norm3(cross(AB, AP)), lab) : norm3(AP);
             if (dl == far) atomicMin(&s_far, e);
@@ -955,16 +1026,16 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
         __syncthreads();
         const bool collinear3 = !(far > 3.0 * distround(2, mx));
         if (!flat3 && !collinear3) {
-            const int kc = sm.HI[s_far];
+            const int kc = sm.HI()[s_far];
             const V3<double> C = v3<double>(PX[kc], PY[kc], PZ[kc]);
             V3<double> nrm = cross(AB, C - A);
             const double ln = norm3(nrm);
             double th = 0.0;
             for (int e = tid; e < m; e += nt) {
-                const int k = sm.HI[e];
+                const int k = sm.HI()[e];
                 th = fmax(th, fdiv(fabs(dot(nrm, v3<double>(PX[k], PY[k], PZ[k]) - A)), ln));
             }
-            th = bred_max(th, sm.red);
+            th = bred_max(th, sm.red());
             flat3 = !(th > 4.0 * distround(3, mx));
         } else {
             flat3 = true;
@@ -975,11 +1046,11 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
             // stack); a cluster too large for the buffers is kept whole and flagged
             bool done = false;
             if (m > 4) {
-                done = hull3d_vertices(PX, PY, PZ, sm.HI, m, sm.KEEP, reinterpret_cast<unsigned*>(sm.HK),
-                                       (size_t)4 * capK, sm.SC, sm.TMP, capK, sm.red, mx);
+                done = hull3d_vertices(PX, PY, PZ, sm.HI(), m, sm.KEEP(), reinterpret_cast<unsigned*>(sm.HK()),
+                                       (size_t)4 * capK, sm.SC(), sm.TMP(), capK, sm.red(), mx);
                 if (!done) status |= 4;
             }
-            if (!done) for (int e = tid; e < m; e += nt) sm.KEEP[sm.HI[e]] = 1;
+            if (!done) for (int e = tid; e < m; e += nt) sm.KEEP()[sm.HI()[e]] = 1;
             __syncthreads();
             continue;
         }
@@ -988,12 +1059,12 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
         bool line2 = m < 3;
         if (!line2) {
             // extremes along the larger-variance remaining axis define the reference line
-            const int ke_lo = sm.HI[e_lo], ke_hi = sm.HI[e_hi];
+            const int ke_lo = sm.HI()[e_lo], ke_hi = sm.HI()[e_hi];
             const double ax_ = PA[u_ax][ke_lo], ay_ = PA[v_ax][ke_lo], bx_ = PA[u_ax][ke_hi], by_ = PA[v_ax][ke_hi];
             const double l2 = fsqrt((bx_ - ax_) * (bx_ - ax_) + (by_ - ay_) * (by_ - ay_));
             double fd2 = 0.0, mx2 = 0.0;
             for (int e = tid; e < m; e += nt) {
-                const int k = sm.HI[e];
+                const int k = sm.HI()[e];
                 const double px = PA[u_ax][k], py = PA[v_ax][k];
                 const double cr = (bx_ - ax_) * (py - ay_) - (by_ - ay_) * (px - ax_);
                 fd2 = fmax(fd2, l2 > 0 ? fdiv(fabs(cr), l2) : fsqrt((px - ax_) * (px - ax_) + (py - ay_) * (py - ay_)));
@@ -1002,7 +1073,7 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
             {
                 double rv[2] = {fd2, mx2};
                 const int ro[2] = {RED_MAX, RED_MAX};
-                bred_multi(rv, ro, 2, sm.red);
+                bred_multi(rv, ro, 2, sm.red());
                 fd2 = rv[0]; mx2 = rv[1];
             }
             line2 = !(fd2 > 3.0 * distround(2, mx2));
@@ -1010,23 +1081,23 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
         if (line2) {
             // 1-D: min and max along the surviving axis, or a single point (contacts.py:143-150)
             if (tid == 0) {
-                sm.KEEP[sm.HI[e_lo]] = 1;
-                if (hi - lo > eps) sm.KEEP[sm.HI[e_hi]] = 1;
+                sm.KEEP()[sm.HI()[e_lo]] = 1;
+                if (hi - lo > eps) sm.KEEP()[sm.HI()[e_hi]] = 1;
             }
             __syncthreads();
             continue;
         }
         PH_MARK(PH_F_STATS);
         // --- planar convex hull (strict vertices only)
-        double* KU = sm.HK; double* KV = sm.HK + capK;
-        for (int e = tid; e < m; e += nt) { const int k = sm.HI[e]; KU[e] = PA[u_ax][k]; KV[e] = PA[v_ax][k]; }
+        double* KU = sm.HK(); double* KV = sm.HK() + capK;
+        for (int e = tid; e < m; e += nt) { const int k = sm.HI()[e]; KU[e] = PA[u_ax][k]; KV[e] = PA[v_ax][k]; }
         __syncthreads();
         // Akl-Toussaint pre-filter: the support points of 8 directions span a polygon inscribed in the hull; points
         // STRICTLY inside it (by a margin far above the hull tolerance) cannot be hull vertices.  Dropping them in
         // parallel leaves only the boundary band for the sequential chain below.
         {
-            __shared__ double s_ev[8][8];          // [warp][direction] best value
-            __shared__ int s_ei[8][8];
+            __shared__ double s_ev[4][8];          // [warp][direction] best value (blockDim.x <= 128, as bred_multi)
+            __shared__ int s_ei[4][8];
             __shared__ double s_px[8], s_py[8];
             const double dxs[8] = {1, 1, 0, -1, -1, -1, 0, 1}, dys[8] = {0, 1, 1, 1, 0, -1, -1, -1};
             double bv[8]; int bi[8];
@@ -1043,8 +1114,8 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
                 }
             }
             const int lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
-#pragma unroll 1
-            for (int q = 0; q < 8; ++q) {
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {          // (unrolled: bv / bi stay in registers)
 #pragma unroll 1
                 for (int o = 16; o > 0; o >>= 1) {
                     const double ov = __shfl_xor_sync(DSDF_FULL, bv[q], o);
@@ -1053,7 +1124,7 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
                 }
                 if (lane == 0) { s_ev[warp][q] = bv[q]; s_ei[warp][q] = bi[q]; }
             }
-            const double mxc_all = bred_max(mxl, sm.red);     // (contains the barriers)
+            const double mxc_all = bred_max(mxl, sm.red());     // (contains the barriers)
             if (tid < 8) {
                 double v = -INFINITY; int ix = 0x7fffffff;
                 for (int ww = 0; ww < nw; ++ww)
@@ -1072,45 +1143,45 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
                     const double len = fsqrt(ex * ex + ey * ey);
                     if (len > 0.0) inside = inside && ((ex * (y - ay_) - ey * (x - ax_)) > margin * len);
                 }
-                sm.SC[e] = inside ? 0 : 1;
+                sm.SC()[e] = inside ? 0 : 1;
             }
             __syncthreads();
-            for (int e = tid; e < m; e += nt) sm.TMP[e] = sm.SC[e];
+            for (int e = tid; e < m; e += nt) sm.TMP()[e] = sm.SC()[e];
             int msurv = 0;
-            block_exclusive_scan(sm.SC, m, &msurv);
+            block_exclusive_scan(sm.SC(), m, &msurv);
             // order-preserving compaction of (KU, KV, HI)
             const int rounds = (m + nt - 1) / nt;
             for (int rd = 0; rd < rounds; ++rd) {
                 const int e = rd * nt + tid;
                 double x = 0, y = 0; int hi_ = 0, dst = -1;
-                if (e < m && sm.TMP[e]) { dst = sm.SC[e]; x = KU[e]; y = KV[e]; hi_ = sm.HI[e]; }
+                if (e < m && sm.TMP()[e]) { dst = sm.SC()[e]; x = KU[e]; y = KV[e]; hi_ = sm.HI()[e]; }
                 __syncthreads();
-                if (dst >= 0) { KU[dst] = x; KV[dst] = y; sm.HI[dst] = hi_; }
+                if (dst >= 0) { KU[dst] = x; KV[dst] = y; sm.HI()[dst] = hi_; }
                 __syncthreads();
             }
             m = msurv;
             PH_MARK(PH_F_AKL);
-            rank_sort_kv(KU, KV, sm.HI, m);
+            rank_sort_kv(KU, KV, sm.HI(), m);
             // exact duplicates (faces sharing a vertex yield the same contact point): only the first of a run (lowest
             // contact index, the sort is stable in it) can be a hull vertex -- compact the others away in parallel so the
             // sequential chain below only walks distinct points
             for (int e = tid; e < m; e += nt) {
                 const int keep = (e == 0) || !(KU[e] == KU[e - 1] && KV[e] == KV[e - 1]);
-                sm.TMP[e] = keep; sm.SC[e] = keep;
+                sm.TMP()[e] = keep; sm.SC()[e] = keep;
             }
             int mu = 0;
-            block_exclusive_scan(sm.SC, m, &mu);
+            block_exclusive_scan(sm.SC(), m, &mu);
             for (int rd = 0; rd < (m + nt - 1) / nt; ++rd) {
                 const int e = rd * nt + tid;
                 double x = 0, y = 0; int hi_ = 0, dst = -1;
-                if (e < m && sm.TMP[e]) { dst = sm.SC[e]; x = KU[e]; y = KV[e]; hi_ = sm.HI[e]; }
+                if (e < m && sm.TMP()[e]) { dst = sm.SC()[e]; x = KU[e]; y = KV[e]; hi_ = sm.HI()[e]; }
                 __syncthreads();
-                if (dst >= 0) { KU[dst] = x; KV[dst] = y; sm.HI[dst] = hi_; }
+                if (dst >= 0) { KU[dst] = x; KV[dst] = y; sm.HI()[dst] = hi_; }
                 __syncthreads();
             }
             m = mu;
             PH_MARK(PH_F_SORT);
-            if (tid == 0) sm.red[39] = mxc_all;
+            if (tid == 0) sm.red()[39] = mxc_all;
             __syncthreads();
         }
         if (tid == 0 || tid == 32) {
@@ -1118,10 +1189,10 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
             // (thread 32, descending) are independent and run concurrently on two warps, each with its own stack.
             // b stays a vertex iff the turn a -> b -> e is left by more than the round-off bound: cr > tol |e - a|,
             // tested without the square root as cr > 0 and cr^2 > tol^2 |e - a|^2.
-            const double mxc = sm.red[39];
+            const double mxc = sm.red()[39];
             const double tol_d = 2.0 * distround(2, mxc), tol2 = tol_d * tol_d;
             const bool up = tid != 0;
-            int* H = up ? sm.TMP : sm.SC;   // stack of sorted positions
+            int* H = up ? sm.TMP() : sm.SC();   // stack of sorted positions
             int top = 0;
             for (int i = 0; i < m; ++i) {
                 const int e = up ? m - 1 - i : i;
@@ -1134,7 +1205,7 @@ __device__ int filter_contacts(const RefineSmem& sm, int capK, int n, double eps
                 }
                 H[top++] = e;
             }
-            for (int t = 0; t < top; ++t) sm.KEEP[sm.HI[H[t]]] = 1;
+            for (int t = 0; t < top; ++t) sm.KEEP()[sm.HI()[H[t]]] = 1;
         }
         __syncthreads();
         PH_MARK(PH_F_CHAIN);
@@ -1159,8 +1230,8 @@ contacts_kernel(const BodyGeom* __restrict__ geom, const int* __restrict__ pairs
                 int* __restrict__ count, int* __restrict__ cbody, int* __restrict__ cface, double* __restrict__ cabc,
                 double* __restrict__ cgeo, int* __restrict__ wstatus, int* __restrict__ pre_ids, int* __restrict__ pre_cnt,
                 const int* __restrict__ vmap, const int* __restrict__ ctrl) {
-    extern __shared__ double smraw[];
     __shared__ int s_cnt;
+    __shared__ DirState s_dir;
     // loop mode (ctrl != NULL, dsdf_steploop.cu): CTA w detects the contacts of virtual world w (poses p[w], outputs [w])
     // with the shapes / per-world meshes / per-world grids of the real world wg = vmap[w]
     const int w = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
@@ -1169,10 +1240,7 @@ contacts_kernel(const BodyGeom* __restrict__ geom, const int* __restrict__ pairs
     if (active && !active[w]) return;
     const int ndirs = 2 * npairs;
     RefineSmem sm;
-    sm.P = smraw; sm.X = sm.P + 9 * (size_t)capK; sm.ABC = sm.X + 3 * (size_t)capK; sm.HK = sm.X + (size_t)capK;
-    sm.red = sm.ABC + 3 * (size_t)capK;
-    sm.ID = reinterpret_cast<int*>(sm.red + 40);
-    sm.SC = sm.ID + capK; sm.CL = sm.SC + capK; sm.HI = sm.CL + capK; sm.KEEP = sm.HI + capK; sm.TMP = sm.KEEP + capK;
+    sm.capK = capK;
     int nout = 0, status = 0;
     for (int pair = 0; pair < npairs; ++pair) {
         const int bi = pairs[2 * pair], bj = pairs[2 * pair + 1];
@@ -1202,39 +1270,36 @@ contacts_kernel(const BodyGeom* __restrict__ geom, const int* __restrict__ pairs
         for (int rev = 0; rev < 2; ++rev) {
             const int d = 2 * pair + rev;
             const int i1 = rev ? bj : bi, i2 = rev ? bi : bj;
-            const BodyGeom g1 = world_geom(geom[i1], wg);
-            const SdfShape s1 = body_shape(g1, shape, wg, nb, i1);
-            const SdfShape s2 = body_shape(geom[i2], shape, wg, nb, i2);
-            const Q4<double> q1 = rev ? qj : qi, q2 = rev ? qi : qj;
-            const V3<double> x1 = rev ? xj : xi, x2 = rev ? xi : xj;
             PH_MARK(-1);
-            const int ncand = gather_candidates(g1, wg, s2, q1, x1, q2, x2, eps, capK, sm.ID, &s_cnt);
+            if (tid == 0) load_dir_state(s_dir, geom, p, shape, w, wg, nb, i1, i2, eps);   // (its last readers are
+            __syncthreads();                                                              //  behind a barrier)
+            const int ncand = gather_candidates(s_dir, wg, eps, capK, sm.ID(), &s_cnt);
             PH_MARK(PH_GATHER);
             if (ncand > capK) status |= 1;
-            DirResult r = search_direction(sm, capK, g1, s1, s2, q1, x1, q2, x2, wg, ncand, eps, tol, fd_eps, detach_b2 != 0);
+            DirResult r = search_direction(sm, s_dir, wg, ncand, eps, tol, fd_eps, detach_b2 != 0);
             if (pre_cnt) {
                 if (tid == 0) pre_cnt[(size_t)w * ndirs + d] = r.count;
-                for (int k = tid; k < r.count; k += nt) pre_ids[((size_t)w * ndirs + d) * capK + k] = sm.ID[k];
+                for (int k = tid; k < r.count; k += nt) pre_ids[((size_t)w * ndirs + d) * capK + k] = sm.ID()[k];
             }
             PH_MARK(-1);
             if (r.valid) status |= filter_contacts(sm, capK, r.count, eps);
-            else { status |= 8; for (int k = tid; k < r.count; k += nt) sm.KEEP[k] = 1; __syncthreads(); }
+            else { status |= 8; for (int k = tid; k < r.count; k += nt) sm.KEEP()[k] = 1; __syncthreads(); }
             PH_MARK(PH_FILTER);
             // append kept contacts in ascending face order
-            for (int k = tid; k < r.count; k += nt) sm.SC[k] = sm.KEEP[k];
+            for (int k = tid; k < r.count; k += nt) sm.SC()[k] = sm.KEEP()[k];
             int nk = 0;
-            block_exclusive_scan(sm.SC, r.count, &nk);
+            block_exclusive_scan(sm.SC(), r.count, &nk);
             for (int k = tid; k < r.count; k += nt) {
-                if (!sm.KEEP[k]) continue;
-                const int o = nout + sm.SC[k];
+                if (!sm.KEEP()[k]) continue;
+                const int o = nout + sm.SC()[k];
                 if (o >= maxc) continue;
                 const size_t oo = (size_t)w * maxc + o;
                 cbody[2 * oo] = i1; cbody[2 * oo + 1] = i2;
-                cface[oo] = sm.ID[k];
-                cabc[3 * oo] = sm.ABC[k]; cabc[3 * oo + 1] = sm.ABC[capK + k]; cabc[3 * oo + 2] = sm.ABC[2 * capK + k];
+                cface[oo] = sm.ID()[k];
+                cabc[3 * oo] = sm.ABC()[k]; cabc[3 * oo + 1] = sm.ABC()[capK + k]; cabc[3 * oo + 2] = sm.ABC()[2 * capK + k];
 #pragma unroll
-                for (int c = 0; c < 9; ++c) cgeo[10 * oo + c] = sm.P[(size_t)c * capK + k];
-                cgeo[10 * oo + 9] = sm.X[k];
+                for (int c = 0; c < 9; ++c) cgeo[10 * oo + c] = sm.P()[(size_t)c * capK + k];
+                cgeo[10 * oo + 9] = sm.X()[k];
             }
             if (nout + nk > maxc) status |= 2;
             nout = min(nout + nk, maxc);
@@ -1253,23 +1318,19 @@ contacts_kernel(const BodyGeom* __restrict__ geom, const int* __restrict__ pairs
 __global__ void __launch_bounds__(CONTACT_THREADS)
 filter_kernel(const double* __restrict__ normals, const double* __restrict__ p1, const int* __restrict__ n, int capK, double eps,
               int* __restrict__ keep, int* __restrict__ status) {
-    extern __shared__ double smraw[];
     const int w = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
     RefineSmem sm;
-    sm.P = smraw; sm.X = sm.P + 9 * (size_t)capK; sm.ABC = sm.X + 3 * (size_t)capK; sm.HK = sm.X + (size_t)capK;
-    sm.red = sm.ABC + 3 * (size_t)capK;
-    sm.ID = reinterpret_cast<int*>(sm.red + 40);
-    sm.SC = sm.ID + capK; sm.CL = sm.SC + capK; sm.HI = sm.CL + capK; sm.KEEP = sm.HI + capK; sm.TMP = sm.KEEP + capK;
+    sm.capK = capK;
     const int m = min(n[w], capK);
     for (int k = tid; k < m; k += nt) {
         const size_t o = ((size_t)w * capK + k) * 3;
 #pragma unroll
-        for (int c = 0; c < 3; ++c) { sm.P[(size_t)c * capK + k] = normals[o + c]; sm.P[(size_t)(3 + c) * capK + k] = p1[o + c]; }
+        for (int c = 0; c < 3; ++c) { sm.P()[(size_t)c * capK + k] = normals[o + c]; sm.P()[(size_t)(3 + c) * capK + k] = p1[o + c]; }
     }
     __syncthreads();
     const int st = filter_contacts(sm, capK, m, eps);
     __syncthreads();
-    for (int k = tid; k < m; k += nt) keep[(size_t)w * capK + k] = sm.KEEP[k];
+    for (int k = tid; k < m; k += nt) keep[(size_t)w * capK + k] = sm.KEEP()[k];
     if (tid == 0) status[w] = st | (n[w] > capK ? 1 : 0);
 }
 

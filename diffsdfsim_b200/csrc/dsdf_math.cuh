@@ -38,13 +38,20 @@ DSDF_MATH_FN double fsqrt(double a) { return a == 0.0 ? a : sqrt(a); }
 // q' = fma(fma(-q, b, a), r, q).  With r the correctly rounded reciprocal and q within one ulp of a/b this is the
 // correctly rounded quotient RN(a/b) (Markstein's theorem), i.e. the same bits as a / b; zero numerators stay exact
 // zeros and the non-finite / tiny-divisor cases take the plain divisions.
-DSDF_MATH_FN void fdiv3(double& x, double& y, double& z, double b) {
-    if (!(b > 1e-290 && b < 1e290)) { x = fdiv(x, b); y = fdiv(y, b); z = fdiv(z, b); return; }
+// (The out-of-line copy takes and returns the three values by value, in registers: through references they would make
+// a round trip through local memory at every call.)
+struct Dbl3 { double x, y, z; };
+DSDF_MATH_FN Dbl3 fdiv3_v(double x, double y, double z, double b) {
+    Dbl3 o;
+    if (!(b > 1e-290 && b < 1e290)) { o.x = fdiv(x, b); o.y = fdiv(y, b); o.z = fdiv(z, b); return o; }
     const double r = 1.0 / b;
-    if (x != 0.0) { const double q = x * r; x = fma(fma(-q, b, x), r, q); }
-    if (y != 0.0) { const double q = y * r; y = fma(fma(-q, b, y), r, q); }
-    if (z != 0.0) { const double q = z * r; z = fma(fma(-q, b, z), r, q); }
+    o.x = x; o.y = y; o.z = z;
+    if (x != 0.0) { const double q = x * r; o.x = fma(fma(-q, b, x), r, q); }
+    if (y != 0.0) { const double q = y * r; o.y = fma(fma(-q, b, y), r, q); }
+    if (z != 0.0) { const double q = z * r; o.z = fma(fma(-q, b, z), r, q); }
+    return o;
 }
+HD void fdiv3(double& x, double& y, double& z, double b) { const Dbl3 o = fdiv3_v(x, y, z, b); x = o.x; y = o.y; z = o.z; }
 HD Dual operator+(Dual a, Dual b) { return Dual(a.v + b.v, a.d + b.d); }
 HD Dual operator-(Dual a, Dual b) { return Dual(a.v - b.v, a.d - b.d); }
 HD Dual operator-(Dual a) { return Dual(-a.v, -a.d); }

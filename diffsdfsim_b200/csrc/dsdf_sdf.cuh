@@ -24,7 +24,7 @@ typedef SdfShapeT<double> SdfShape;
 // a shape parameter as a scalar of the evaluation type S
 template <class S> __device__ __forceinline__ S par(S proto, double c) { return cst(proto, c); }
 __device__ __forceinline__ Dual par(Dual, Dual c) { return c; }
-__device__ __forceinline__ SdfShape shape_values(const SdfShape& s) { return s; }
+__device__ __forceinline__ const SdfShape& shape_values(const SdfShape& s) { return s; }
 __device__ __forceinline__ SdfShape shape_values(const SdfShapeT<Dual>& s) {
     SdfShape r;
     r.kind = s.kind; r.a = s.a.v; r.b = s.b.v; r.c = s.c.v; r.scale = s.scale.v; r.grid = s.grid; r.res = s.res;
