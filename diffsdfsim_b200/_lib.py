@@ -28,6 +28,7 @@ SIGNATURES = {
     'dsdf_contacts_detect': (c_i, [c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_d, c_d, c_d, c_d, c_i, c_i, c_i]
                              + [c_p] * 11),
     'dsdf_contacts_phase_cycles': (c_i, [c_p, c_i]),
+    'dsdf_dynamics_phase_cycles': (c_i, [c_p, c_i]),
     'dsdf_filter_contacts': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_p, c_p, c_p]),
     'dsdf_contact_geometry_backward': (c_i, [c_p, c_p, c_p, c_i, c_i, c_d, c_i, c_i] + [c_p] * 10),
     'dsdf_dynamics_assemble': (c_i, [c_p] * 12 + [c_i] * 4 + [c_p] * 7),

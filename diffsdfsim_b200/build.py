@@ -21,8 +21,10 @@ FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std
 # body's normal to use on flat-flat contacts) that the reference takes with un-fused IEEE multiply/add (torch
 # element-wise ops): compile that file without FMA contraction so the same ties break the same way.
 _NOFMA = ['-fmad=false']
-EXTRA = {'dsdf_contacts_bwd.cu': _NOFMA, 'dsdf_contacts.cu': _NOFMA + (['-DDSDF_PHASE_PROFILE'] if os.environ.get('DSDF_PHASE_PROFILE') else [])
-         + (['-DDSDF_CONTACT_MINBLOCKS=' + os.environ['DSDF_CONTACT_MINBLOCKS']] if os.environ.get('DSDF_CONTACT_MINBLOCKS') else [])}
+_PHASES = ['-DDSDF_PHASE_PROFILE'] if os.environ.get('DSDF_PHASE_PROFILE') else []
+EXTRA = {'dsdf_contacts_bwd.cu': _NOFMA, 'dsdf_contacts.cu': _NOFMA + _PHASES
+         + (['-DDSDF_CONTACT_MINBLOCKS=' + os.environ['DSDF_CONTACT_MINBLOCKS']] if os.environ.get('DSDF_CONTACT_MINBLOCKS') else []),
+         'dsdf_dynsolve.cu': _PHASES}
 
 
 def _sources():

@@ -35,6 +35,27 @@ __device__ __forceinline__ double warp_max(double v) {
     return v;
 }
 
+// two minima and two maxima over the warp, the four butterflies interleaved (independent shuffles per level)
+__device__ __forceinline__ void warp_minmax2(double& mn0, double& mn1, double& mx0, double& mx1) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double a = __shfl_xor_sync(DSDF_FULL, mn0, o), b = __shfl_xor_sync(DSDF_FULL, mn1, o);
+        const double c = __shfl_xor_sync(DSDF_FULL, mx0, o), d = __shfl_xor_sync(DSDF_FULL, mx1, o);
+        mn0 = fmin(mn0, a); mn1 = fmin(mn1, b); mx0 = fmax(mx0, c); mx1 = fmax(mx1, d);
+    }
+}
+
+// a / b given r = 1 / b (correctly rounded): q = RN(a r) corrected by one exact-remainder step, fma(fma(-q, b, a), r, q),
+// is the correctly rounded quotient RN(a / b) (Markstein's theorem), i.e. the bits of a / b, as long as nothing over- or
+// underflows.  Operands outside [2^-500, 2^500] in magnitude (zeros, non-finite values included) take the plain
+// division, so the reciprocal of a divisor that repeats replaces the dependent divisions without changing a bit.
+__device__ __forceinline__ bool div_rcp_ok(double x) { const double ax = fabs(x); return ax > 0x1p-500 && ax < 0x1p500; }
+__device__ __forceinline__ double div_rcp(double a, double b, double r) {
+    if (!(div_rcp_ok(a) && div_rcp_ok(b))) return a / b;
+    const double q = __dmul_rn(a, r);
+    return fma(fma(-q, b, a), r, q);
+}
+
 // Deterministic block reductions; `red` is >= 33 doubles of shared memory. Result broadcast to all threads.
 enum { RED_SUM = 0, RED_MIN = 1, RED_MAX = 2 };
 template <int OP>
@@ -131,8 +152,9 @@ __device__ inline void warp_trsv_upper(const double* LU, int ld, int n, double* 
         const bool act = lane < w;
         double v = act ? x[r] : 0.0;
         const double dg = act ? LU[r * ld + r] : 1.0;
+        const double rdg = 1.0 / dg;           // every lane its own diagonal at once, off the dependent chain below
         for (int kk = w - 1; kk >= 0; --kk) {
-            if (lane == kk) v /= dg;
+            if (lane == kk) v = div_rcp(v, dg, rdg);
             double xk = __shfl_sync(DSDF_FULL, v, kk);
             if (act && lane < kk) v -= LU[r * ld + c0 + kk] * xk;
         }
@@ -165,10 +187,16 @@ __device__ inline int warp_lu(double* A, int ld, int n, int* perm) {
     for (int i = lane; i < n; i += 32) perm[i] = i;
     __syncwarp();
     for (int k = 0; k < n; ++k) {
+        // pivot search over the m = n - k remaining rows by the lowest g lanes, g = 8, 16 or 32 the smallest >= min(m, 32);
+        // lanes L and L + g, L + 2g, ... read the same rows, so every lane holds the result after log2(g) butterfly levels.
+        // The combine keeps the largest |a| and the lowest index on ties (NaN entries never win), an order-free
+        // selection: the same pivot as the full-warp search.
+        const int m = n - k, g = m <= 8 ? 8 : (m <= 16 ? 16 : 32);
         double best = -1.0; int bi = k;
-        for (int i = k + lane; i < n; i += 32) { double v = fabs(A[i * ld + k]); if (v > best) { best = v; bi = i; } }
+        for (int i = k + (lane & (g - 1)); i < n; i += g) { double v = fabs(A[i * ld + k]); if (v > best) { best = v; bi = i; } }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
+            if (o >= g) continue;                  // warp-uniform
             double ob = __shfl_xor_sync(DSDF_FULL, best, o); int oi = __shfl_xor_sync(DSDF_FULL, bi, o);
             if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
         }

@@ -48,7 +48,11 @@ struct WarpTeam {
     __device__ __forceinline__ static void sync() { __syncwarp(); }
     __device__ __forceinline__ static double sum(double v) { return warp_sum(v); }
     __device__ __forceinline__ static double min(double v) { return warp_min(v); }
-    __device__ __forceinline__ static double max(double v) { return warp_max(v); }
+    // two minima and two maxima at once: four independent butterflies, interleaved
+    __device__ __forceinline__ static void minmax(double& mn0, double& mn1, double& mx0, double& mx1) {
+        warp_minmax2(mn0, mn1, mx0, mx1);
+    }
+    __device__ __forceinline__ static bool any(bool p) { return __any_sync(DSDF_FULL, p); }
     __device__ __forceinline__ static int lu(double* A, int ld, int n, int* perm) { return warp_lu(A, ld, n, perm); }
     __device__ __forceinline__ static void lu_solve(const double* LU, int ld, int n, const int* perm, const double* b,
                                                     double* x) {
@@ -65,7 +69,23 @@ struct CtaTeam {
     __device__ __forceinline__ static double* red() { __shared__ double r[33]; return r; }
     __device__ __forceinline__ static double sum(double v) { return block_reduce<RED_SUM>(v, red()); }
     __device__ __forceinline__ static double min(double v) { return block_reduce<RED_MIN>(v, red()); }
-    __device__ __forceinline__ static double max(double v) { return block_reduce<RED_MAX>(v, red()); }
+    __device__ __forceinline__ static void minmax(double& mn0, double& mn1, double& mx0, double& mx1) {
+        __shared__ double r[4 * 8 + 4];                // 4 values per warp (256 threads), then the results
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
+        warp_minmax2(mn0, mn1, mx0, mx1);
+        __syncthreads();                               // protect r from the previous use
+        if (lane == 0) { r[4 * warp] = mn0; r[4 * warp + 1] = mn1; r[4 * warp + 2] = mx0; r[4 * warp + 3] = mx1; }
+        __syncthreads();
+        if (warp == 0) {
+            double a = INFINITY, b = INFINITY, c = -INFINITY, d = -INFINITY;
+            if (lane < nw) { a = r[4 * lane]; b = r[4 * lane + 1]; c = r[4 * lane + 2]; d = r[4 * lane + 3]; }
+            warp_minmax2(a, b, c, d);
+            if (lane == 0) { r[32] = a; r[33] = b; r[34] = c; r[35] = d; }
+        }
+        __syncthreads();
+        mn0 = r[32]; mn1 = r[33]; mx0 = r[34]; mx1 = r[35];
+    }
+    __device__ __forceinline__ static bool any(bool p) { return __syncthreads_or(p) != 0; }
     __device__ __forceinline__ static int lu(double* A, int ld, int n, int* perm) {
         __shared__ int piv[2];                         // pivot row, failure flag
         if (threadIdx.x == 0) piv[1] = 0;
@@ -79,8 +99,31 @@ struct CtaTeam {
         block_lu_solve(LU, ld, n, perm, b, x);
     }
 };
-// i = rank, rank + size, ... < n over the team of the enclosing template (`Team`)
-#define TFOR(i, n) for (int i = Team::rank(); i < (n); i += Team::size())
+// i = rank, rank + size, ... < n over the team of the enclosing template (`Team`).  Rolled: a lane owns at most a few
+// rows, so unrolling only adds instruction-cache misses (the one-warp forward is instruction-fetch bound otherwise).
+#define TFOR(i, n) _Pragma("unroll 1") for (int i = Team::rank(); i < (n); i += Team::size())
+
+// Optional per-phase cycle counters of the forward kernel (build with -DDSDF_PHASE_PROFILE; read back with
+// dsdf_dynamics_phase_cycles).  DP_ITERS counts the loop passes (the initial point included).
+enum { DP_LOAD = 0, DP_RESID, DP_FACTOR, DP_ASSEMBLY, DP_LU, DP_SOLVE0, DP_RATIO, DP_SOLVE1, DP_UPDATE, DP_BEST,
+       DP_ITERS, DP_COUNT };
+#ifdef DSDF_PHASE_PROFILE
+__device__ unsigned long long g_dyn_phase[DP_COUNT];
+template <class Team> __device__ __noinline__ void dp_mark(int k) {      // k < 0: (re)start the clock
+    __shared__ long long t0;
+    Team::sync();
+    if (Team::rank() == 0) {
+        const long long t = clock64();
+        if (k >= 0) atomicAdd(&g_dyn_phase[k], (unsigned long long)(t - t0));
+        t0 = t;
+    }
+}
+#define DP_MARK(k) dp_mark<Team>(k)
+#define DP_ADD(k, v) do { if (Team::rank() == 0) atomicAdd(&g_dyn_phase[k], (unsigned long long)(v)); } while (0)
+#else
+#define DP_MARK(k) do {} while (0)
+#define DP_ADD(k, v) do {} while (0)
+#endif
 
 // ---- per-world layout: a body region (shared memory) and a contact region (shared memory after the body region for
 // the warp; the global workspace for the CTA).  Offsets in doubles.
@@ -254,18 +297,27 @@ template <class Team> __device__ __forceinline__ void Gx_all(const DynCtx& c, co
     }
     Team::sync();
 }
-// (G' w)[I] through the contact list of I's body
-__device__ __forceinline__ double Gtw_row(const DynCtx& c, const double* w, int I) {
-    const int per = c.L.per, half = c.L.half, b = I / 6, k6 = I % 6;
-    double acc = 0.0;
-    for (int t = c.bstart[b]; t < c.bstart[b + 1]; ++t) {
-        const int cc = c.blist[t] >> 1, k = (c.blist[t] & 1) * 6 + k6;
+// G' w in two steps.  Gtw_terms: the term of every (contact, side, component), i.e. of column k = 6 side + k6 of the
+// contact's rows, by the whole team into YG (only live inside dyn_factor; 12 doubles per contact, contact-major, so the
+// term of list entry 2 cc + side, component k6, sits at 6 (2 cc + side) + k6).  Gtw_row: (G' w)[I], the terms of I's
+// body summed in ascending contact order.  The same expression per term and the same order of the sum as walking the
+// contact list term by term, so the same bits; but the terms no longer sit on the chain of one lane.
+template <class Team> __device__ __forceinline__ void Gtw_terms(const DynCtx& c, const double* w) {
+    const int per = c.L.per, half = c.L.half;
+    TFOR(e, c.nc * 12) {
+        const int cc = e / 12, k = e % 12;
         const double* Gc = c.G + (size_t)cc * c.L.gs + k;
         const double* wc = w + cc * per;
         double a2 = Gc[0] * wc[0];
         for (int q = 1; q <= half; ++q) a2 += Gc[12 * q] * (wc[q] - wc[q + half]);
-        acc += a2;
+        c.YG[e] = a2;
     }
+    Team::sync();
+}
+__device__ __forceinline__ double Gtw_row(const DynCtx& c, int I) {
+    const int b = I / 6, k6 = I % 6;
+    double acc = 0.0;
+    for (int t = c.bstart[b]; t < c.bstart[b + 1]; ++t) acc += c.YG[6 * c.blist[t] + k6];
     return acc;
 }
 // solve B_c u = t for every contact in place on t (contact-major), thread per contact
@@ -286,7 +338,8 @@ template <class Team> __device__ __forceinline__ void block_solve(const DynCtx& 
 }
 
 // factor: a = 1/d, den, YG, K = [[Q + sum G' B^-1 G, A'],[A,0]] -> LU.  Returns 1 on a singular K.
-template <class Team> __device__ __forceinline__ int dyn_factor(DynCtx& c, const double* d, int fd) {
+// prof: take the phase counters (the forward kernel's call).
+template <class Team> __device__ __forceinline__ int dyn_factor(DynCtx& c, const double* d, int fd, bool prof = false) {
     const DynLayout& L = c.L;
     const int per = L.per, nF = L.nF, ld = L.ldF, half = L.half;
     // a = 1/d is B's diagonal (batch.py:496); the kernel keeps 1/a and 1/den so the hot loops multiply
@@ -314,6 +367,7 @@ template <class Team> __device__ __forceinline__ int dyn_factor(DynCtx& c, const
         c.YG[e] = acc * c.den[cc];
     }
     Team::sync();
+    if (prof) DP_MARK(DP_FACTOR);
     // M~_FF = Q_FF + sum_c G_c' B_c^-1 G_c restricted to the free components; thread per entry.  Entry (If, jf) gathers
     // the contacts that touch BOTH bodies, walking the list of I's body.
     TFOR(e, nF * nF) {
@@ -337,7 +391,10 @@ template <class Team> __device__ __forceinline__ int dyn_factor(DynCtx& c, const
         c.K[If * ld + jf] = acc;
     }
     Team::sync();
-    return Team::lu(c.K, ld, nF, c.perm);
+    if (prof) DP_MARK(DP_ASSEMBLY);
+    const int fail = Team::lu(c.K, ld, nF, c.perm);
+    if (prof) DP_MARK(DP_LU);
+    return fail;
 }
 
 // dx of [[M~, A'], [A, 0]] [dx; dy] = rhs with A a 0/1 selection of the pinned components and rhs_y = 0 (b = 0, x_P = 0):
@@ -366,9 +423,10 @@ __device__ __forceinline__ void dyn_solve(DynCtx& c, const double* d, int fd, co
     TFOR(r, c.ni) { const double tv = (rz ? rz[r] : 0.0) - (rs ? rs[r] / d[r] : 0.0); t[r] = tv; dz[r] = tv; }
     Team::sync();
     block_solve<Team>(c, t, fd);                                    // t <- u = B^-1 t (dz keeps a copy of t)
+    Gtw_terms<Team>(c, t);
     TFOR(I, nq) {
         double acc = rxy ? -rxy[I] : 0.0;
-        if (I < nz) acc -= Gtw_row(c, t, I);
+        if (I < nz) acc -= Gtw_row(c, I);
         rhs[I] = acc;
     }
     Team::sync();
@@ -378,9 +436,10 @@ __device__ __forceinline__ void dyn_solve(DynCtx& c, const double* d, int fd, co
     TFOR(r, c.ni) dz[r] = gx[r] + dz[r];                            // G dx + t
     Team::sync();
     block_solve<Team>(c, dz, fd);
+    if (L.neq > 0) Gtw_terms<Team>(c, dz);
     TFOR(m, L.neq) {                                                // multipliers of the pinned rows
         const int b = c.eq[2 * m], k = c.eq[2 * m + 1], I = 6 * b + k;
-        double acc = (rxy ? -rxy[I] : 0.0) - Gtw_row(c, dz, I);
+        double acc = (rxy ? -rxy[I] : 0.0) - Gtw_row(c, I);
         for (int j = 0; j < 6; ++j) acc -= c.Qb[36 * b + 6 * k + j] * dxy[6 * b + j];
         dxy[nz + m] = acc;
     }
@@ -388,14 +447,30 @@ __device__ __forceinline__ void dyn_solve(DynCtx& c, const double* d, int fd, co
     Team::sync();
 }
 
-template <class Team> __device__ __forceinline__ double dyn_ratio_step(const DynCtx& c, const double* v, const double* dv) {
-    double mx = -INFINITY;
-    TFOR(r, c.ni) mx = fmax(mx, -v[r] / dv[r]);
-    mx = Team::max(mx);
-    const double repl = fmax(1.0, mx);
-    double mn = INFINITY;
-    TFOR(r, c.ni) mn = fmin(mn, dv[r] > 0.0 ? repl : -v[r] / dv[r]);
-    return Team::min(mn);
+// Step length of one call site, min(ratio(z, dz), ratio(s, ds)) (batch.py get_step), with
+//     ratio(v, dv) = min_r (dv[r] > 0 ? repl : -v[r] / dv[r]),   repl = max(1, max_r -v[r] / dv[r]).
+// One pass and one division per row and vector: each lane keeps the maximum of q = -v/dv over its rows, the minimum of q
+// over its rows with !(dv > 0) (dv <= 0 or NaN: the rows that take q) and whether any row has dv > 0; then the four
+// reductions run as interleaved butterflies.  ratio = any ? min(min_q, repl) : min_q.  This is the two-pass result
+// bit for bit: fmin / fmax return one of their operands exactly and ignore a NaN operand in either position, so the
+// minimum of a set does not depend on the order or grouping in which it is taken, and repl (>= 1) only joins the set when
+// some row has dv > 0.  (Equal values have equal bits except +-0, and repl never ties a zero: the zeros meet each other
+// in the same order in both forms.)  Rows with dv == 0 give q = -v/0 (an infinity, or NaN for v == 0) in both forms and take the q
+// branch in both.  The maxima are the same operations in the same order as before.
+template <class Team> __device__ __forceinline__ double dyn_ratio_step(const DynCtx& c, const double* z, const double* dz,
+                                                                       const double* s, const double* ds) {
+    double mxz = -INFINITY, mxs = -INFINITY, mnz = INFINITY, mns = INFINITY;
+    bool pz = false, ps = false;
+    TFOR(r, c.ni) {
+        const double qz = -z[r] / dz[r], qs = -s[r] / ds[r];
+        mxz = fmax(mxz, qz); mxs = fmax(mxs, qs);
+        if (dz[r] > 0.0) pz = true; else mnz = fmin(mnz, qz);
+        if (ds[r] > 0.0) ps = true; else mns = fmin(mns, qs);
+    }
+    Team::minmax(mnz, mns, mxz, mxs);
+    pz = Team::any(pz); ps = Team::any(ps);
+    const double rz = pz ? fmin(mnz, fmax(1.0, mxz)) : mnz, rs = ps ? fmin(mns, fmax(1.0, mxs)) : mns;
+    return fmin(rz, rs);
 }
 
 // work: the global workspace of the CTA kernel (contact regions, one per world); unused by the warp kernel
@@ -434,6 +509,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
         }
         return;
     }
+    DP_MARK(-1);
     DynCtx c = dyn_ctx(smd, Team::kContactsInSmem ? smd + L.body : work + (size_t)w * L.contact, L);
     dyn_load<Team>(c, ws, p, v, mass, Ibody, fric, rest, f, dt[w], count, cbody, cgeo, eq_rows, maxc, fd);
     auto hrow = [&](int r) { return (r % per == 0) ? c.h[r / per] : 0.0; };
@@ -452,7 +528,9 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
     bool have_best = false;
     double best_res = INFINITY, mu_gap = 0.0, sz = 0.0;
     int stalled = 0;
+    DP_MARK(DP_LOAD);
     for (int it = -1; it < max_iter; ++it) {
+        DP_ADD(DP_ITERS, 1);
         double res = 0.0;
         if (it < 0) {
             TFOR(r, ni) { d[r] = 1.0; rz[r] = -hrow(r); }
@@ -461,6 +539,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
             // residuals (batch.py:117-131)
             double nrx = 0.0, nry = 0.0, nrz = 0.0;
             sz = 0.0;
+            Gtw_terms<Team>(c, z);
             TFOR(I, nq) {
                 double acc;
                 if (I < nz) {
@@ -469,7 +548,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
                     const double ay = fp < 0 ? xy[nz + (-fp - 1)] : 0.0;
                     double qx = 0.0;
                     for (int j = 0; j < 6; ++j) qx += xy[6 * b + j] * c.Qb[36 * b + 6 * k + j];
-                    acc = ay + Gtw_row(c, z, I) + qx + pv[I];
+                    acc = ay + Gtw_row(c, I) + qx + pv[I];
                     nrx += acc * acc;
                 } else {
                     const int m = I - nz;
@@ -491,7 +570,8 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
             TFOR(r, ni) d[r] = z[r] / s[r];
         }
         Team::sync();
-        if (dyn_factor<Team>(c, d, fd)) { status |= DSDF_LCP_FACTOR_FAIL; if (it >= 0) break; }
+        DP_MARK(DP_RESID);
+        if (dyn_factor<Team>(c, d, fd, true)) { status |= DSDF_LCP_FACTOR_FAIL; if (it >= 0) break; }
         if (it >= 0) {
             iters = it + 1;
             if (!have_best || res < best_res) {
@@ -507,6 +587,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
             }
             if (stalled == not_improved_lim || best_res < eps || mu_gap > 1e32) break;
         }
+        DP_MARK(DP_BEST);
         bool init_done = false;
         for (int pass = 0; pass < 2; ++pass) {
             // pass 0: initial solve (it < 0) or affine direction (rs = z); pass 1: corrector (rs in rz)
@@ -517,6 +598,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
             double* o_s = pass == 0 ? (it < 0 ? s : dsa) : ds;
             double* o_z = pass == 0 ? (it < 0 ? z : dza) : dz;
             dyn_solve<Team>(c, d, fd, a_rxy, a_rs, a_rz, o_xy, o_s, o_z);
+            DP_MARK(pass == 0 ? DP_SOLVE0 : DP_SOLVE1);
             if (it < 0) {
                 if (ni > 0) {                                   // batch.py:100-110
                     double ms = INFINITY, mz = INFINITY;
@@ -528,11 +610,12 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
                     }
                     Team::sync();
                 }
+                DP_MARK(DP_RATIO);
                 init_done = true;
                 break;
             }
             if (pass == 0) {
-                double alpha = fmin(fmin(dyn_ratio_step<Team>(c, z, dza), dyn_ratio_step<Team>(c, s, dsa)), 1.0);
+                double alpha = fmin(dyn_ratio_step<Team>(c, z, dza, s, dsa), 1.0);
                 double t3 = 0.0;
                 TFOR(r, ni) t3 += (s[r] + alpha * dsa[r]) * (z[r] + alpha * dza[r]);
                 t3 = Team::sum(t3);
@@ -540,6 +623,7 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
                 // corrector: rs = (-mu sig + dsa dza) / s  (stored in rz, which is free now)
                 TFOR(r, ni) rz[r] = (-mu_gap * sig + dsa[r] * dza[r]) / s[r];
                 Team::sync();
+                DP_MARK(DP_RATIO);
             }
         }
         if (init_done) {
@@ -553,10 +637,11 @@ dyn_forward_kernel(const double* __restrict__ p, const double* __restrict__ v, c
         TFOR(i, nq) dxy[i] += dxya[i];
         TFOR(r, ni) { ds[r] += dsa[r]; dz[r] += dza[r]; }
         Team::sync();
-        const double alpha = fmin(0.999 * fmin(dyn_ratio_step<Team>(c, z, dz), dyn_ratio_step<Team>(c, s, ds)), 1.0);
+        const double alpha = fmin(0.999 * dyn_ratio_step<Team>(c, z, dz, s, ds), 1.0);
         TFOR(i, nq) xy[i] += alpha * dxy[i];
         TFOR(r, ni) { s[r] += alpha * ds[r]; z[r] += alpha * dz[r]; }
         Team::sync();
+        DP_MARK(DP_UPDATE);
     }
     if (ni > 0 && have_best && best_res > 1.0) status |= DSDF_LCP_INACCURATE;
     Team::sync();
@@ -864,6 +949,20 @@ int dsdf_dynamics_solve_backward(const double* p, const double* v, const double*
         if (rc) return rc;
     }
     return 0;
+}
+
+int dsdf_dynamics_phase_cycles(unsigned long long* out11, int reset) {   /* out: DP_COUNT = 11 counters */
+#ifdef DSDF_PHASE_PROFILE
+    if (out11 && cudaMemcpyFromSymbol(out11, g_dyn_phase, sizeof(unsigned long long) * DP_COUNT) != cudaSuccess) return 1;
+    if (reset) {
+        unsigned long long z[DP_COUNT] = {0};
+        if (cudaMemcpyToSymbol(g_dyn_phase, z, sizeof(z)) != cudaSuccess) return 1;
+    }
+    return 0;
+#else
+    (void)out11; (void)reset;
+    return -1;
+#endif
 }
 
 }  // extern "C"

@@ -181,6 +181,11 @@ int dsdf_filter_contacts(const double* normals, const double* p1, const int32_t*
  * [overlap, gather, sort+init, frank-wolfe, push+compact, geometry, filter, append]; returns -1 unless the library
  * was built with -DDSDF_PHASE_PROFILE (DSDF_PHASE_PROFILE=1 python -m diffsdfsim_b200.build). Host pointer out8. */
 int dsdf_contacts_phase_cycles(unsigned long long* out8, int reset);
+/* Profiling aid: cumulative SM cycles (lane / thread 0 of every CTA) per phase of the dynamics forward kernel
+ * [load, residuals, factor (a, den, AP, YG), M~_FF assembly, LU, KKT solve pass 0, ratio step + corrector,
+ * KKT solve pass 1, step update, best-iterate tracking] and, last, the number of loop passes (the initial point
+ * included); returns -1 unless the library was built with -DDSDF_PHASE_PROFILE. Host pointer out11. */
+int dsdf_dynamics_phase_cycles(unsigned long long* out11, int reset);
 /* VJP of cgeo w.r.t. the poses (the reference's grad-enabled second _compute_contacts, contacts.py:262-264):
  * gp (W,nb,7) from ggeo (W,maxc,10).  wmap (W) or NULL: row w carries the poses / contacts of world wmap[w], whose
  * shapes and per-world meshes / grids are used (a compact batch of rows; NULL: row = world).

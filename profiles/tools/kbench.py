@@ -39,12 +39,27 @@ if rc == 0:
     names += ['iters', 'cand', 'pre', 'f.cluster', 'f.stats', 'f.akl', 'f.sort(+dedupe)', 'f.chain']
     for n, v in zip(names, buf):
         print('   %-14s %5.1f %%   %8.0f cycles/world/launch' % (n, 100.0 * v / max(tot, 1), v / 6 / W))
+dbuf = (ctypes.c_ulonglong * 11)()
+DYN_NAMES = ['load', 'residuals', 'factor', 'assembly', 'lu', 'solve0', 'ratio+corr', 'solve1', 'update', 'best']
+def dyn_phases(label, nworlds):
+    # per world-launch; the counters cover every timed launch and the warm-up one
+    if L.dsdf_dynamics_phase_cycles(dbuf, 1) != 0:
+        return
+    tot = sum(dbuf[:10])
+    launches = 6 * nworlds
+    print('   %s: %.1f loop passes per world, %.0f cycles per world' % (label, dbuf[10] / launches, tot / launches))
+    for n, v in zip(DYN_NAMES, dbuf):
+        print('   %-14s %5.1f %%   %8.0f cycles/world/launch' % (n, 100.0 * v / max(tot, 1), v / launches))
 with torch.no_grad():
     dt = torch.full((W,), world.dt, dtype=torch.float64, device='cuda')
+    L.dsdf_dynamics_phase_cycles(dbuf, 1)
     ms = timeit(lambda: world.engine.solve(world, dt, act))
 print('dynamics_solve %.3f ms / launch, max_nc %d' % (ms, world.max_nc))
+dyn_phases('dense', W)
 one = torch.zeros(W, dtype=torch.uint8, device='cuda'); one[7] = 1
 ms1 = timeit(lambda: world.detector.detect(p, world.shape, cs, one, eps=world.eps, tol=world.tol, fd_eps=Defaults3D.EPSILON, body_eps=world.body_eps))
 with torch.no_grad():
+    L.dsdf_dynamics_phase_cycles(dbuf, 1)
     ms2 = timeit(lambda: world.engine.solve(world, dt, one))
 print('single active world: contacts %.3f ms, dynamics %.3f ms' % (ms1, ms2))
+dyn_phases('single world', 1)
